@@ -96,10 +96,11 @@ class ClockSampler:
 
 
 def load_golden_scene():
-    """The headline scene as a committed RTBS blob + camera (tests/golden/book2_final.rtbs, .json - written by
+    """The headline scene as a committed RTBS blob + camera (tests/golden/book2_final.rtbs.xz, .json - written by
     tests/golden/make_golden.py scenes): the reference arm maps only oracle/, never the product's libraries."""
+    import lzma
     orc = importlib.import_module("pyoracle")
-    blob = (ROOT / "tests" / "golden" / f"{SCENE}.rtbs").read_bytes()
+    blob = lzma.decompress((ROOT / "tests" / "golden" / f"{SCENE}.rtbs.xz").read_bytes())
     meta = json.loads((ROOT / "tests" / "golden" / f"{SCENE}.json").read_text())
     return orc, orc.OracleScene(blob), orc.camera_from_dict(meta["camera"]), meta
 
@@ -181,7 +182,11 @@ def main():
     ap.add_argument("--ref-spp", type=int, default=16, help="samples per pixel per step of the --impl reference arm")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-reference-gpu", action="store_true", help="skip the reference megakernel run beside ours (A/B runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the framebuffer of the last timed step "
+                    "(radiance sums + sample count, float32, 800x800x4; rank 0 after the reduce) to DIR/accum.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.gpus > 1 and world == 1:
@@ -250,6 +255,10 @@ def main():
     clocks = sampler.stop()
     ms = ev0.elapsed_time(ev1)
     cnt = r.counters()
+    if args.dump_outputs and rank == 0:
+        # what rtb_render left in the accumulator after the last timed step (inputs are fixed by seed and sample range)
+        Path(args.dump_outputs).mkdir(parents=True, exist_ok=True)
+        np.save(Path(args.dump_outputs) / "accum.npy", r.download_accum())
     rank_ms = [ms]
     if world > 1:
         gathered = [torch.zeros(1, dtype=torch.float64, device="cuda") for _ in range(world)]

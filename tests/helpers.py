@@ -99,6 +99,56 @@ REF_TRACE_DTYPE = np.dtype([("t", np.float32), ("n", np.float32, 3), ("p", np.fl
 assert REF_TRACE_DTYPE.itemsize == 32
 
 
+def _trace_estimates(rays, index, t=None):
+    """Float32 hit records recomputed from the ray and the sphere in a fixed order: t from the quadratic (the near root,
+    else the far one) unless given, p = o + d t (rounded once), n = (p - c) / r, moving centres at c0 (1 - time) + c1 time;
+    on misses t = FLT_MAX and p = n = 0.  Equal or within a few ulps of the reference's records on most rays.  The
+    spheres are the ones the reference built (tests/golden/ref_scene_book2_bouncing.bin), not the product's."""
+    from pathlib import Path
+    raw = np.fromfile(Path(__file__).resolve().parent / "golden" / "ref_scene_book2_bouncing.bin", dtype=np.uint8)
+    rec = np.frombuffer(raw[4:], dtype=np.float32).reshape(int(np.frombuffer(raw[:4], dtype=np.int32)[0]), 16)
+    hit = index >= 0
+    sp = rec[np.maximum(index, 0)]                                   # [moving, c0 | c, r (static) / c1 (moving), r (moving)]
+    moving = sp[:, 0] == 1.0
+    f0, f1 = np.float32(0), np.float32(1)
+    with np.errstate(over="ignore", invalid="ignore", divide="ignore"):
+        tm = rays["time"][:, None]
+        c0 = sp[:, 1:4]; c1 = sp[:, 4:7]; r = np.where(moving, sp[:, 7], sp[:, 4])
+        c = np.where(moving[:, None], c0 * (f1 - tm) + c1 * tm, c0)
+        if t is None:
+            oc = rays["o"] - c; d = rays["d"]
+            dot = lambda x, y: x[:, 0] * y[:, 0] + x[:, 1] * y[:, 1] + x[:, 2] * y[:, 2]
+            a, hb, cc = dot(d, d), dot(d, oc), dot(oc, oc) - r * r
+            sq = np.sqrt(np.maximum(hb * hb - a * cc, f0))
+            near = (-hb - sq) / a
+            t = np.where(hit, np.where(near > np.float32(0.001), near, (-hb + sq) / a), np.finfo(np.float32).max).astype(np.float32)
+        p = (rays["o"].astype(np.float64) + rays["d"].astype(np.float64) * t.astype(np.float64)[:, None]).astype(np.float32)
+        p = np.where(hit[:, None], p, f0)
+        n = np.where(hit[:, None], (p - c) / r[:, None], f0)
+    return t, p, n
+
+
+def encode_reference_trace(rays, rec):
+    """The reference's hit records as stored in tests/golden/ref_trace_book2_bouncing.npz: the sphere index as it is, t as
+    the difference of its bit pattern from the estimate's (a few ulps), point and normal as the bitwise XOR with their
+    estimates from that t (mostly zero): small integers, so the file is a fraction of the records' size."""
+    t_est, _, _ = _trace_estimates(rays, rec["index"])
+    _, p_est, n_est = _trace_estimates(rays, rec["index"], rec["t"])
+    return {"index": rec["index"].astype(np.int16), "t_diff": (rec["t"].view(np.uint32) - t_est.view(np.uint32)).view(np.int32),
+            "p_xor": rec["p"].view(np.uint32) ^ p_est.view(np.uint32), "n_xor": rec["n"].view(np.uint32) ^ n_est.view(np.uint32)}
+
+
+def load_reference_trace(rays, path):
+    """Inverse of encode_reference_trace: the exact records (t, n, p, index) the reference's device code returned."""
+    z = np.load(path)
+    index = z["index"].astype(np.int32)
+    t_est, _, _ = _trace_estimates(rays, index)
+    t = (t_est.view(np.uint32) + z["t_diff"].view(np.uint32)).view(np.float32)
+    _, p_est, n_est = _trace_estimates(rays, index, t)
+    return {"t": t, "index": index, "p": (z["p_xor"] ^ p_est.view(np.uint32)).view(np.float32),
+            "n": (z["n_xor"] ^ n_est.view(np.uint32)).view(np.float32)}
+
+
 def test_spheres(rtb):
     """The 488 spheres of SphereTest::_populate_world (google_testing/test.cpp:36-85): SceneBook2BVH's spheres, the
     moving ones static at center0 - (center.xyz, radius) rows in construction order."""

@@ -94,14 +94,33 @@ def test_bvh_bit_exact_vs_reference_golden(rtb, orc):
     assert np.array_equal(wn.view(np.uint8), gn.view(np.uint8)) and wr == gr
 
 
-@pytest.mark.skipif(not (ROOT / "oracle" / "_ref" / "ref_bvh").exists(), reason="reference-derived checker not built (needs /root/reference)")
-@pytest.mark.parametrize("builder,n", [(0, 3000), (0, 1), (0, 2), (0, 37), (2, 120)])
-def test_bvh_bit_exact_vs_reference_live(rtb, orc, builder, n, tmp_path):
-    """Random boxes with duplicate sort keys (the reference uses an unstable std::sort) through the reference's own BVH.cu."""
+BVH_CASES = [(0, 3000), (0, 1), (0, 2), (0, 37), (2, 120)]
+
+
+def _duplicate_key_boxes(builder, n):
+    """Seeded random boxes with duplicate sort keys (the reference uses an unstable std::sort)."""
     rng = np.random.default_rng(n + builder)
     c = rng.uniform(-50, 50, (n, 3)).astype(np.float32); r = rng.uniform(0.1, 3, (n, 1)).astype(np.float32)
     c[::3, 0] = np.round(c[::3, 0]); c[::5] = c[0]
-    boxes = np.concatenate([c - r, c + r], 1)
+    return np.concatenate([c - r, c + r], 1)
+
+
+@pytest.mark.parametrize("builder,n", BVH_CASES)
+def test_bvh_builders_product_equals_oracle(rtb, orc, builder, n):
+    """The product's builders and the oracle's restatement give the same node array, primitive order and root on the
+    boxes of test_bvh_bit_exact_vs_reference_live, which needs the reference-derived checker."""
+    boxes = _duplicate_key_boxes(builder, n)
+    gn, go, gr = orc.bvh_build(boxes, builder, rtb.BVH_NODE_DTYPE)
+    got = rtb.bvh_build(boxes, builder)
+    assert len(gn) == 2 * n - 1 and sorted(go.tolist()) == list(range(n))
+    assert np.array_equal(got[0].view(np.uint8), gn.view(np.uint8)) and np.array_equal(got[1], go) and got[2] == gr
+
+
+@pytest.mark.skipif(not (ROOT / "oracle" / "_ref" / "ref_bvh").exists(), reason="reference-derived checker not built (make -C oracle ref with a checkout of the reference)")
+@pytest.mark.parametrize("builder,n", BVH_CASES)
+def test_bvh_bit_exact_vs_reference_live(rtb, orc, builder, n, tmp_path):
+    """Random boxes with duplicate sort keys (the reference uses an unstable std::sort) through the reference's own BVH.cu."""
+    boxes = _duplicate_key_boxes(builder, n)
     fin, fout = tmp_path / "in.bin", tmp_path / "out.bin"
     fin.write_bytes(struct.pack("i", n) + boxes.tobytes())
     subprocess.run([str(ROOT / "oracle" / "_ref" / "ref_bvh"), str(fin), str(fout), str(builder)], check=True)
@@ -181,23 +200,25 @@ def test_sphere_index_recipe_cpu(rtb, orc):
     assert (hits["object"].reshape(H, W) == truth).mean() > 0.9999
 
 
-@pytest.mark.skipif(not (ROOT / "oracle" / "_ref" / "ref_sphere_index").exists(), reason="reference-derived checker not built (needs /root/reference)")
 def test_sphere_index_recipe_reference_functions(rtb, orc, tmp_path):
     """The reference's own unit test (google_testing/test.cpp:87-106), with the reference's own functions as the truth:
     _sphere_closest_intersection (SphereHittable.cuh:15-33) and PinholeCamera (cu_Cameras.cuh:12-31) compiled from the
-    reference's headers (oracle/_ref/ref_sphere_index host).  The committed golden is that binary's output; the camera
-    the product's rtb_camera_pinhole builds and the rays numpy builds from it are the reference's, bit for bit; and the
+    reference's headers (oracle/_ref/ref_sphere_index host).  The committed golden is that binary's output (run live as
+    well when the binary is present, and then the rays numpy builds must be the reference's, bit for bit); the camera
+    the product's rtb_camera_pinhole builds is the reference's, bit for bit; and the
     oracle's BVH trace names the reference's sphere on all 921,600 pixels but the handful where a sphere is grazed
     within float32 rounding (the reference's host code does not contract multiply-adds, the arithmetic spec does)."""
     from helpers import grazing_only, reference_sphere_index, test_spheres
     W, H = 1280, 720
-    idx, cam12, ref_rays = reference_sphere_index(rtb, "host", tmp_path, W, H)
     gold = np.load(GOLDEN / "ref_sphere_index_host_1280x720.npz")
-    assert np.array_equal(gold["index"].reshape(-1).astype(np.int32), idx) and np.array_equal(gold["camera"], cam12)
+    idx, cam12 = gold["index"].reshape(-1).astype(np.int32), gold["camera"]
     cam = rtb.make_camera("pinhole", (0, 1, -4), (0, 1, 0), (0, 1, 0), 90.0, W / H)
     assert np.array_equal(np.array([*cam.o, *cam.u, *cam.v, *cam.w], dtype=np.float32), cam12)
     rays = camera_rays(rtb, cam, W, H, "test")
-    assert np.array_equal(rays["d"].view(np.uint32), ref_rays["d"].view(np.uint32)) and np.array_equal(rays["o"], ref_rays["o"])
+    if (ROOT / "oracle" / "_ref" / "ref_sphere_index").exists():
+        live, live_cam12, ref_rays = reference_sphere_index(rtb, "host", tmp_path, W, H)
+        assert np.array_equal(live, idx) and np.array_equal(live_cam12, cam12)
+        assert np.array_equal(rays["d"].view(np.uint32), ref_rays["d"].view(np.uint32)) and np.array_equal(rays["o"], ref_rays["o"])
     sp = test_spheres(rtb)
     s = rtb.Scene(); m = s.lambertian(albedo=(0.5, 0.5, 0.5))
     s.set_root(s.bvh([s.sphere(c[:3], float(c[3]), m) for c in sp]))
@@ -215,11 +236,11 @@ def test_oracle_hit_records_match_reference_device(rtb, orc):
     (camera rays with shutter times, random segments, grazing rays; moving spheres at many times) by
     `oracle/_ref/ref_render trace` - tests/golden/ref_trace_book2_bouncing.npz.  The sphere hit is the same one; t, point and
     normal lie inside the binary32 rounding bound of the reference's formula (see helpers.check_against_reference_trace)."""
-    from helpers import check_against_reference_trace, reference_trace_rays
+    from helpers import check_against_reference_trace, load_reference_trace, reference_trace_rays
     rays = reference_trace_rays(rtb)
     s = rtb.Scene.named("book2_bouncing")
     got = orc.OracleScene(s.serialize()).trace_rays(rays, rtb.HIT_DTYPE)
-    print(check_against_reference_trace(rtb, rays, got, np.load(GOLDEN / "ref_trace_book2_bouncing.npz")))
+    print(check_against_reference_trace(rtb, rays, got, load_reference_trace(rays, GOLDEN / "ref_trace_book2_bouncing.npz")))
 
 
 def test_medium_transmission_known_answer(rtb, orc):
@@ -334,15 +355,17 @@ def test_analytic_perlin_lattice(rtb, orc):
 
 
 def test_committed_headline_scene_is_current(rtb, orc):
-    """tests/golden/book2_final.rtbs + .json (what `bench.py --impl reference` renders without touching the product) is
+    """tests/golden/book2_final.rtbs.xz + .json (what `bench.py --impl reference` renders without touching the product) is
     what the host mirror builds today, byte for byte, camera included."""
     import json
+    import lzma
     s = rtb.Scene.named("book2_final")
-    assert (GOLDEN / "book2_final.rtbs").read_bytes() == s.serialize()
+    blob = lzma.decompress((GOLDEN / "book2_final.rtbs.xz").read_bytes())
+    assert blob == s.serialize()
     meta = json.loads((GOLDEN / "book2_final.json").read_text())
     assert (meta["width"], meta["height"], meta["max_depth"]) == (s.info.width, s.info.height, s.info.max_depth)
     cam = orc.camera_from_dict(meta["camera"])
     assert bytes(cam) == bytes(s.info.camera)
-    a, _, ra = orc.OracleScene((GOLDEN / "book2_final.rtbs").read_bytes()).render(cam, 24, 24, 0, 2, 12, seed=3)
+    a, _, ra = orc.OracleScene(blob).render(cam, 24, 24, 0, 2, 12, seed=3)
     b, _, rb = orc.OracleScene(s.serialize()).render(s.info.camera, 24, 24, 0, 2, 12, seed=3)
     assert np.array_equal(a, b) and ra == rb

@@ -92,12 +92,13 @@ def test_hit_records_match_reference_device(rtb, renderer):
     and normal inside the binary32 rounding bound of the reference's formula (helpers.check_against_reference_trace says
     why north_star's flat 1e-5 cannot be the bar on the r = 1000 sphere, and checks it where it can)."""
     from conftest import GOLDEN
-    from helpers import check_against_reference_trace, reference_trace_rays
+    from helpers import check_against_reference_trace, load_reference_trace, reference_trace_rays
     rays = reference_trace_rays(rtb)
     scene = rtb.Scene.named("book2_bouncing")
     renderer.set_scene(scene)
     got = renderer.trace_rays(rays)
-    print("reference device hit records:", check_against_reference_trace(rtb, rays, got, np.load(GOLDEN / "ref_trace_book2_bouncing.npz")))
+    gold = load_reference_trace(rays, GOLDEN / "ref_trace_book2_bouncing.npz")
+    print("reference device hit records:", check_against_reference_trace(rtb, rays, got, gold))
 
 
 @pytest.mark.parametrize("name,lo,hi", [("book2_bouncing", -12, 12), ("book1_final", -12, 12), ("book2_quads", -6, 9)])
