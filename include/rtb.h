@@ -122,6 +122,20 @@ int rtb_scene_set_background(rtb_scene* s, int mode, const float rgb[3]);
 enum rtb_world_bvh_mode { RTB_WORLD_BVH_QUALITY = 0, RTB_WORLD_BVH_AS_BUILT = 1, RTB_WORLD_BVH_GPU_LBVH = 2 };
 int rtb_scene_set_world_bvh(rtb_scene* s, int mode);
 
+/* Light importance sampling ("Ray Tracing: The Rest of Your Life", mixture pdfs), opt-in per scene.  `objects` names
+ * n <= RTB_MAX_SAMPLED_LIGHTS emitters, each a sphere, a quad, or a translate / rotate_y chain ending in one; it is
+ * sampled where the chain puts it (the chain from the listed object down, composed as the flattener composes instances).
+ * At every Lambertian or isotropic scatter, half of the directions then aim at a point drawn on one of the listed
+ * objects (chosen uniformly; quads: uniform in area; spheres: uniform in the cone they subtend) and half are the
+ * material's own (cosine-weighted / uniform) directions; the throughput is weighted by scattering pdf / mixture pdf
+ * (DESIGN.md §5b).  The expected image does not depend on the list - any list, even one naming objects that do not
+ * emit, gives the same converged image - only the noise does.  n = 0 clears the list; a scene without one renders,
+ * serialises and hashes exactly as if this had never been called.  Moving spheres, triangles, boxes, lists, BVHs and
+ * media return RTB_ERR_UNSUPPORTED; bad ids, n outside [0, 16], a quad without area return RTB_ERR_INVALID (the list
+ * is then left unchanged). */
+#define RTB_MAX_SAMPLED_LIGHTS 16
+int rtb_scene_set_sampled_lights(rtb_scene* s, const int* objects, int n);
+
 int rtb_scene_num_objects(const rtb_scene* s);
 /* Children of a list / BVH / mesh group (1 for translate, rotate_y, constant_medium; 0 for primitives). */
 int rtb_scene_num_children(const rtb_scene* s, int object);

@@ -12,6 +12,10 @@
  *   rtbs_object   [n_objects]
  *   int32         children[n_children]     (LIST / BVH members)
  *   uint8         blob[n_blob_bytes]       (image texels RGB8; Perlin tables)
+ *   int32         n_lights                 (version 2 only: the scene's sampled lights,
+ *   int32         lights[n_lights]          rtb_scene_set_sampled_lights)
+ *
+ * A scene without sampled lights is written as version 1; readers accept versions 1 and 2.
  */
 #ifndef RTB_SCENE_FORMAT_H
 #define RTB_SCENE_FORMAT_H
@@ -20,6 +24,7 @@
 
 #define RTBS_MAGIC 0x53425452u /* "RTBS" */
 #define RTBS_VERSION 1u
+#define RTBS_VERSION_LIGHTS 2u
 
 typedef struct rtbs_header {
 	uint32_t magic, version;

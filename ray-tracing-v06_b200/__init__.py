@@ -22,7 +22,8 @@ _HERE = Path(__file__).resolve().parent
 LIB_PATH = Path(os.environ["RTB_LIB"]) if os.environ.get("RTB_LIB") else _HERE / "librtb200.so"   # RTB_LIB: experimental builds only
 SCENES_LIB_PATH = _HERE / "librtb200_scenes.so"
 DEBUG_LIB_PATH = _HERE / "librtb200_debug.so"     # the same library built with -DRTB_DEBUG_BOUNDS=1 (select it with RTB_LIB)
-BOUNDS_CLASSES = ("stack", "node", "primitive", "material", "texture", "queue", "path", "bin")
+BOUNDS_CLASSES = ("stack", "node", "primitive", "material", "texture", "queue", "path", "bin")   # (light indices count as "primitive")
+MAX_SAMPLED_LIGHTS = 16
 
 RTB_OK = 0
 TEX_SOLID, TEX_CHECKER, TEX_IMAGE, TEX_NOISE = 0, 1, 2, 3
@@ -79,7 +80,13 @@ class Profile(C.Structure):
 
 
 class SceneInfo(C.Structure):
-    _fields_ = [("camera", Camera), ("width", C.c_int32), ("height", C.c_int32), ("spp", C.c_int32), ("max_depth", C.c_int32)]
+    _fields_ = [("camera", Camera), ("width", C.c_int32), ("height", C.c_int32), ("spp", C.c_int32), ("max_depth", C.c_int32),
+                ("n_lights", C.c_int32), ("lights", C.c_int32 * 8)]
+
+    @property
+    def light_ids(self) -> list[int]:
+        """The emitters the scene's author names for light sampling (pass them to Scene.sample_lights)."""
+        return [int(self.lights[i]) for i in range(self.n_lights)]
 
 
 RAY_DTYPE = np.dtype([("o", np.float32, 3), ("time", np.float32), ("d", np.float32, 3), ("pad", np.float32)])
@@ -120,6 +127,7 @@ ABI = {
     "rtb_scene_set_root": (C.c_int, [_P, C.c_int]),
     "rtb_scene_set_background": (C.c_int, [_P, C.c_int, _F3]),
     "rtb_scene_set_world_bvh": (C.c_int, [_P, C.c_int]),
+    "rtb_scene_set_sampled_lights": (C.c_int, [_P, C.POINTER(C.c_int), C.c_int]),
     "rtb_scene_num_children": (C.c_int, [_P, C.c_int]),
     "rtb_scene_num_objects": (C.c_int, [_P]),
     "rtb_object_bounds": (C.c_int, [_P, C.c_int, _F3]),
@@ -329,6 +337,12 @@ class Scene:
     def set_root(self, obj): _check(lib().rtb_scene_set_root(self.handle, obj), "rtb_scene_set_root")
     def set_background(self, mode, rgb=(0, 0, 0)): _check(lib().rtb_scene_set_background(self.handle, mode, _f3(rgb)), "rtb_scene_set_background")
     def set_world_bvh(self, mode): _check(lib().rtb_scene_set_world_bvh(self.handle, mode), "rtb_scene_set_world_bvh")
+    def sample_lights(self, ids):
+        """Light importance sampling towards these objects (spheres / quads, optionally under translate / rotate_y);
+        an empty list turns it off (rtb_scene_set_sampled_lights)."""
+        ids = [int(i) for i in ids]
+        arr = (C.c_int * max(len(ids), 1))(*ids)
+        _check(lib().rtb_scene_set_sampled_lights(self.handle, arr, len(ids)), "rtb_scene_set_sampled_lights")
     def num_objects(self): return lib().rtb_scene_num_objects(self.handle)
 
     def bounds(self, obj) -> np.ndarray:

@@ -766,12 +766,74 @@ __device__ __forceinline__ bool texture_needs_uv(const SceneView& sv, int tex) {
 	return kind != RTB_TEX_SOLID && kind != RTB_TEX_NOISE;   // checker children may be images
 }
 
+// ------------------------------------------------------------------------------------------------
+// light sampling: the half-and-half mixture of the material's own directions and directions towards the sampled lights
+// (DESIGN.md §5b, "Ray Tracing: The Rest of Your Life")
+
+struct LightKey { uint32_t seed, pixel, sample, bounce; };   // what the STREAM_LIGHT block of a scatter is drawn from
+
+// pdf (per solid angle) of light i's own sampling for the direction u (unit) from p
+__device__ __forceinline__ float light_pdf(const SceneView& sv, int i, v3 p, v3 u) {
+	const float4* lp = sv.lights + 4 * i;
+	const float4 q0 = ldg4(lp);
+	const float4 info = ldg4(sv.lights + 4 * sv.n_lights + i);
+	if (__float_as_int(info.x) == PRIM_QUAD) {
+		const float t = planar_hit(p, u, lp, q0, false, FLT_MAX);
+		if (!(t > 0.0f) || !(t < FLT_MAX)) return 0.0f;
+		const v3 N = rt::mk(ldg4(lp + 1).w, ldg4(lp + 2).w, ldg4(lp + 3).w);
+		return (t * t) / (fabsf(rt::dot(u, N)) * info.y);
+	}
+	const v3 e = rt::sub(xyz(q0), p);
+	const float d2 = rt::dot(e, e), R2 = q0.w * q0.w;
+	if (!(d2 > R2)) return 0.0f;                                     // inside or on the light: it cannot be sampled
+	if (!(sphere_closest(p, u, rt::dot(u, u), xyz(q0), q0.w) < FLT_MAX)) return 0.0f;
+	return rt::cone_pdf(rt::cone_cos_max(d2, R2));
+}
+
+// Direction and weight (scattering pdf / mixture pdf) of a Lambertian (ISO = false) or isotropic scatter; false: the
+// path ends black.
+template <bool ISO>
+__device__ __forceinline__ bool light_mix(const SceneView& sv, const Surface& s, const rt::f4& r, const LightKey& lk, v3& dir, float& w) {
+	const rt::f4 l = rt::rng4(lk.seed, lk.pixel, lk.sample, lk.bounce, rt::STREAM_LIGHT);
+	const int n = sv.n_lights;
+	if (l.x < 0.5f) {                                                // towards a point on light k
+		int k = (int)(l.y * (float)n); k = k < n - 1 ? k : n - 1;
+		RTB_CHECK(k >= 0 && k < sv.n_lights, RTB_BOUNDS_PRIM);
+		const float4* lp = sv.lights + 4 * k;
+		const float4 q0 = ldg4(lp);
+		if (__float_as_int(ldg4(sv.lights + 4 * n + k).x) == PRIM_QUAD) {
+			const v3 e = rt::sub(rt::madd(xyz(ldg4(lp + 2)), l.w, rt::madd(xyz(ldg4(lp + 1)), l.z, xyz(q0))), s.p);
+			if (!(rt::dot(e, e) > 0.0f)) return false;
+			dir = rt::normalize(e);
+		} else {
+			const v3 e = rt::sub(xyz(q0), s.p);
+			const float d2 = rt::dot(e, e), R2 = q0.w * q0.w;
+			if (!(d2 > R2)) return false;
+			dir = rt::cone_direction(e, rt::cone_cos_max(d2, R2), l.z, l.w);
+		}
+	} else if (ISO) {
+		dir = rt::unit_sphere(r.x, r.y);
+	} else {
+		dir = rt::add(s.n_shade, rt::unit_sphere(r.x, r.y));
+		if (rt::near_zero(dir, 1e-9f)) return false;
+	}
+	const v3 u = rt::normalize(dir);
+	const float spdf = ISO ? RT_INV_4PI : fmaxf(0.0f, rt::dot(s.n_shade, u)) * RT_INV_PI;
+	if (!(spdf > 0.0f)) return false;
+	float sum = 0.0f;
+	for (int i = 0; i < n; ++i) sum += light_pdf(sv, i, s.p, u);
+	w = rt::mixture_weight(spdf, sum / (float)n);
+	return w > 0.0f;
+}
+
 // Material::Scatter for every material kind.  Returns 0 = absorbed (path ends black),
 // 1 = scattered (dir/attenuation valid), 2 = emitted (attenuation holds the emitted radiance).
 // With DEFER, an image / noise albedo of a scattering material is not evaluated here: attenuation is
 // left at 1 and defer_tex names the texture, to be multiplied in later by texture_kernel (dense warps).
-template <bool DEFER>
-__device__ __forceinline__ int scatter(const SceneView& sv, int mat, const Surface& s, v3 d, const rt::f4& r, v3& dir, v3& att, int& defer_tex) {
+// With LIGHTS, Lambertian and isotropic scatters draw from the light mixture and set w (1 otherwise).
+template <bool DEFER, bool LIGHTS>
+__device__ __forceinline__ int scatter(const SceneView& sv, int mat, const Surface& s, v3 d, const rt::f4& r, const LightKey& lk,
+                                       v3& dir, v3& att, float& w, int& defer_tex) {
 	RTB_CHECK(mat >= 0 && mat < sv.n_materials, RTB_BOUNDS_MATERIAL);
 	const float4 m0 = ldg4(sv.materials + 2 * mat), m1 = ldg4(sv.materials + 2 * mat + 1);
 	const int kind = __float_as_int(m0.x), tex = __float_as_int(m0.y);
@@ -786,6 +848,7 @@ __device__ __forceinline__ int scatter(const SceneView& sv, int mat, const Surfa
 	}
 	switch (kind) {
 	case RTB_MAT_LAMBERTIAN: {   // LambertianAbstract / LambertianTexture  cu_materials.cuh:26-40,52-64
+		if (LIGHTS) { att = albedo; return light_mix<false>(sv, s, r, lk, dir, w) ? 1 : 0; }
 		dir = rt::add(s.n_shade, rt::unit_sphere(r.x, r.y));
 		if (rt::near_zero(dir, 1e-9f)) return 0;
 		att = albedo; return 1;
@@ -819,6 +882,7 @@ __device__ __forceinline__ int scatter(const SceneView& sv, int mat, const Surfa
 		att = albedo; return 1;
 	}
 	case RTB_MAT_ISOTROPIC: {    // book isotropic::scatter
+		if (LIGHTS) { att = albedo; return light_mix<true>(sv, s, r, lk, dir, w) ? 1 : 0; }
 		dir = rt::unit_sphere(r.x, r.y);
 		att = albedo; return 1;
 	}
@@ -843,7 +907,7 @@ __device__ __forceinline__ v3 background(const SceneView& sv, v3 d) {
 // been written to contrib[path].
 struct DeferredTex { int tex; float u, v; v3 p; };
 
-template <bool DEFER>
+template <bool DEFER, bool LIGHTS>
 __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t batch, uint32_t bounce,
                                               const float4& fo, const float4& fd, v3 thr, float t, int code,
                                               float4& no, float4& nd, v3& nthr, DeferredTex& dt) {
@@ -866,7 +930,8 @@ __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchPa
 	path_pixel_sample(bp, batch, path, pixel, sample);
 	const rt::f4 r = rt::rng4(bp.seed, pixel, sample, bounce, rt::STREAM_SCATTER);
 	v3 dir, att;
-	const int res = scatter<DEFER>(sv, info.x, s, d, r, dir, att, dt.tex);
+	float w = 1.0f;
+	const int res = scatter<DEFER, LIGHTS>(sv, info.x, s, d, r, LightKey{bp.seed, pixel, sample, bounce}, dir, att, w, dt.tex);
 	dt.u = s.u; dt.v = s.v; dt.p = s.p;
 	if (res == 2) {                                       // emitter: throughput * emitted, path ends
 		v3 c = rt::mulv(thr, att);
@@ -876,7 +941,7 @@ __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchPa
 	if (res != 1 || bounce + 1 >= bp.max_depth) { dt.tex = -1; return false; }   // absorbed, or out of depth: black   Renderer.cu:164,180
 	// scatter_ray = Ray(at(t), dir, time); o += d * 0.001   Renderer.cu:168-175
 	v3 o2 = rt::madd(dir, 0.001f, s.p);
-	nthr = rt::mulv(thr, att);
+	nthr = LIGHTS ? rt::mulv(rt::mul(thr, w), att) : rt::mulv(thr, att);   // (thr * w) * albedo: the order texture_kernel keeps
 	no = make_float4(o2.x, o2.y, o2.z, fo.w);
 	nd = make_float4(dir.x, dir.y, dir.z, fd.w);
 	return true;
@@ -949,6 +1014,7 @@ __device__ __forceinline__ void bin_table_flush(uint32_t* s_key, uint32_t* s_cnt
 #ifndef SHADE_MIN_BLOCKS
 #define SHADE_MIN_BLOCKS 8   // 8 x 128 threads x 64 registers = the whole register file (6 / 9 / 10 blocks: 11.7 / 10.9 / 12.4 ms)
 #endif
+template <bool LIGHTS>
 __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS)
 shade_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int q) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -979,7 +1045,7 @@ shade_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int 
 			float4 fo, fd; ld_ray(rod + 2 * (size_t)i, fo, fd);
 			const float4 ft = ldq(rt_ + i);
 			const int2 h = ldq(wv.hit + i);
-			alive = shade_segment<true>(sv, bp, wv, batch, bounce, fo, fd, xyz(ft), __int_as_float(h.x), h.y, no, nd, nthr, dt);
+			alive = shade_segment<true, LIGHTS>(sv, bp, wv, batch, bounce, fo, fd, xyz(ft), __int_as_float(h.x), h.y, no, nd, nthr, dt);
 		}
 		// live-path compaction: warp ballot/popc, one global atomic per block
 		const uint32_t mask = __ballot_sync(FULL_MASK, alive);
@@ -1181,7 +1247,7 @@ bin_permute_kernel(SceneView sv, WaveView wv, uint32_t bounce, int q_from) {
 // One persistent launch then runs every remaining path to completion (traverse + shade fused, one
 // thread per path); later traverse/shade launches of the batch see tail_from and return at once.
 
-template <bool MEDIA, int STACK>
+template <bool MEDIA, int STACK, bool LIGHTS>
 __global__ void __launch_bounds__(TRAVERSE_THREADS)
 tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int q, uint32_t threshold) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -1207,7 +1273,7 @@ tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int 
 			trace_ray<(MEDIA ? 2 : 0)>(sv, xyz(fo), xyz(fd), fo.w, mr, s_stack + threadIdx.x, STACK, t, code);
 			float4 no, nd; v3 nthr;
 			DeferredTex dt;
-			if (!shade_segment<false>(sv, bp, wv, batch, b, fo, fd, thr, t, code, no, nd, nthr, dt)) break;
+			if (!shade_segment<false, LIGHTS>(sv, bp, wv, batch, b, fo, fd, thr, t, code, no, nd, nthr, dt)) break;
 			fo = no; fd = nd; thr = nthr;
 		}
 	}
@@ -1357,12 +1423,12 @@ void query_occupancy(int device, LaunchCfg& lc) {
 	int occ_t = 0, occ_tm = 0, occ_s = 0, occ_g = 0;
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_t, traverse_kernel<0, STACK_SIZE>, TRAVERSE_THREADS, 0);
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_tm, traverse_kernel<2, STACK_SIZE>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, shade_kernel, SHADE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, shade_kernel<false>, SHADE_THREADS, 0);
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_g, generate_kernel, STREAM_THREADS, 0);
 	int occ_trav = occ_t < occ_tm ? occ_t : occ_tm;
 	int occ_l = 0, occ_lm = 0;
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_l, tail_kernel<false, STACK_SIZE>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_lm, tail_kernel<true, STACK_SIZE>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_l, tail_kernel<false, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_lm, tail_kernel<true, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
 	int occ_tail = occ_l < occ_lm ? occ_l : occ_lm;
 	lc.blocks_tail = sms * (occ_tail > 0 ? occ_tail : 1);
 	lc.sms = sms;
@@ -1395,16 +1461,21 @@ void launch_traverse(const SceneView& sv, const BatchParams& bp, const WaveView&
 }
 void launch_tail(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t bounce, int q, uint32_t threshold, const LaunchCfg& lc, cudaStream_t st) {
 	const bool deep = sv.tree_depth > STACK_SIZE - 2;
-	if (sv.has_media) {
-		if (deep) tail_kernel<true, DEEP_STACK_SIZE><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold);
-		else tail_kernel<true, STACK_SIZE><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold);
+#define RTB_LAUNCH_TAIL(M, L) \
+	do { if (deep) tail_kernel<M, DEEP_STACK_SIZE, L><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); \
+	     else tail_kernel<M, STACK_SIZE, L><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); } while (0)
+	if (sv.n_lights > 0) {   // (light sampling: its own instantiations, so the kernels of scenes without it stay as they were)
+		if (sv.has_media) RTB_LAUNCH_TAIL(true, true);
+		else RTB_LAUNCH_TAIL(false, true);
 	} else {
-		if (deep) tail_kernel<false, DEEP_STACK_SIZE><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold);
-		else tail_kernel<false, STACK_SIZE><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold);
+		if (sv.has_media) RTB_LAUNCH_TAIL(true, false);
+		else RTB_LAUNCH_TAIL(false, false);
 	}
+#undef RTB_LAUNCH_TAIL
 }
 void launch_shade(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t bounce, int q, const LaunchCfg& lc, cudaStream_t st) {
-	shade_kernel<<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
+	if (sv.n_lights > 0) shade_kernel<true><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
+	else shade_kernel<false><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
 }
 void launch_texture(const SceneView& sv, const WaveView& wv, uint32_t bounce, int q_out, const LaunchCfg& lc, cudaStream_t st) {
 	const int blocks = lc.sms * 2 < lc.blocks_stream ? lc.sms * 2 : lc.blocks_stream;   // short work lists: a small grid keeps the launch cheap

@@ -33,6 +33,10 @@ struct SceneView {
 	// bounds, directions on a 2^dir_bits square of the octahedral map; 0 / 0 switches binning off.
 	float bin_min[3], bin_scale[3];   // cell coordinate = (o - bin_min) * bin_scale, clamped to [0, 2^org_bits)
 	int32_t bin_org_bits, bin_dir_bits;
+	// Sampled lights (DESIGN.md §5b): n_lights world-space records (4 x float4, SPHERE / QUAD layout), then n_lights
+	// float4 (type bits, quad area, 0, 0).  n_lights = 0: no light sampling (the kernels without it are launched).
+	const float4* lights;
+	int32_t n_lights;
 };
 
 // One batch = `samples_per_batch` consecutive samples of every pixel of the row range.

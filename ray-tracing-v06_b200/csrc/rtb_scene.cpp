@@ -17,6 +17,7 @@
 #include <cstring>
 #include <functional>
 #include <future>
+#include <string>
 #include <thread>
 
 #include "rtmath.h"
@@ -373,10 +374,13 @@ extern "C" int rtb_object_bounds(const rtb_scene* s, int object, float out6[6]) 
 
 extern "C" size_t rtb_scene_serialize(const rtb_scene* s, void* buf, size_t cap) {
 	if (!s) return 0;
+	// A scene without sampled lights is written as RTBS v1, byte for byte; one with them as v2 (the list appended).
+	const bool lights = !s->sampled_lights.empty();
 	size_t need = sizeof(rtbs_header) + s->textures.size() * sizeof(rtbs_texture) + s->materials.size() * sizeof(rtbs_material) +
-	              s->objects.size() * sizeof(rtbs_object) + s->children.size() * 4 + s->blob.size();
+	              s->objects.size() * sizeof(rtbs_object) + s->children.size() * 4 + s->blob.size() +
+	              (lights ? 4 + s->sampled_lights.size() * 4 : 0);
 	if (!buf || cap < need) return need;
-	rtbs_header h{}; h.magic = RTBS_MAGIC; h.version = RTBS_VERSION;
+	rtbs_header h{}; h.magic = RTBS_MAGIC; h.version = lights ? RTBS_VERSION_LIGHTS : RTBS_VERSION;
 	h.n_textures = (uint32_t)s->textures.size(); h.n_materials = (uint32_t)s->materials.size();
 	h.n_objects = (uint32_t)s->objects.size(); h.n_children = (uint32_t)s->children.size();
 	h.n_blob_bytes = (uint32_t)s->blob.size(); h.root_object = s->root; h.background_mode = s->background_mode;
@@ -389,6 +393,11 @@ extern "C" size_t rtb_scene_serialize(const rtb_scene* s, void* buf, size_t cap)
 	put(s->objects.data(), s->objects.size() * sizeof(rtbs_object));
 	put(s->children.data(), s->children.size() * 4);
 	put(s->blob.data(), s->blob.size());
+	if (lights) {
+		const int32_t n = (int32_t)s->sampled_lights.size();
+		put(&n, 4);
+		put(s->sampled_lights.data(), s->sampled_lights.size() * 4);
+	}
 	return need;
 }
 
@@ -861,6 +870,40 @@ struct Flattener {
 		return fail(RTB_ERR_INVALID, "unknown object kind");
 	}
 };
+
+// Sampled light `id` (DESIGN.md §5b): its translate / rotate_y chain composed into one world-from-object transform, the
+// sphere or quad at its end as a world-space record (the SPHERE / QUAD layout of DevPrim) and its DevLightInfo.
+int light_record(const rtb_scene& s, int id, DevPrim& rec, DevLightInfo& info) {
+	if (id < 0 || id >= (int)s.objects.size()) return fail(RTB_ERR_INVALID, "sampled light: bad object id " + std::to_string(id));
+	Xf x;
+	int cur = id;
+	for (int guard = 0; guard < 64; ++guard) {
+		const rtbs_object& o = s.objects[cur];
+		if (o.kind == RTB_OBJ_TRANSLATE) { x = Flattener::compose_translate(x, o.f); cur = s.children[o.child_begin]; continue; }
+		if (o.kind == RTB_OBJ_ROTATE_Y) { x = Flattener::compose_rotate(x, o.f[1], o.f[2]); cur = s.children[o.child_begin]; continue; }
+		rec = DevPrim{}; info = DevLightInfo{};
+		if (o.kind == RTB_OBJ_SPHERE) {
+			float c[3]; x.point(o.f, c);
+			const float r = std::fabs(o.f[3]);
+			if (!(r > 0.0f) || !std::isfinite(r)) return fail(RTB_ERR_INVALID, "sampled light " + std::to_string(id) + ": the sphere has no radius");
+			rec.q[0] = c[0]; rec.q[1] = c[1]; rec.q[2] = c[2]; rec.q[3] = r;
+			info.type = PRIM_SPHERE;
+			return RTB_OK;
+		}
+		if (o.kind == RTB_OBJ_QUAD) {
+			float Q[3], u[3], v[3]; x.point(o.f, Q); x.vec(o.f + 3, u); x.vec(o.f + 6, v);
+			rec = Flattener::planar_record(Q, u, v);
+			const rt::v3 n = rt::cross(rt::mk(u[0], u[1], u[2]), rt::mk(v[0], v[1], v[2]));
+			const float area = sqrtf(rt::dot(n, n));
+			if (!(area > 0.0f) || !std::isfinite(area)) return fail(RTB_ERR_INVALID, "sampled light " + std::to_string(id) + ": the quad has no area");
+			info.type = PRIM_QUAD; info.area = area;
+			return RTB_OK;
+		}
+		return fail(RTB_ERR_UNSUPPORTED, "sampled light " + std::to_string(id) +
+		                                     ": only spheres and quads (optionally under translate / rotate_y) can be sampled");
+	}
+	return fail(RTB_ERR_INVALID, "sampled light " + std::to_string(id) + ": instance chain too deep");
+}
 }  // namespace
 
 int flatten(rtb_scene& s, FlatScene& out, const GpuBuildContext* gpu) {
@@ -1055,6 +1098,12 @@ int flatten(rtb_scene& s, FlatScene& out, const GpuBuildContext* gpu) {
 		d.width = t.width; d.height = t.height; d.blob_offset = t.blob_offset; d.pad = 0;
 	}
 	out.blob = s.blob;
+	for (int id : s.sampled_lights) {
+		DevPrim rec; DevLightInfo info;
+		rc = light_record(s, id, rec, info);
+		if (rc) return rc;
+		out.lights.push_back(rec); out.light_info.push_back(info);
+	}
 	out.background_mode = s.background_mode;
 	memcpy(out.background, s.background, 12);
 	out.flatten_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_start).count();
@@ -1086,7 +1135,25 @@ extern "C" int rtb_scene_flatten_hash(rtb_scene* s, uint64_t* hash_out) {
 	if (!fs.prim_type.empty()) mix(fs.prim_type.data(), fs.prim_type.size() * sizeof(fs.prim_type[0]));
 	if (!fs.pre_list.empty()) mix(fs.pre_list.data(), fs.pre_list.size() * sizeof(fs.pre_list[0]));
 	mix(&fs.root_ref, sizeof fs.root_ref);
+	if (!fs.lights.empty()) {   // (only then: the hashes of scenes without sampled lights stay what they were)
+		mix(fs.lights.data(), fs.lights.size() * sizeof(rtb::DevPrim));
+		mix(fs.light_info.data(), fs.light_info.size() * sizeof(rtb::DevLightInfo));
+	}
 	*hash_out = h;
+	return RTB_OK;
+}
+
+extern "C" int rtb_scene_set_sampled_lights(rtb_scene* s, const int* objects, int n) {
+	if (!s) return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_sampled_lights: null scene");
+	if (n < 0 || n > RTB_MAX_SAMPLED_LIGHTS) return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_sampled_lights: n must be in [0, " + std::to_string(RTB_MAX_SAMPLED_LIGHTS) + "]");
+	if (n > 0 && !objects) return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_sampled_lights: null object list");
+	for (int i = 0; i < n; ++i) {   // validate everything first: a refused list leaves the scene as it was
+		rtb::DevPrim rec; rtb::DevLightInfo info;
+		const int rc = rtb::light_record(*s, objects[i], rec, info);
+		if (rc) return rc;
+	}
+	s->sampled_lights.assign(objects, objects + n);
+	s->version++;
 	return RTB_OK;
 }
 

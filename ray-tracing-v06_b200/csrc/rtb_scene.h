@@ -21,6 +21,7 @@ struct rtb_scene {
 	uint64_t uid = 0;       // unique per rtb_scene_create
 	uint64_t version = 0;   // bumped by every mutating call: lets a renderer skip re-flattening an unchanged scene
 	float background[3] = {0, 0, 0};
+	std::vector<int32_t> sampled_lights;   // rtb_scene_set_sampled_lights: object ids (empty: no light sampling)
 
 	// Filled by flatten(): the world BVH in the reference's node layout (parity hook).
 	std::vector<rtb_bvh_node> world_nodes;

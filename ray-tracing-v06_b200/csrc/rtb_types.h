@@ -53,6 +53,10 @@ struct alignas(64) DevPrim { float q[16]; };
 
 struct alignas(8) DevPrimInfo { int32_t material; int32_t object; };
 
+// Light table of a scene with sampled lights (DESIGN.md §5b): one world-space DevPrim per light (SPHERE or QUAD record
+// layout), then one DevLightInfo per light.
+struct alignas(16) DevLightInfo { int32_t type; float area; float pad0, pad1; };   // PRIM_SPHERE / PRIM_QUAD; quad area
+
 struct alignas(16) DevMaterial { int32_t kind, tex; float param, pad; float albedo[4]; };  // 32 B
 
 struct alignas(16) DevTexture {                                                             // 48 B
@@ -73,6 +77,8 @@ struct FlatScene {
 	std::vector<DevMaterial> materials;
 	std::vector<DevTexture> textures;
 	std::vector<uint8_t> blob;
+	std::vector<DevPrim> lights;         // sampled lights in world space (empty: no light sampling)
+	std::vector<DevLightInfo> light_info;
 	int32_t n_media = 0;
 	int32_t background_mode = 0;
 	float background[3] = {0, 0, 0};

@@ -84,7 +84,7 @@ RT_HD u4 philox4x32_10(u4 c, uint32_t k0, uint32_t k1) {
 RT_HD float uniform01(uint32_t x) { return fmaf((float)x, 2.3283064365386963e-10f, 1.1641532182693481e-10f); }
 
 // Stream ids (counter word z)
-enum { STREAM_SCATTER = 0, STREAM_LENS = 1, STREAM_MEDIUM0 = 16 };
+enum { STREAM_SCATTER = 0, STREAM_LENS = 1, STREAM_LIGHT = 2, STREAM_MEDIUM0 = 16 };
 #define RT_CAMERA_BOUNCE 0xFFFFFFFFu
 
 struct f4 { float x, y, z, w; };
@@ -158,6 +158,35 @@ RT_HD void unit_disc(float u0, float u1, float& dx, float& dy) {
 	float r = sqrtf(u0);
 	float s, c; sincos2pi(u1, s, c);
 	dx = r * c; dy = r * s;
+}
+
+// ---------------------------------------------------------------- light sampling (DESIGN.md §5b)
+#define RT_INV_PI 0.31830988618379067f
+#define RT_INV_4PI 0.07957747154594767f
+#define RT_2PI 6.28318530717958647692f
+
+// cos of the half-angle of the cone a sphere of squared radius R2 subtends from squared distance d2 (> R2)
+RT_HD float cone_cos_max(float d2, float R2) { return sqrtf(1.0f - R2 / d2); }
+// Book 3 sphere::pdf_value: 1 / solid angle of that cone
+RT_HD float cone_pdf(float cmax) { return 1.0f / (RT_2PI * (1.0f - cmax)); }
+// Book 3 random_to_sphere in the orthonormal basis around e = centre - p (d2 = dot(e, e) > R2): a unit direction
+// uniform in the cone, from the uniforms (u0 azimuth, u1 height).
+RT_HD v3 cone_direction(v3 e, float cmax, float u0, float u1) {
+	const float z = fmaf(u1, cmax - 1.0f, 1.0f);
+	const float z2 = fmaf(-z, z, 1.0f);
+	const float sz = sqrtf(z2 < 0.0f ? 0.0f : z2);
+	float sn, cs; sincos2pi(u0, sn, cs);
+	const float x = cs * sz, y = sn * sz;
+	const v3 W = normalize(e);
+	const v3 A = fabsf(W.x) > 0.9f ? mk(0.0f, 1.0f, 0.0f) : mk(1.0f, 0.0f, 0.0f);
+	const v3 V = normalize(cross(W, A));
+	const v3 U = cross(W, V);
+	return normalize(mk(fmaf(z, W.x, fmaf(y, V.x, x * U.x)), fmaf(z, W.y, fmaf(y, V.y, x * U.y)), fmaf(z, W.z, fmaf(y, V.z, x * U.z))));
+}
+// Weight of a direction drawn from the half-and-half mixture: scattering pdf / mixture pdf (<= 0: the path ends black)
+RT_HD float mixture_weight(float spdf, float lpdf) {
+	const float mix = fmaf(0.5f, lpdf, 0.5f * spdf);
+	return mix > 0.0f ? spdf / mix : 0.0f;
 }
 
 }  // namespace rt

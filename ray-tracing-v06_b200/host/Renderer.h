@@ -12,7 +12,9 @@
 #include <glm/glm.hpp>
 #include <stdexcept>
 #include <string>
+#include <vector>
 
+#include "rt_engine/geometry/HittableList.cuh"
 #include "rt_engine/geometry/hittable.cuh"
 #include "rt_engine/shaders/cu_Cameras.cuh"
 #include "rtb_context.h"
@@ -74,6 +76,17 @@ public:
 	static Renderer MakeRenderer(uint32_t render_width, uint32_t render_height, uint32_t samples_per_pixel, uint32_t max_depth,
 	                             const PinholeCamera* cam, const Hittable* d_world_ptr) {
 		M m{}; m.pinhole_cam = cam; return _make(render_width, render_height, samples_per_pixel, max_depth, d_world_ptr, m);
+	}
+	// Book 3's cam.render(world, lights): the same renderer with light importance sampling towards `lights` - a HittableList
+	// of spheres / quads (each optionally under translate / rotate_y), or one such object (rtb_scene_set_sampled_lights).
+	template <typename Cam>
+	static Renderer MakeRenderer(uint32_t render_width, uint32_t render_height, uint32_t samples_per_pixel, uint32_t max_depth,
+	                             const Cam* cam, const Hittable* d_world_ptr, const Hittable* lights) {
+		std::vector<int> ids;
+		if (const HittableList* l = dynamic_cast<const HittableList*>(lights)) ids = l->memberIds();
+		else if (lights) ids.push_back(lights->rtb_object);
+		rtb_host::check(rtb_scene_set_sampled_lights(rtb_host::scene(), ids.data(), (int)ids.size()), "rtb_scene_set_sampled_lights");
+		return MakeRenderer(render_width, render_height, samples_per_pixel, max_depth, cam, d_world_ptr);
 	}
 
 	void Render() {

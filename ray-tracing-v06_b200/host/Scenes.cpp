@@ -17,6 +17,7 @@
 #include <unistd.h>
 #include <cstring>
 #include <functional>
+#include <initializer_list>
 #include <map>
 #include <memory>
 #include <string>
@@ -198,11 +199,17 @@ struct Keep {
 	}
 };
 
-void finish(rtb_scene_info* info, const Hittable* world, const rtb_camera& cam, int w, int h, int spp, int depth, bool black_background) {
+// `lights`: the emitters a user would hand to light sampling (rtb_scene_info::lights); they are only listed, not set.
+void finish(rtb_scene_info* info, const Hittable* world, const rtb_camera& cam, int w, int h, int spp, int depth, bool black_background,
+            std::initializer_list<const Hittable*> lights = {}) {
 	rtb_host::check(rtb_scene_set_root(rtb_host::scene(), world->rtb_object), "rtb_scene_set_root");
 	const float black[3] = {0, 0, 0};
 	rtb_host::check(rtb_scene_set_background(rtb_host::scene(), black_background ? RTB_BG_CONSTANT : RTB_BG_SKY_GRADIENT, black), "rtb_scene_set_background");
-	if (info) { info->camera = cam; info->width = w; info->height = h; info->spp = spp; info->max_depth = depth; }
+	if (info) {
+		info->camera = cam; info->width = w; info->height = h; info->spp = spp; info->max_depth = depth;
+		info->n_lights = 0;
+		for (const Hittable* l : lights) if (info->n_lights < 8) info->lights[info->n_lights++] = l->rtb_object;
+	}
 }
 
 rtb_camera book2_camera(glm::vec3 from, glm::vec3 at, float vfov, float aspect) {
@@ -302,7 +309,7 @@ void build_book2_simple_light(rtb_scene_info* info) {
 	auto light = k.mat(new diffuse_light(glm::vec3(4, 4, 4)));
 	std::vector<const Hittable*> objs{k.sphere(Sphere(glm::vec3(0, -1000, 0), 1000), m), k.sphere(Sphere(glm::vec3(0, 2, 0), 2), m),
 	                                  k.sphere(Sphere(glm::vec3(0, 7, 0), 2), light), k.quad(glm::vec3(3, 1, -2), glm::vec3(2, 0, 0), glm::vec3(0, 2, 0), light)};
-	finish(info, k.list(objs), book2_camera(glm::vec3(26, 3, 6), glm::vec3(0, 2, 0), 20.0f, 400.0f / 225.0f), 400, 225, 100, 50, true);
+	finish(info, k.list(objs), book2_camera(glm::vec3(26, 3, 6), glm::vec3(0, 2, 0), 20.0f, 400.0f / 225.0f), 400, 225, 100, 50, true, {objs[2], objs[3]});
 }
 
 void cornell_walls(Keep& k, std::vector<const Hittable*>& objs, glm::vec3 light_q, glm::vec3 light_u, glm::vec3 light_v, glm::vec3 emit) {
@@ -324,7 +331,7 @@ void build_book2_cornell(rtb_scene_info* info) {
 	auto white = k.mat(new Lambertian(glm::vec3(.73f, .73f, .73f)));
 	objs.push_back(k.translate(k.rotate_y(k.box(glm::vec3(0, 0, 0), glm::vec3(165, 330, 165), white), 15.0f), glm::vec3(265, 0, 295)));
 	objs.push_back(k.translate(k.rotate_y(k.box(glm::vec3(0, 0, 0), glm::vec3(165, 165, 165), white), -18.0f), glm::vec3(130, 0, 65)));
-	finish(info, k.list(objs), book2_camera(glm::vec3(278, 278, -800), glm::vec3(278, 278, 0), 40.0f, 1.0f), 600, 600, 200, 50, true);
+	finish(info, k.list(objs), book2_camera(glm::vec3(278, 278, -800), glm::vec3(278, 278, 0), 40.0f, 1.0f), 600, 600, 200, 50, true, {objs[2]});
 }
 
 // Config 4 — Cornell box, the two rotated boxes as smoke / fog
@@ -336,7 +343,7 @@ void build_book2_cornell_smoke(rtb_scene_info* info) {
 	auto box2 = k.translate(k.rotate_y(k.box(glm::vec3(0, 0, 0), glm::vec3(165, 165, 165), white), -18.0f), glm::vec3(130, 0, 65));
 	objs.push_back(k.medium(box1, 0.01f, k.mat(new isotropic(glm::vec3(0, 0, 0)))));
 	objs.push_back(k.medium(box2, 0.01f, k.mat(new isotropic(glm::vec3(1, 1, 1)))));
-	finish(info, k.list(objs), book2_camera(glm::vec3(278, 278, -800), glm::vec3(278, 278, 0), 40.0f, 1.0f), 600, 600, 1000, 50, true);
+	finish(info, k.list(objs), book2_camera(glm::vec3(278, 278, -800), glm::vec3(278, 278, 0), 40.0f, 1.0f), 600, 600, 1000, 50, true, {objs[2]});
 }
 
 // Config 5 — Book 2 final scene.  Random draws from cuHostRND(512, 1984), one per statement.
@@ -386,7 +393,7 @@ void build_book2_final(rtb_scene_info* info) {
 	}
 	world.push_back(k.translate(k.rotate_y(k.bvh(boxes2), 15.0f), glm::vec3(-100, 270, 395)));
 
-	finish(info, k.list(world), book2_camera(glm::vec3(478, 278, -600), glm::vec3(278, 278, 0), 40.0f, 1.0f), 800, 800, 10000, 40, true);
+	finish(info, k.list(world), book2_camera(glm::vec3(478, 278, -600), glm::vec3(278, 278, 0), 40.0f, 1.0f), 800, 800, 10000, 40, true, {world[1]});
 }
 
 // A procedural triangle mesh (a subdivided icosahedron, 1,280 faces) written to and read back through the OBJ

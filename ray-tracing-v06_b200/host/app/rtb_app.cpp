@@ -3,7 +3,7 @@
 // build the camera, build the scene, MakeRenderer, Render, DownloadRenderbuffer, write the image.
 //
 //   rtb_app [scene] [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--gpus N]
-//           [--out image.png|image.ppm|image.pfm] [--resume ckpt.rtba] [--checkpoint ckpt.rtba]
+//           [--out image.png|image.ppm|image.pfm] [--resume ckpt.rtba] [--checkpoint ckpt.rtba] [--sample-lights]
 //   rtb_app --obj model.obj [...]     a Wavefront OBJ mesh (MeshHandle) on a checkered floor under the sky
 //
 // scene = one of rtb_scenes_name(i) (default book2_bouncing, which goes through SceneBook2BVH::Factory
@@ -12,6 +12,8 @@
 // (FirstApp.cpp:108-122) - uint8 = value * 255.999f, RGB, rows flipped (row 0 of the float buffer is the bottom of the
 // image) - and is quantised on the device; .png / .ppm carry it, .pfm keeps the raw floats.  --checkpoint saves the
 // radiance sums after the render; --resume loads such a file and renders --spp MORE samples on top of it (single GPU).
+// --sample-lights turns on light importance sampling (rtb_scene_set_sampled_lights) towards the emitters the named scene
+// lists (rtb_scene_info::lights): the same converged image with less noise per sample; refused for scenes that list none.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -40,6 +42,7 @@ static bool write_image(const std::string& path, uint32_t width, uint32_t height
 int main(int argc, char** argv) {
 	std::string scene_name = "book2_bouncing", out = "render.ppm", obj_path, resume_path, checkpoint_path;
 	int width = 0, height = 0, spp = 0, depth = 0, gpus = 0;
+	bool sample_lights = false;
 	uint32_t seed = 1984;   // the reference's seed (Renderer.cu:51, Scenes.cu:190)
 	for (int i = 1; i < argc; ++i) {
 		std::string a = argv[i];
@@ -54,8 +57,13 @@ int main(int argc, char** argv) {
 		else if (a == "--checkpoint" && i + 1 < argc) checkpoint_path = argv[++i];
 		else if (a == "--out" && i + 1 < argc) out = argv[++i];
 		else if (a == "--obj" && i + 1 < argc) obj_path = argv[++i];
+		else if (a == "--sample-lights") sample_lights = true;
 		else if (a == "--list") { for (int k = 0; k < rtb_scenes_count(); ++k) printf("%s\n", rtb_scenes_name(k)); return 0; }
 		else scene_name = a;
+	}
+	if (sample_lights && (!obj_path.empty() || scene_name == "book2_bouncing")) {
+		fprintf(stderr, "rtb_app: --sample-lights: %s lists no lights to sample\n", obj_path.empty() ? scene_name.c_str() : obj_path.c_str());
+		return 1;
 	}
 	if (gpus > 1) Renderer::UseGpus(gpus);
 	try {
@@ -104,6 +112,11 @@ int main(int argc, char** argv) {
 			rtb_scene_info info{};
 			rtb_scene* s = rtb_scenes_build(scene_name.c_str(), &info);
 			if (!s) { fprintf(stderr, "rtb_app: %s\n", rtb_scenes_last_error()); return 1; }
+			if (sample_lights) {
+				if (info.n_lights == 0) { fprintf(stderr, "rtb_app: --sample-lights: %s lists no lights to sample\n", scene_name.c_str()); rtb_scene_destroy(s); return 1; }
+				rtb_host::check(rtb_scene_set_sampled_lights(s, info.lights, info.n_lights), "rtb_scene_set_sampled_lights");
+				printf("Sampling %d light%s.\n", info.n_lights, info.n_lights > 1 ? "s" : "");
+			}
 			if (!width) width = info.width;
 			if (!height) height = info.height;
 			rtb_render_params p{};

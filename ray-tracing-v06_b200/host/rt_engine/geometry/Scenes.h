@@ -47,6 +47,9 @@ extern "C" {
 typedef struct rtb_scene_info {
 	rtb_camera camera;
 	int32_t width, height, spp, max_depth;
+	// The scene's emitters as its author names them for light sampling (Book 3's `lights` list): pass them to
+	// rtb_scene_set_sampled_lights to turn it on.  The named scenes never do that themselves.
+	int32_t n_lights, lights[8];
 } rtb_scene_info;
 
 int rtb_scenes_count(void);
