@@ -272,6 +272,40 @@ int  rtb_load_accum(rtb_renderer* r, const char* path, uint32_t* width_out, uint
 uint32_t rtb_renderer_sample_cursor(const rtb_renderer* r);
 int  rtb_get_counters(rtb_renderer* r, rtb_counters* out);
 
+/* Adaptive sampling (DESIGN.md §5c): rounds of samples for the pixels whose estimated display-space error is still above
+ * `tolerance`, until none is, every remaining one has p->sample_end samples, or max_rounds rounds have run.
+ *
+ * A pixel's error e is one standard error of its mean, taken through the clamp and square root of rtb_resolve; a pixel is
+ * rendered in the next round while the maximum of e over its 3x3 neighbourhood (clipped to the row range) is above the
+ * tolerance, and it has taken part in every round so far.  Every pixel first gets min_spp samples.  A stopped pixel never
+ * resumes, so an active pixel always holds samples [0, cursor) - the same sums, bit for bit, that a uniform render of
+ * `cursor` samples per pixel holds for it.  The decision is a pure function of the accumulators: a render continued in
+ * another call, or from a loaded checkpoint, goes on exactly as the uninterrupted one.  tolerance = 10^(-D/20) leaves the
+ * image about D dB from its converged value.
+ *
+ * p->sample_begin must be 0; p->sample_end is the cap (min_spp <= cap <= 2^24).  RTB_RENDER_CLEAR starts from zero; without
+ * it the call continues from what the accumulators hold (a render from sample 0 with RTB_RENDER_VARIANCE, an earlier
+ * adaptive call, a checkpoint).  Sums of squares are always accumulated.  Rows outside the row range are untouched.
+ * The call blocks (it reads the number of active pixels once per round) and is ordered after and before `stream` as
+ * rtb_render is; rtb_get_counters reports the device time of the whole call and its paths and rays.  Returns
+ * RTB_ERR_INVALID for bad arguments, RTB_ERR_STATE when continuing an accumulator of another size, or one in which a pixel
+ * holding the cursor's samples has no sums of squares (a render without RTB_RENDER_VARIANCE), whatever the cursor.  After
+ * an error the sample cursor still covers the rounds rendered, and the call is ordered before `stream` as on success. */
+typedef struct rtb_adaptive_params {
+	float    tolerance;    /* display-space standard error at which a pixel stops (DESIGN.md §5c); >= 0, finite */
+	uint32_t min_spp;      /* every pixel gets at least this many samples; >= 2 */
+	uint32_t max_rounds;   /* 0 = until no pixel is active or every active pixel has p->sample_end samples */
+	uint32_t reserved;
+} rtb_adaptive_params;
+typedef struct rtb_adaptive_stats {
+	uint32_t rounds, cursor;   /* rounds run by this call; sample cursor after it */
+	uint32_t active_pixels;    /* pixels the next round would render (0 = done) */
+	uint32_t reserved;
+	uint64_t samples;          /* camera paths started by this call */
+} rtb_adaptive_stats;
+int  rtb_render_adaptive(rtb_renderer* r, const rtb_render_params* p, const rtb_adaptive_params* a,
+                         rtb_adaptive_stats* out, void* stream);
+
 /* Per-kernel-class device time, measured with CUDA events around every launch on the stream the
  * kernels run on.  Profiling renders run as plain stream launches (no CUDA graph) and are meant for
  * the roofline accounting of bench.py, not for the headline timing. */
@@ -287,7 +321,7 @@ int  rtb_renderer_set_profiling(rtb_renderer* r, int on);
 int  rtb_get_profile(rtb_renderer* r, rtb_profile* out);   /* synchronizes; totals since the last call */
 /* The individual launches behind rtb_get_profile, in launch order (call it BEFORE rtb_get_profile, which resets):
  * ms_out[i] = device time, class_out[i] = 0 generate, 1 traverse, 2 shade (+ texture), 3 accumulate, 4 tail check,
- * 5 ray binning.
+ * 5 ray binning, 6 the select step of an adaptive round (rtb_render_adaptive; not in rtb_get_profile's totals).
  * Returns the number of launches recorded (may exceed cap). */
 int  rtb_get_profile_launches(rtb_renderer* r, float* ms_out, int32_t* class_out, int cap);
 int  rtb_reset_counters(rtb_renderer* r);

@@ -34,7 +34,7 @@ BUILDER_NAMES = {0: "host_sah", 1: "as_built", 2: "gpu_lbvh", 3: "host_median_fa
 CAM_PINHOLE, CAM_DEFOCUS, CAM_MOTION = 0, 1, 2
 RENDER_CLEAR, RENDER_VARIANCE = 1, 2
 REDUCE_AUTO, REDUCE_NCCL, REDUCE_P2P = 0, 1, 2
-PROFILE_CLASSES = {0: "generate", 1: "traverse", 2: "shade", 3: "accumulate", 4: "tail", 5: "bin"}
+PROFILE_CLASSES = {0: "generate", 1: "traverse", 2: "shade", 3: "accumulate", 4: "tail", 5: "bin", 6: "adaptive_select"}
 MISS_DIST = np.float32(3.402823466e38)
 
 
@@ -66,6 +66,20 @@ class RenderParams(C.Structure):
 
 class Counters(C.Structure):
     _fields_ = [("paths", C.c_uint64), ("rays", C.c_uint64), ("launches", C.c_uint64), ("batches", C.c_uint64), ("render_ms", C.c_double)]
+
+
+class AdaptiveParams(C.Structure):
+    _fields_ = [("tolerance", C.c_float), ("min_spp", C.c_uint32), ("max_rounds", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class AdaptiveStats(C.Structure):
+    _fields_ = [("rounds", C.c_uint32), ("cursor", C.c_uint32), ("active_pixels", C.c_uint32), ("reserved", C.c_uint32), ("samples", C.c_uint64)]
+
+
+def tolerance_for_db(db: float) -> float:
+    """Adaptive-sampling tolerance for a PSNR target (DESIGN.md §5c): 10^(-D/20).  When every pixel meets it, the image is
+    about D dB from its converged value; two independent renders at that target are about D - 3 dB apart."""
+    return float(10.0 ** (-float(db) / 20.0))
 
 
 class SceneStats(C.Structure):
@@ -154,6 +168,7 @@ ABI = {
     "rtb_download": (C.c_int, [_P, _P]),
     "rtb_download_accum": (C.c_int, [_P, _P, _P]),
     "rtb_get_counters": (C.c_int, [_P, C.POINTER(Counters)]),
+    "rtb_render_adaptive": (C.c_int, [_P, C.POINTER(RenderParams), C.POINTER(AdaptiveParams), C.POINTER(AdaptiveStats), _P]),
     "rtb_reset_counters": (C.c_int, [_P]),
     "rtb_queue_lengths": (C.c_int, [_P, _P, C.c_int]),
     "rtb_renderer_set_profiling": (C.c_int, [_P, C.c_int]),
@@ -413,6 +428,24 @@ class Renderer:
                          (RENDER_CLEAR if clear else 0) | (RENDER_VARIANCE if variance else 0), samples_per_batch)
         _check(lib().rtb_render(self.handle, C.byref(p), stream), "rtb_render")
         self.width, self.height = width, height
+
+    def render_adaptive(self, width, height, max_spp, max_depth, *, tolerance=None, target_db=None, min_spp=64, max_rounds=0,
+                        seed=1984, clear=True, rows=(0, 0), samples_per_batch=0, stream=None) -> dict:
+        """Adaptive sampling (rtb_render_adaptive, DESIGN.md §5c): rounds of samples for the pixels whose display-space
+        standard error (maximum over their 3x3 neighbourhood) is above `tolerance` - or tolerance_for_db(target_db) - after
+        at least min_spp samples, up to max_spp.  Blocks.  Without `clear` it continues from what the accumulators hold.
+        Returns the call's rounds, sample cursor, active pixels left and camera paths; per-pixel counts are in
+        download_accum()[..., 3]."""
+        if (tolerance is None) == (target_db is None):
+            raise ValueError("render_adaptive: give exactly one of tolerance and target_db")
+        tol = float(tolerance) if tolerance is not None else tolerance_for_db(target_db)
+        p = RenderParams(width, height, 0, max_spp, rows[0], rows[1], max_depth, seed,
+                         (RENDER_CLEAR if clear else 0) | RENDER_VARIANCE, samples_per_batch)
+        a = AdaptiveParams(tol, min_spp, max_rounds, 0)
+        st = AdaptiveStats()
+        _check(lib().rtb_render_adaptive(self.handle, C.byref(p), C.byref(a), C.byref(st), stream), "rtb_render_adaptive")
+        self.width, self.height = width, height
+        return {"rounds": int(st.rounds), "cursor": int(st.cursor), "active_pixels": int(st.active_pixels), "samples": int(st.samples)}
 
     def synchronize(self):
         _check(lib().rtb_synchronize(self.handle), "rtb_synchronize")

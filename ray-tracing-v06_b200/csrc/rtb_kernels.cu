@@ -113,13 +113,24 @@ __device__ __forceinline__ BatchParams with_call_params(const BatchParams& in, c
 	return bp;
 }
 
+// Local pixel -> global pixel of an adaptive round: entry pl of the list, which holds pixels of the row range
+// [first, first + count) and is at most `count` long.
+__device__ __forceinline__ uint32_t listed_pixel(const uint32_t* list, uint32_t pl, uint32_t first, uint32_t count) {
+	RTB_CHECK(pl < count, RTB_BOUNDS_PATH);
+	const uint32_t p = __ldg(list + pl);
+	RTB_CHECK(p - first < count, RTB_BOUNDS_PATH);
+	return p;
+}
+
 // Path id -> (global pixel index, absolute sample index).  Paths of a batch are laid out
-// sample-major: id = local_sample * npix + local_pixel, local pixels row-major from row_begin.
+// sample-major: id = local_sample * npix + local_pixel, local pixels row-major from row_begin
+// (LIST: local pixel pl is bp.pixel_list[pl]).
+template <bool LIST = false>
 __device__ __forceinline__ void path_pixel_sample(const BatchParams& bp, uint32_t batch, uint32_t path,
                                                   uint32_t& pixel, uint32_t& sample) {
 	uint32_t sl = path / bp.npix;
 	uint32_t pl = path - sl * bp.npix;
-	pixel = bp.row_begin * bp.width + pl;
+	pixel = LIST ? listed_pixel(bp.pixel_list(), pl, bp.row_begin * bp.width, bp.n_rows * bp.width) : bp.row_begin * bp.width + pl;
 	sample = bp.sample_begin + batch * bp.samples_per_batch + sl;
 }
 
@@ -133,6 +144,7 @@ __device__ __forceinline__ uint32_t batch_sample_count(const BatchParams& bp, ui
 // ------------------------------------------------------------------------------------------------
 // generate
 
+template <bool LIST>
 __global__ void __launch_bounds__(STREAM_THREADS)
 generate_kernel(BatchParams bp_in, rtb_camera cam, WaveView wv) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -153,7 +165,7 @@ generate_kernel(BatchParams bp_in, rtb_camera cam, WaveView wv) {
 	const float px = 1.0f / (float)bp.width, py = 1.0f / (float)bp.height;   // pixel_size  Renderer.cu:188
 	for (uint32_t path = tid; path < n; path += stride) {
 		uint32_t pixel, sample;
-		path_pixel_sample(bp, batch, path, pixel, sample);
+		path_pixel_sample<LIST>(bp, batch, path, pixel, sample);
 		uint32_t y = pixel / bp.width, x = pixel - y * bp.width;
 		rt::f4 r = rt::rng4(bp.seed, pixel, sample, RT_CAMERA_BOUNCE, rt::STREAM_SCATTER);
 		// ndc = (vec2(x,y) + 0.5) * pixel_size * 2 - 1 ; jitter = point in unit disc * pixel_size   Renderer.cu:192,199
@@ -269,8 +281,11 @@ __device__ __forceinline__ float box_hit(v3 o, v3 d, float idx, float idy, float
 // Free-flight uniforms of the media a ray meets.  Medium m of a path segment uses component (m & 3)
 // of Philox(seed, pixel; sample, bounce, STREAM_MEDIUM0 + (m >> 2)); the block is generated lazily,
 // only when some medium's boundary interval survives the geometric rejections, and shared by up to
-// four media.
-struct MediumRng {
+// four media.  LIST: the batch is an adaptive round, and the pixel is gathered from its list - lazily too.
+template <bool LIST> struct MediumRngList {};
+template <> struct MediumRngList<true> { const uint32_t* list; uint32_t range; };   // the pixel list; pixels of the row range
+template <bool LIST>
+struct MediumRngT : MediumRngList<LIST> {
 	uint32_t seed, path, bounce;
 	uint32_t npix, pixel0, sample0;   // batch layout (warp-uniform): the path's pixel and sample are only worked out
 	                                  // (an integer division) when a block of uniforms is actually drawn
@@ -280,20 +295,27 @@ struct MediumRng {
 		const uint32_t b = m >> 2;
 		if (b != block) {
 			const uint32_t sl = path / npix, pl = path - sl * npix;      // path_pixel_sample
-			u = rt::rng4(seed, pixel0 + pl, sample0 + sl, bounce, rt::STREAM_MEDIUM0 + b); block = b;
+			uint32_t pixel;
+			if constexpr (LIST) pixel = listed_pixel(this->list, pl, pixel0, this->range);
+			else pixel = pixel0 + pl;
+			u = rt::rng4(seed, pixel, sample0 + sl, bounce, rt::STREAM_MEDIUM0 + b); block = b;
 		}
 		const uint32_t c = m & 3u;
 		return c == 0 ? u.x : (c == 1 ? u.y : (c == 2 ? u.z : u.w));
 	}
 };
-__device__ __forceinline__ MediumRng make_medium_rng(const BatchParams& bp, uint32_t batch, uint32_t path, uint32_t bounce) {
-	MediumRng r; r.seed = bp.seed; r.path = path; r.bounce = bounce; r.block = 0xFFFFFFFFu;
+using MediumRng = MediumRngT<false>;
+template <bool LIST = false>
+__device__ __forceinline__ MediumRngT<LIST> make_medium_rng(const BatchParams& bp, uint32_t batch, uint32_t path, uint32_t bounce) {
+	MediumRngT<LIST> r; r.seed = bp.seed; r.path = path; r.bounce = bounce; r.block = 0xFFFFFFFFu;
 	r.npix = bp.npix; r.pixel0 = bp.row_begin * bp.width; r.sample0 = bp.sample_begin + batch * bp.samples_per_batch;
+	if constexpr (LIST) { r.list = bp.pixel_list(); r.range = bp.n_rows * bp.width; }
 	r.u.x = r.u.y = r.u.z = r.u.w = 0.0f; return r;
 }
 
 // constant_medium::hit (book) over a convex boundary interval [t1,t2] found for any-sign t.
-__device__ __forceinline__ float medium_sample(float t1, float t2, float a, float neg_inv_density, MediumRng& mr, uint32_t medium, float tbest) {
+template <class MR>
+__device__ __forceinline__ float medium_sample(float t1, float t2, float a, float neg_inv_density, MR& mr, uint32_t medium, float tbest) {
 	if (!(t2 > t1 + 0.0001f)) return FLT_MAX;     // second boundary query: interval(t1 + 0.0001, inf)
 	if (t1 < 0.0f) t1 = 0.0f;                     // ray_t.min (the reference accepts t >= 0)
 	if (t2 > tbest) t2 = tbest;                   // ray_t.max = closest so far
@@ -305,7 +327,8 @@ __device__ __forceinline__ float medium_sample(float t1, float t2, float a, floa
 	return t1 + hit_distance / len;
 }
 
-__device__ __forceinline__ float medium_sphere_hit(v3 o, v3 d, float a, float4 q0, float nid, MediumRng& mr, uint32_t medium, float tbest) {
+template <class MR>
+__device__ __forceinline__ float medium_sphere_hit(v3 o, v3 d, float a, float4 q0, float nid, MR& mr, uint32_t medium, float tbest) {
 	v3 oc = rt::sub(o, xyz(q0));
 	float hb = rt::dot(d, oc);
 	float cc = fmaf(-q0.w, q0.w, rt::dot(oc, oc));
@@ -315,7 +338,8 @@ __device__ __forceinline__ float medium_sphere_hit(v3 o, v3 d, float a, float4 q
 	return medium_sample((-hb - sq) / a, (-hb + sq) / a, a, nid, mr, medium, tbest);
 }
 
-__device__ __forceinline__ float medium_box_hit(v3 o, v3 d, float a, float4 q0, float4 q1, float4 q2, MediumRng& mr, uint32_t medium, float tbest) {
+template <class MR>
+__device__ __forceinline__ float medium_box_hit(v3 o, v3 d, float a, float4 q0, float4 q1, float4 q2, MR& mr, uint32_t medium, float tbest) {
 	// world -> object: translate back, rotate by -theta about y (book translate::hit / rotate_y::hit)
 	float cs = q0.w, sn = q1.w;
 	v3 ot = rt::sub(o, xyz(q2));
@@ -371,8 +395,8 @@ __device__ __forceinline__ float slab_dir(float d) { return fabsf(d) < 1e-20f ? 
 #ifndef RTB_UNIFIED_LEAF
 #define RTB_UNIFIED_LEAF 1
 #endif
-template <bool MEDIA>
-__device__ __forceinline__ float leaf_test(const SceneView& sv, int code, v3 o, v3 d, float a, float time, MediumRng& mr, float tbest,
+template <bool MEDIA, class MR>
+__device__ __forceinline__ float leaf_test(const SceneView& sv, int code, v3 o, v3 d, float a, float time, MR& mr, float tbest,
                                            const RaySlab& rs, int& hit_code) {
 	hit_code = code;
 	const int type = code & 15;
@@ -470,8 +494,8 @@ __device__ __forceinline__ float leaf_test(const SceneView& sv, int code, v3 o, 
 
 // MEDIA: 0 = the scene has no media; 1 = all of them are in the pre-test list (the walk itself never meets
 // one: no RNG state is carried through the loop); 2 = more than the list holds, the rest are BVH leaves.
-template <int MEDIA, bool STATS = false>
-__device__ __forceinline__ void trace_ray(const SceneView& sv, v3 o, v3 d, float time, MediumRng& mr,
+template <int MEDIA, bool STATS = false, class MR>
+__device__ __forceinline__ void trace_ray(const SceneView& sv, v3 o, v3 d, float time, MR& mr,
                                           int* __restrict__ stack, int stack_cap, float& tbest_out, int& code_out, int* stats_out = nullptr) {
 	const float a = rt::dot(d, d);
 	float tbest = FLT_MAX;
@@ -606,7 +630,8 @@ __device__ __forceinline__ void trace_ray(const SceneView& sv, v3 o, v3 d, float
 #endif
 // STACK = entries of the per-thread stack in shared memory: 16 when the tree is shallow enough (8 KB per
 // block instead of 16 KB leaves 64 KB more L1 per SM: -2 % on the Book 2 final scene), 32 otherwise.
-template <int MEDIA, int STACK>
+// LIST (adaptive rounds, media only: without media the walk never derives a pixel): the media RNG gathers the pixel.
+template <int MEDIA, int STACK, bool LIST>
 __global__ void __launch_bounds__(TRAVERSE_THREADS, TRAVERSE_MIN_BLOCKS)
 traverse_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int q) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -628,7 +653,7 @@ traverse_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, i
 		const uint32_t i = base + lane;
 		if (i < n) {
 			float4 fo, fd; ld_ray(rod + 2 * (size_t)i, fo, fd);
-			MediumRng mr = make_medium_rng(bp, batch, __float_as_uint(fd.w), bounce);
+			MediumRngT<LIST> mr = make_medium_rng<LIST>(bp, batch, __float_as_uint(fd.w), bounce);
 			float t; int code;
 			trace_ray<MEDIA>(sv, xyz(fo), xyz(fd), fo.w, mr, s_stack + threadIdx.x, STACK, t, code);
 			RTB_CHECK(i < wv.capacity, RTB_BOUNDS_QUEUE);
@@ -907,7 +932,7 @@ __device__ __forceinline__ v3 background(const SceneView& sv, v3 d) {
 // been written to contrib[path].
 struct DeferredTex { int tex; float u, v; v3 p; };
 
-template <bool DEFER, bool LIGHTS>
+template <bool DEFER, bool LIGHTS, bool LIST>
 __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t batch, uint32_t bounce,
                                               const float4& fo, const float4& fd, v3 thr, float t, int code,
                                               float4& no, float4& nd, v3& nthr, DeferredTex& dt) {
@@ -927,7 +952,7 @@ __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchPa
 	Surface s;
 	reconstruct(sv, code, o, d, fo.w, t, texture_needs_uv(sv, tex), s);
 	uint32_t pixel, sample;
-	path_pixel_sample(bp, batch, path, pixel, sample);
+	path_pixel_sample<LIST>(bp, batch, path, pixel, sample);
 	const rt::f4 r = rt::rng4(bp.seed, pixel, sample, bounce, rt::STREAM_SCATTER);
 	v3 dir, att;
 	float w = 1.0f;
@@ -1014,7 +1039,7 @@ __device__ __forceinline__ void bin_table_flush(uint32_t* s_key, uint32_t* s_cnt
 #ifndef SHADE_MIN_BLOCKS
 #define SHADE_MIN_BLOCKS 8   // 8 x 128 threads x 64 registers = the whole register file (6 / 9 / 10 blocks: 11.7 / 10.9 / 12.4 ms)
 #endif
-template <bool LIGHTS>
+template <bool LIGHTS, bool LIST>
 __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS)
 shade_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int q) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -1045,7 +1070,7 @@ shade_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int 
 			float4 fo, fd; ld_ray(rod + 2 * (size_t)i, fo, fd);
 			const float4 ft = ldq(rt_ + i);
 			const int2 h = ldq(wv.hit + i);
-			alive = shade_segment<true, LIGHTS>(sv, bp, wv, batch, bounce, fo, fd, xyz(ft), __int_as_float(h.x), h.y, no, nd, nthr, dt);
+			alive = shade_segment<true, LIGHTS, LIST>(sv, bp, wv, batch, bounce, fo, fd, xyz(ft), __int_as_float(h.x), h.y, no, nd, nthr, dt);
 		}
 		// live-path compaction: warp ballot/popc, one global atomic per block
 		const uint32_t mask = __ballot_sync(FULL_MASK, alive);
@@ -1247,7 +1272,7 @@ bin_permute_kernel(SceneView sv, WaveView wv, uint32_t bounce, int q_from) {
 // One persistent launch then runs every remaining path to completion (traverse + shade fused, one
 // thread per path); later traverse/shade launches of the batch see tail_from and return at once.
 
-template <bool MEDIA, int STACK, bool LIGHTS>
+template <bool MEDIA, int STACK, bool LIGHTS, bool LIST>
 __global__ void __launch_bounds__(TRAVERSE_THREADS)
 tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int q, uint32_t threshold) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -1265,7 +1290,7 @@ tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int 
 	for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
 		float4 fo, fd; ld_ray(rod + 2 * (size_t)i, fo, fd);
 		v3 thr = xyz(rt_[i]);
-		MediumRng mr = make_medium_rng(bp, batch, __float_as_uint(fd.w), bounce0);
+		MediumRngT<LIST> mr = make_medium_rng<LIST>(bp, batch, __float_as_uint(fd.w), bounce0);
 		for (uint32_t b = bounce0; b < bp.max_depth; ++b) {
 			if (b > bounce0) ++extra;
 			mr.bounce = b; mr.block = 0xFFFFFFFFu;
@@ -1273,7 +1298,7 @@ tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int 
 			trace_ray<(MEDIA ? 2 : 0)>(sv, xyz(fo), xyz(fd), fo.w, mr, s_stack + threadIdx.x, STACK, t, code);
 			float4 no, nd; v3 nthr;
 			DeferredTex dt;
-			if (!shade_segment<false, LIGHTS>(sv, bp, wv, batch, b, fo, fd, thr, t, code, no, nd, nthr, dt)) break;
+			if (!shade_segment<false, LIGHTS, LIST>(sv, bp, wv, batch, b, fo, fd, thr, t, code, no, nd, nthr, dt)) break;
 			fo = no; fd = nd; thr = nthr;
 		}
 	}
@@ -1285,6 +1310,9 @@ tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int 
 // ------------------------------------------------------------------------------------------------
 // accumulate + batch epilogue + resolve
 
+// LIST: the sums of local pixel pl go to pixel_list[pl], with the same float operations as dense, and the sums of squares
+// are always kept (the stopping rule needs them).
+template <bool LIST>
 __global__ void __launch_bounds__(STREAM_THREADS)
 accumulate_kernel(BatchParams bp_in, WaveView wv, float4* __restrict__ accum, float4* __restrict__ accum2) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -1297,13 +1325,13 @@ accumulate_kernel(BatchParams bp_in, WaveView wv, float4* __restrict__ accum, fl
 		for (uint32_t s = 0; s < ns; ++s) {   // fixed sample order: deterministic sums
 			const float4 c = wv.contrib[(size_t)s * bp.npix + pl];
 			sx += c.x; sy += c.y; sz += c.z;
-			if (bp.variance) { qx = fmaf(c.x, c.x, qx); qy = fmaf(c.y, c.y, qy); qz = fmaf(c.z, c.z, qz); }
+			if (LIST || bp.variance) { qx = fmaf(c.x, c.x, qx); qy = fmaf(c.y, c.y, qy); qz = fmaf(c.z, c.z, qz); }
 		}
-		const uint32_t gid = bp.row_begin * bp.width + pl;
+		const uint32_t gid = LIST ? listed_pixel(bp.pixel_list(), pl, bp.row_begin * bp.width, bp.n_rows * bp.width) : bp.row_begin * bp.width + pl;
 		float4 a = accum[gid];
 		a.x += sx; a.y += sy; a.z += sz; a.w += (float)ns;
 		accum[gid] = a;
-		if (bp.variance) {
+		if (LIST || bp.variance) {
 			float4 q = accum2[gid];
 			q.x += qx; q.y += qy; q.z += qz; q.w += (float)ns;
 			accum2[gid] = q;
@@ -1330,6 +1358,122 @@ resolve_kernel(const float4* __restrict__ accum, float4* __restrict__ out, uint3
 		float r = a.x * inv, g = a.y * inv, b = a.z * inv;
 		r = fminf(fmaxf(r, 0.0f), 1.0f); g = fminf(fmaxf(g, 0.0f), 1.0f); b = fminf(fmaxf(b, 0.0f), 1.0f);
 		out[i] = make_float4(sqrtf(r), sqrtf(g), sqrtf(b), 1.0f);  // clamp, gamma 2, alpha 1   :209-214
+	}
+}
+
+// ------------------------------------------------------------------------------------------------
+// adaptive select step (DESIGN.md §5c): which pixels the next round of rtb_render_adaptive renders
+//   adaptive_error   e_p = one standard error of the pixel's mean in display space (clamp, then sqrt, as resolve does)
+//   adaptive_count   window maximum W_p of e over the 3x3 neighbourhood + candidate test, active pixels per block
+//   adaptive_scan    exclusive prefix sums of the block counts, and the total
+//   adaptive_write   every active pixel to its slot of the list: ascending pixel order, so camera rays stay coherent
+// The rule is evaluated in binary32 in the order DESIGN.md writes it (-fmad=false: nothing is contracted), so
+// tests/adaptive_rule.py reproduces every decision.  Maxima and minima propagate NaN.
+
+__device__ __forceinline__ float nan_max(float a, float b) { return a != a ? a : (b != b ? b : fmaxf(a, b)); }
+__device__ __forceinline__ float nan_min(float a, float b) { return a != a ? a : (b != b ? b : fminf(a, b)); }
+
+__device__ __forceinline__ float display_error(float S, float Q, float n) {
+	const float m = S / n;
+	const float v = nan_max((Q - S * m) / (n - 1.0f), 0.0f);
+	const float s = sqrtf(v / n);
+	const float hi = sqrtf(nan_min(nan_max(m + s, 0.0f), 1.0f)), lo = sqrtf(nan_min(nan_max(m - s, 0.0f), 1.0f));
+	return (hi - lo) * 0.5f;
+}
+
+__global__ void __launch_bounds__(STREAM_THREADS)
+adaptive_error_kernel(AdaptiveView av) {
+	const uint32_t n = av.width * av.n_rows, first = av.row_begin * av.width;
+	const uint32_t stride = gridDim.x * blockDim.x;
+	for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+		const float4 a = av.accum[first + i], q = av.accum2[first + i];
+		const float er = display_error(a.x, q.x, a.w), eg = display_error(a.y, q.y, a.w), eb = display_error(a.z, q.z, a.w);
+		av.err[first + i] = nan_max(nan_max(er, eg), eb);
+	}
+}
+
+#define SELECT_THREADS 1024   // pixels per block of the select step (one per thread)
+
+// Whether pixel first + i takes part in the next round; `no_sq` = it holds the cursor's samples but no sums of squares, so
+// the rule cannot be evaluated for it (checked before the window: without sums of squares every error reads as 0).
+__device__ __forceinline__ bool adaptive_active(const AdaptiveView& av, uint32_t i, bool& no_sq) {
+	no_sq = false;
+	if (i >= av.width * av.n_rows) return false;
+	const uint32_t first = av.row_begin * av.width;
+	const float4 a = av.accum[first + i];
+	if (!(a.w == (float)av.cursor)) return false;                 // missed a round: never comes back
+	no_sq = !(av.accum2[first + i].w == a.w);
+	if (no_sq || av.cursor >= av.max_spp) return false;
+	if (av.cursor >= av.min_spp) {
+		const int y = (int)(i / av.width), x = (int)(i - (uint32_t)y * av.width);
+		const int y0 = max(y - 1, 0), y1 = min(y + 1, (int)av.n_rows - 1), x0 = max(x - 1, 0), x1 = min(x + 1, (int)av.width - 1);
+		float w = 0.0f;
+		for (int yy = y0; yy <= y1; ++yy)
+			for (int xx = x0; xx <= x1; ++xx) {
+				const float e = av.err[first + (uint32_t)yy * av.width + (uint32_t)xx];
+				w = fmaxf(w, e != e ? INFINITY : e);
+			}
+		if (w <= av.tolerance) return false;
+	}
+	return true;
+}
+
+__global__ void __launch_bounds__(SELECT_THREADS)
+adaptive_count_kernel(AdaptiveView av) {
+	__shared__ uint32_t s_count;
+	if (threadIdx.x == 0) s_count = 0u;
+	__syncthreads();
+	bool no_sq;
+	const bool active = adaptive_active(av, blockIdx.x * SELECT_THREADS + threadIdx.x, no_sq);
+	if (no_sq) atomicOr(av.result + 1, 1u);
+	const uint32_t mask = __ballot_sync(FULL_MASK, active);
+	if ((threadIdx.x & 31) == 0 && mask) atomicAdd(&s_count, (uint32_t)__popc(mask));
+	__syncthreads();
+	if (threadIdx.x == 0) av.block_count[blockIdx.x] = s_count;
+}
+
+// One block: exclusive prefix sums of the block counts in place, in chunks of SELECT_THREADS, and the total.
+__global__ void __launch_bounds__(SELECT_THREADS)
+adaptive_scan_kernel(AdaptiveView av, uint32_t n_blocks) {
+	__shared__ uint32_t s_part[SELECT_THREADS];
+	uint32_t carry = 0;
+	for (uint32_t base = 0; base < n_blocks; base += SELECT_THREADS) {
+		const uint32_t b = base + threadIdx.x;
+		const uint32_t c = b < n_blocks ? av.block_count[b] : 0u;
+		s_part[threadIdx.x] = c;
+		__syncthreads();
+		for (uint32_t off = 1; off < SELECT_THREADS; off <<= 1) {
+			const uint32_t v = threadIdx.x >= off ? s_part[threadIdx.x - off] : 0u;
+			__syncthreads();
+			s_part[threadIdx.x] += v;
+			__syncthreads();
+		}
+		if (b < n_blocks) av.block_count[b] = carry + s_part[threadIdx.x] - c;
+		carry += s_part[SELECT_THREADS - 1];
+		__syncthreads();
+	}
+	if (threadIdx.x == 0) av.result[0] = carry;
+}
+
+__global__ void __launch_bounds__(SELECT_THREADS)
+adaptive_write_kernel(AdaptiveView av) {
+	__shared__ uint32_t s_warp[SELECT_THREADS / 32];
+	const uint32_t i = blockIdx.x * SELECT_THREADS + threadIdx.x;
+	bool no_sq;
+	const bool active = adaptive_active(av, i, no_sq);
+	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+	const uint32_t mask = __ballot_sync(FULL_MASK, active);
+	if (lane == 0) s_warp[warp] = __popc(mask);
+	__syncthreads();
+	if (threadIdx.x == 0) {
+		uint32_t tot = 0;
+		for (int w = 0; w < SELECT_THREADS / 32; ++w) { const uint32_t c = s_warp[w]; s_warp[w] = tot; tot += c; }
+	}
+	__syncthreads();
+	if (active) {
+		const uint32_t pos = av.block_count[blockIdx.x] + s_warp[warp] + __popc(mask & ((1u << lane) - 1u));
+		RTB_CHECK(pos < av.width * av.n_rows, RTB_BOUNDS_PATH);
+		av.list[pos] = av.row_begin * av.width + i;
 	}
 }
 
@@ -1421,14 +1565,14 @@ void query_occupancy(int device, LaunchCfg& lc) {
 	cudaGetDeviceProperties(&prop, device);
 	int sms = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : 148;
 	int occ_t = 0, occ_tm = 0, occ_s = 0, occ_g = 0;
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_t, traverse_kernel<0, STACK_SIZE>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_tm, traverse_kernel<2, STACK_SIZE>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, shade_kernel<false>, SHADE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_g, generate_kernel, STREAM_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_t, traverse_kernel<0, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_tm, traverse_kernel<2, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, shade_kernel<false, false>, SHADE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_g, generate_kernel<false>, STREAM_THREADS, 0);
 	int occ_trav = occ_t < occ_tm ? occ_t : occ_tm;
 	int occ_l = 0, occ_lm = 0;
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_l, tail_kernel<false, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_lm, tail_kernel<true, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_l, tail_kernel<false, STACK_SIZE, false, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_lm, tail_kernel<true, STACK_SIZE, false, false>, TRAVERSE_THREADS, 0);
 	int occ_tail = occ_l < occ_lm ? occ_l : occ_lm;
 	lc.blocks_tail = sms * (occ_tail > 0 ? occ_tail : 1);
 	lc.sms = sms;
@@ -1443,39 +1587,50 @@ void query_occupancy(int device, LaunchCfg& lc) {
 }
 
 void launch_generate(const BatchParams& bp, const rtb_camera& cam, const WaveView& wv, const LaunchCfg& lc, cudaStream_t st) {
-	generate_kernel<<<lc.blocks_stream, STREAM_THREADS, 0, st>>>(bp, cam, wv);
+	if (bp.pixel_list()) generate_kernel<true><<<lc.blocks_stream, STREAM_THREADS, 0, st>>>(bp, cam, wv);
+	else generate_kernel<false><<<lc.blocks_stream, STREAM_THREADS, 0, st>>>(bp, cam, wv);
 }
 void launch_traverse(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t bounce, int q, const LaunchCfg& lc, cudaStream_t st) {
 	// media need the per-path RNG inside traversal; scenes without media skip that code entirely
 	// a walk keeps at most depth - 1 entries on its stack: 16 entries for shallow trees, 32 normally, 64 for the deep
 	// trees a linear BVH over a large mesh can be (the flattener never hands over more than RTB_TREE_DEPTH_MAX levels)
 	const bool small = sv.tree_depth <= 17, deep = sv.tree_depth > STACK_SIZE - 2;
-#define RTB_LAUNCH_TRAVERSE(M) \
-	do { if (small) traverse_kernel<M, 16><<<lc.blocks_traverse, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q); \
-	     else if (deep) traverse_kernel<M, DEEP_STACK_SIZE><<<lc.blocks_traverse, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q); \
-	     else traverse_kernel<M, STACK_SIZE><<<lc.blocks_traverse, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q); } while (0)
-	if (sv.has_media == 0) RTB_LAUNCH_TRAVERSE(0);
-	else if (sv.has_media == 1) RTB_LAUNCH_TRAVERSE(1);
-	else RTB_LAUNCH_TRAVERSE(2);
+	// (adaptive rounds: only the walks with media derive a pixel, so only they have list-mode instantiations)
+#define RTB_LAUNCH_TRAVERSE(M, L) \
+	do { if (small) traverse_kernel<M, 16, L><<<lc.blocks_traverse, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q); \
+	     else if (deep) traverse_kernel<M, DEEP_STACK_SIZE, L><<<lc.blocks_traverse, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q); \
+	     else traverse_kernel<M, STACK_SIZE, L><<<lc.blocks_traverse, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q); } while (0)
+	if (sv.has_media == 0) RTB_LAUNCH_TRAVERSE(0, false);
+	else if (sv.has_media == 1) { if (bp.pixel_list()) RTB_LAUNCH_TRAVERSE(1, true); else RTB_LAUNCH_TRAVERSE(1, false); }
+	else { if (bp.pixel_list()) RTB_LAUNCH_TRAVERSE(2, true); else RTB_LAUNCH_TRAVERSE(2, false); }
 #undef RTB_LAUNCH_TRAVERSE
 }
 void launch_tail(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t bounce, int q, uint32_t threshold, const LaunchCfg& lc, cudaStream_t st) {
 	const bool deep = sv.tree_depth > STACK_SIZE - 2;
-#define RTB_LAUNCH_TAIL(M, L) \
-	do { if (deep) tail_kernel<M, DEEP_STACK_SIZE, L><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); \
-	     else tail_kernel<M, STACK_SIZE, L><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); } while (0)
-	if (sv.n_lights > 0) {   // (light sampling: its own instantiations, so the kernels of scenes without it stay as they were)
-		if (sv.has_media) RTB_LAUNCH_TAIL(true, true);
-		else RTB_LAUNCH_TAIL(false, true);
-	} else {
-		if (sv.has_media) RTB_LAUNCH_TAIL(true, false);
-		else RTB_LAUNCH_TAIL(false, false);
-	}
+#define RTB_LAUNCH_TAIL(M, L, P) \
+	do { if (deep) tail_kernel<M, DEEP_STACK_SIZE, L, P><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); \
+	     else tail_kernel<M, STACK_SIZE, L, P><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); } while (0)
+#define RTB_LAUNCH_TAIL_LM(P) \
+	do { if (sv.n_lights > 0) {   /* (light sampling: its own instantiations, so the kernels of scenes without it stay as they were) */ \
+	         if (sv.has_media) RTB_LAUNCH_TAIL(true, true, P); \
+	         else RTB_LAUNCH_TAIL(false, true, P); \
+	     } else { \
+	         if (sv.has_media) RTB_LAUNCH_TAIL(true, false, P); \
+	         else RTB_LAUNCH_TAIL(false, false, P); \
+	     } } while (0)
+	if (bp.pixel_list()) RTB_LAUNCH_TAIL_LM(true);
+	else RTB_LAUNCH_TAIL_LM(false);
+#undef RTB_LAUNCH_TAIL_LM
 #undef RTB_LAUNCH_TAIL
 }
 void launch_shade(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t bounce, int q, const LaunchCfg& lc, cudaStream_t st) {
-	if (sv.n_lights > 0) shade_kernel<true><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
-	else shade_kernel<false><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
+	if (bp.pixel_list()) {
+		if (sv.n_lights > 0) shade_kernel<true, true><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
+		else shade_kernel<false, true><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
+	} else {
+		if (sv.n_lights > 0) shade_kernel<true, false><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
+		else shade_kernel<false, false><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q);
+	}
 }
 void launch_texture(const SceneView& sv, const WaveView& wv, uint32_t bounce, int q_out, const LaunchCfg& lc, cudaStream_t st) {
 	const int blocks = lc.sms * 2 < lc.blocks_stream ? lc.sms * 2 : lc.blocks_stream;   // short work lists: a small grid keeps the launch cheap
@@ -1488,8 +1643,20 @@ void launch_bin_rays(const SceneView& sv, const WaveView& wv, uint32_t bounce, i
 	bin_permute_kernel<<<lc.blocks_bin, BIN_THREADS, BIN_PERMUTE_SMEM, st>>>(sv, wv, bounce, q_from);
 }
 void launch_accumulate(const BatchParams& bp, const WaveView& wv, float4* accum, float4* accum2, const LaunchCfg& lc, cudaStream_t st) {
-	accumulate_kernel<<<lc.blocks_stream, STREAM_THREADS, 0, st>>>(bp, wv, accum, accum2);
+	if (bp.pixel_list()) accumulate_kernel<true><<<lc.blocks_stream, STREAM_THREADS, 0, st>>>(bp, wv, accum, accum2);
+	else accumulate_kernel<false><<<lc.blocks_stream, STREAM_THREADS, 0, st>>>(bp, wv, accum, accum2);
 	end_batch_kernel<<<1, 32, 0, st>>>(bp, wv);
+}
+uint32_t adaptive_select_blocks(uint32_t n_pixels) { return (n_pixels + SELECT_THREADS - 1) / SELECT_THREADS; }
+void launch_adaptive_select(const AdaptiveView& av, const LaunchCfg& lc, cudaStream_t st) {
+	const uint32_t n = av.width * av.n_rows, nb = adaptive_select_blocks(n);
+	if (av.cursor >= av.min_spp) {   // (before min_spp every candidate is active whatever its error)
+		int blocks = (int)((n + STREAM_THREADS - 1) / STREAM_THREADS); if (blocks > lc.blocks_stream) blocks = lc.blocks_stream; if (blocks < 1) blocks = 1;
+		adaptive_error_kernel<<<blocks, STREAM_THREADS, 0, st>>>(av);
+	}
+	adaptive_count_kernel<<<nb, SELECT_THREADS, 0, st>>>(av);
+	adaptive_scan_kernel<<<1, SELECT_THREADS, 0, st>>>(av, nb);
+	adaptive_write_kernel<<<nb, SELECT_THREADS, 0, st>>>(av);
 }
 void launch_resolve(const float4* accum, float4* out, uint32_t n, cudaStream_t st) {
 	int blocks = (int)((n + STREAM_THREADS - 1) / STREAM_THREADS); if (blocks > 148 * 8) blocks = 148 * 8; if (blocks < 1) blocks = 1;

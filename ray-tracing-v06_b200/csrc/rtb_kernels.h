@@ -52,6 +52,38 @@ struct BatchParams {
 	// A render's batches can be dealt to two lanes (two streams with their own queues, so that the thin late bounces of one
 	// batch overlap the full early bounces of the next): the lane's k-th batch is batch_base + k * batch_stride.
 	uint32_t batch_base, batch_stride;
+	// Adaptive rounds (DESIGN.md §5c): npix = the number of listed pixels, and local pixel pl is pixel_list()[pl] instead of
+	// row_begin * width + pl.  Null = dense (every pixel of the row range); the launchers pick the list-mode kernels by it.
+	// (Kept as two 32-bit words after two unused ones: the struct stays 4-byte aligned and grows by 16 bytes, so every kernel
+	// parameter after it keeps its offset modulo 16.  With 8 bytes more, the camera parameter of generate_kernel moved to
+	// another alignment, the compiler picked other constant loads, and bench.py measured that layout 0.18 % slower.)
+	uint32_t unused[2];
+	uint32_t pixel_list_lo, pixel_list_hi;
+	__host__ __device__ const uint32_t* pixel_list() const {
+		return reinterpret_cast<const uint32_t*>(((uint64_t)pixel_list_hi << 32) | pixel_list_lo);
+	}
+	__host__ __device__ void set_pixel_list(const uint32_t* p) {
+		pixel_list_lo = (uint32_t)(uintptr_t)p; pixel_list_hi = (uint32_t)((uint64_t)(uintptr_t)p >> 32);
+	}
+};
+// The layout the comment above depends on.  A field added to BatchParams moves every kernel parameter after it: keep the
+// size a multiple of 16 bytes more than the 52 of the fields before the list (tools/sass_diff.py against the previous build
+// shows whether the dense kernels still compile to the same instructions), then update these numbers.
+static_assert(alignof(BatchParams) == 4 && sizeof(BatchParams) == 68 && offsetof(BatchParams, unused) == 52 &&
+              offsetof(BatchParams, pixel_list_lo) == 60, "BatchParams layout changed: see the comment above");
+
+// Buffers and parameters of the adaptive select step (rtb_render_adaptive): the error of every pixel of the row range, then
+// the ascending list of the pixels the next round renders and its length.
+struct AdaptiveView {
+	const float4* accum;        // (sums, count)
+	const float4* accum2;       // (sums of squares, count)
+	float* err;                 // [width * height] display-space standard error e_p
+	uint32_t* list;             // [width * height] the active pixels, ascending
+	uint32_t* block_count;      // [blocks of the select step] active pixels per block, then their exclusive prefix sums
+	uint32_t* result;           // [0] active pixels, [1] nonzero when a pixel holding the cursor has no sums of squares
+	uint32_t width, row_begin, n_rows;
+	uint32_t cursor, min_spp, max_spp;
+	float tolerance;
 };
 
 // Wavefront queues, double buffered.  A ray is a 32-byte record (o.xyz, time)(d.xyz, path id bits) - one DRAM sector, so
@@ -89,6 +121,10 @@ void launch_texture(const SceneView& sv, const WaveView& wv, uint32_t bounce, in
 // moves to its bin's range in queue q_from ^ 1.
 void launch_bin_rays(const SceneView& sv, const WaveView& wv, uint32_t bounce, int q_from, const LaunchCfg& lc, cudaStream_t st);
 void launch_accumulate(const BatchParams& bp, const WaveView& wv, float4* accum, float4* accum2, const LaunchCfg& lc, cudaStream_t st);
+// Adaptive select step: per-pixel error (skipped while cursor < min_spp: every candidate is active then), window and
+// candidate test, ascending compaction into av.list; av.result[0..1] must be zero before.  Blocks of the select step:
+uint32_t adaptive_select_blocks(uint32_t n_pixels);
+void launch_adaptive_select(const AdaptiveView& av, const LaunchCfg& lc, cudaStream_t st);
 void launch_resolve(const float4* accum, float4* out, uint32_t n, cudaStream_t st);
 void launch_quantize(const float4* accum, uint8_t* rgb, uint32_t width, uint32_t height, int flip_rows, cudaStream_t st);
 

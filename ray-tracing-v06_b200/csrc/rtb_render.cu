@@ -6,6 +6,7 @@
 // SoA buffers instead of ~3 device allocations + a <<<1,1>>> constructor launch per object.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -94,6 +95,8 @@ void rtb_renderer_destroy(rtb_renderer* r) {
 	for (cudaEvent_t e : r->prof_events) cudaEventDestroy(e);
 	if (r->stream2) cudaStreamSynchronize(r->stream2);
 	cudaFree(r->d_scene); cudaFree(r->d_accum); cudaFree(r->d_accum2); cudaFree(r->d_out); cudaFree(r->d_wave); cudaFree(r->d_wave2); cudaFree(r->d_rgb8);
+	cudaFree(r->d_err); cudaFree(r->d_list); cudaFree(r->d_block); cudaFree(r->d_select);
+	if (r->h_select) cudaFreeHost(r->h_select);
 	for (cudaEvent_t e : {r->ev_lane[0], r->ev_lane[1], r->ev_fork}) if (e) cudaEventDestroy(e);
 	if (r->stream2) cudaStreamDestroy(r->stream2);
 	for (cudaEvent_t e : {r->ev_in, r->ev_out, r->ev_t0, r->ev_t1}) if (e) cudaEventDestroy(e);
@@ -240,16 +243,42 @@ static int ensure_framebuffer(rtb_renderer* r, uint32_t w, uint32_t h) {
 	if (r->width == w && r->height == h && r->d_accum) return RTB_OK;
 	CUDA_TRY(cudaStreamSynchronize(r->stream));
 	cudaFree(r->d_accum); cudaFree(r->d_accum2); cudaFree(r->d_out); cudaFree(r->d_rgb8);
+	cudaFree(r->d_err); cudaFree(r->d_list); cudaFree(r->d_block); cudaFree(r->d_select);
 	r->d_accum = r->d_accum2 = r->d_out = nullptr; r->d_rgb8 = nullptr; r->sample_cursor = 0;
+	r->d_err = nullptr; r->d_list = r->d_block = r->d_select = nullptr;
 	size_t bytes = (size_t)w * h * sizeof(float4);
 	CUDA_TRY(cudaMalloc(&r->d_accum, bytes));
 	CUDA_TRY(cudaMalloc(&r->d_accum2, bytes));
 	CUDA_TRY(cudaMalloc(&r->d_out, bytes));
-	CUDA_TRY(cudaMemset(r->d_accum, 0, bytes));
-	CUDA_TRY(cudaMemset(r->d_accum2, 0, bytes));
-	CUDA_TRY(cudaMemset(r->d_out, 0, bytes));
+	// (zeroed on the renderer's stream: it is non-blocking, so a cudaMemset on the legacy stream would not be ordered
+	// before the work enqueued on it next)
+	CUDA_TRY(cudaMemsetAsync(r->d_accum, 0, bytes, r->stream));
+	CUDA_TRY(cudaMemsetAsync(r->d_accum2, 0, bytes, r->stream));
+	CUDA_TRY(cudaMemsetAsync(r->d_out, 0, bytes, r->stream));
 	r->width = w; r->height = h;
 	free_graph(r);
+	return RTB_OK;
+}
+
+// Buffers of the adaptive select step, for the current framebuffer size (allocated by the first adaptive render after each
+// resize, so that uniform renders allocate exactly what they did before adaptive sampling existed).
+static int ensure_adaptive_buffers(rtb_renderer* r) {
+	if (r->d_err && r->d_list && r->d_block && r->d_select && r->h_select) return RTB_OK;
+	// all or nothing: a failure part-way leaves every device pointer null, and the next call starts over
+	cudaFree(r->d_err); cudaFree(r->d_list); cudaFree(r->d_block); cudaFree(r->d_select);
+	r->d_err = nullptr; r->d_list = r->d_block = r->d_select = nullptr;
+	const size_t n = (size_t)r->width * r->height;
+	cudaError_t e = cudaMalloc(&r->d_err, n * sizeof(float));
+	if (e == cudaSuccess) e = cudaMalloc(&r->d_list, n * sizeof(uint32_t));
+	if (e == cudaSuccess) e = cudaMalloc(&r->d_block, (size_t)adaptive_select_blocks((uint32_t)n) * sizeof(uint32_t));
+	if (e == cudaSuccess) e = cudaMalloc(&r->d_select, 256);
+	if (e == cudaSuccess && !r->h_select) e = cudaMallocHost(&r->h_select, 2 * sizeof(uint32_t));
+	if (e != cudaSuccess) {
+		cudaFree(r->d_err); cudaFree(r->d_list); cudaFree(r->d_block); cudaFree(r->d_select);
+		r->d_err = nullptr; r->d_list = r->d_block = r->d_select = nullptr;
+		cudaGetLastError();
+		return fail(RTB_ERR_NOMEM, std::string("rtb_render_adaptive: allocating the select buffers: ") + cudaGetErrorString(e));
+	}
 	return RTB_OK;
 }
 
@@ -263,6 +292,9 @@ static int ensure_wave(rtb_renderer* r, int lane, size_t paths, uint32_t depth) 
 	CUDA_TRY(cudaStreamSynchronize(r->stream));
 	if (r->stream2) CUDA_TRY(cudaStreamSynchronize(r->stream2));
 	free_graph(r);
+	// the path / ray totals (rtb_get_counters) live in the queue buffer: carry them over to the new one
+	unsigned long long totals[2] = {0, 0};
+	if (d_wave) CUDA_TRY(cudaMemcpy(totals, wv.totals, sizeof totals, cudaMemcpyDeviceToHost));
 	cudaFree(d_wave); d_wave = nullptr;
 	if (paths < wave_paths) paths = wave_paths;     // grow-only in both dimensions: alternating sizes do not thrash
 	if (depth < wave_depth) depth = wave_depth;
@@ -278,7 +310,7 @@ static int ensure_wave(rtb_renderer* r, int lane, size_t paths, uint32_t depth) 
 	size_t o_bcnt = take(nbins * 4), o_bcur = take(nbins * 4);
 	cudaError_t e = cudaMalloc(&d_wave, off);
 	if (e != cudaSuccess) { d_wave = nullptr; cudaGetLastError(); return fail(RTB_ERR_NOMEM, std::string("cudaMalloc of the wavefront queues: ") + cudaGetErrorString(e)); }
-	CUDA_TRY(cudaMemset(d_wave, 0, off));
+	CUDA_TRY(cudaMemsetAsync(d_wave, 0, off, r->stream));   // (ordered before the batch that follows; lane 1 starts after an event on this stream)
 	uint8_t* b = static_cast<uint8_t*>(d_wave);
 	wv.ray_od[0] = (float4*)(b + o_od0); wv.ray_od[1] = (float4*)(b + o_od1);
 	wv.thr[0] = (float4*)(b + o_t0); wv.thr[1] = (float4*)(b + o_t1);
@@ -289,6 +321,10 @@ static int ensure_wave(rtb_renderer* r, int lane, size_t paths, uint32_t depth) 
 	wv.capacity = (uint32_t)P; wv.n_bins = (uint32_t)nbins;
 	wv.batch_index = (uint32_t*)(b + o_batch); wv.tail_from = wv.batch_index + 1; wv.totals = (unsigned long long*)(b + o_tot);
 	wv.call_params = wv.batch_index + 8;   // (same 256-byte block)
+	if (totals[0] || totals[1]) {
+		CUDA_TRY(cudaMemcpyAsync(wv.totals, totals, sizeof totals, cudaMemcpyHostToDevice, r->stream));
+		CUDA_TRY(cudaStreamSynchronize(r->stream));   // (the source is on this stack frame)
+	}
 	wave_paths = P; wave_depth = depth;
 	return RTB_OK;
 }
@@ -341,6 +377,33 @@ static int capture_batch_graph(rtb_renderer* r, const WaveView& wv, const BatchP
 	return RTB_OK;
 }
 
+// Paths one batch of an automatic batch size aims at, for `npix` pixels: 64 M (~9.7 GB of queues; larger batches keep
+// late, thin bounces full), RTB_BATCH_PATHS, or less when device memory is short.
+static uint64_t batch_path_budget(rtb_renderer* r, uint64_t npix, uint32_t samples_per_batch) {
+	uint64_t target_paths = 64ull << 20;
+	if (const char* e = getenv("RTB_BATCH_PATHS")) { uint64_t v = strtoull(e, nullptr, 10); if (v > 0) target_paths = v; }
+	if (!samples_per_batch && target_paths > r->wave_paths) {
+		// the queues cost RTB_WAVE_BYTES_PER_PATH per path: an automatic batch never asks for more than half of what is free
+		// (a smaller device, several renderers per device, a large scene) - it gets smaller instead of failing
+		size_t free_b = 0, total_b = 0;
+		if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
+			const uint64_t cap = (uint64_t)(free_b / 2 + r->wave_paths * RTB_WAVE_BYTES_PER_PATH) / RTB_WAVE_BYTES_PER_PATH;
+			if (target_paths > cap) target_paths = cap > npix ? cap : npix;
+		} else cudaGetLastError();
+	}
+	return target_paths;
+}
+
+// Samples per batch for `spp` samples of `npix` pixels: the caller's samples_per_batch, else as many as the budget holds,
+// evened out so that every batch has the same size.
+static uint64_t batch_samples(uint64_t target_paths, uint64_t npix, uint32_t spp, uint32_t samples_per_batch) {
+	uint64_t S = samples_per_batch ? samples_per_batch : target_paths / npix;
+	if (S < 1) S = 1;
+	if (S > spp) S = spp ? spp : 1;
+	if (!samples_per_batch && spp) { uint64_t nb = (spp + S - 1) / S; S = (spp + nb - 1) / nb; }   // equal-sized batches
+	return S;
+}
+
 int rtb_render(rtb_renderer* r, const rtb_render_params* p, void* user_stream) {
 	if (!r || !p) return fail(RTB_ERR_INVALID, "rtb_render: null argument");
 	if (!r->has_scene) return fail(RTB_ERR_STATE, "rtb_render: no scene (rtb_renderer_set_scene)");
@@ -357,21 +420,7 @@ int rtb_render(rtb_renderer* r, const rtb_render_params* p, void* user_stream) {
 
 	const uint32_t spp = p->sample_end - p->sample_begin;
 	const uint64_t npix = (uint64_t)p->width * (row_end - row_begin);
-	uint64_t target_paths = 64ull << 20;   // ~9.7 GB of queues; larger batches keep late, thin bounces full (RTB_BATCH_PATHS overrides)
-	if (const char* e = getenv("RTB_BATCH_PATHS")) { uint64_t v = strtoull(e, nullptr, 10); if (v > 0) target_paths = v; }
-	if (!p->samples_per_batch && target_paths > r->wave_paths) {
-		// the queues cost RTB_WAVE_BYTES_PER_PATH per path: an automatic batch never asks for more than half of what is free
-		// (a smaller device, several renderers per device, a large scene) - it gets smaller instead of failing
-		size_t free_b = 0, total_b = 0;
-		if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
-			const uint64_t cap = (uint64_t)(free_b / 2 + r->wave_paths * RTB_WAVE_BYTES_PER_PATH) / RTB_WAVE_BYTES_PER_PATH;
-			if (target_paths > cap) target_paths = cap > npix ? cap : npix;
-		} else cudaGetLastError();
-	}
-	uint64_t S = p->samples_per_batch ? p->samples_per_batch : target_paths / npix;
-	if (S < 1) S = 1;
-	if (S > spp) S = spp ? spp : 1;
-	if (!p->samples_per_batch && spp) { uint64_t nb = (spp + S - 1) / S; S = (spp + nb - 1) / nb; }   // equal-sized batches
+	const uint64_t S = batch_samples(batch_path_budget(r, npix, p->samples_per_batch), npix, spp, p->samples_per_batch);
 	if (npix * S >= (1ull << 31)) return fail(RTB_ERR_INVALID, "rtb_render: batch too large (lower samples_per_batch)");
 	rc = ensure_wave(r, 0, (size_t)(npix * S), p->max_depth);
 	if (rc) return rc;
@@ -472,6 +521,108 @@ int rtb_render(rtb_renderer* r, const rtb_render_params* p, void* user_stream) {
 	// ... and let the caller's stream see the result
 	CUDA_TRY(cudaEventRecord(r->ev_out, st));
 	CUDA_TRY(cudaStreamWaitEvent(us, r->ev_out, 0));
+	return RTB_OK;
+}
+
+// Adaptive sampling (DESIGN.md §5c).  Each round: the select step on the device writes the ascending list of active pixels
+// and their count, the host reads the count (one sync per round), and the round renders samples [c, c + k) of every listed
+// pixel through enqueue_batch in list mode.  The shape of a round (pixel count, batch size) changes from round to round,
+// so rounds run on one lane and without a CUDA graph.
+int rtb_render_adaptive(rtb_renderer* r, const rtb_render_params* p, const rtb_adaptive_params* a, rtb_adaptive_stats* out, void* user_stream) {
+	if (!r || !p || !a) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: null argument");
+	if (!r->has_scene) return fail(RTB_ERR_STATE, "rtb_render_adaptive: no scene (rtb_renderer_set_scene)");
+	if (!r->has_cam) return fail(RTB_ERR_STATE, "rtb_render_adaptive: no camera (rtb_renderer_set_camera)");
+	if (p->width == 0 || p->height == 0 || p->max_depth == 0) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: zero width/height/max_depth");
+	if (p->sample_begin != 0) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: sample_begin must be 0 (the call continues from the accumulator's own cursor)");
+	if (a->min_spp < 2) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: min_spp must be at least 2");
+	if (p->sample_end < a->min_spp || p->sample_end > (1u << 24)) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: need min_spp <= sample_end <= 2^24");
+	if (!(a->tolerance >= 0.0f) || !(a->tolerance <= 3.402823466e+38f)) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: tolerance must be finite and >= 0");
+	uint32_t row_begin = p->row_begin, row_end = p->row_end;
+	if (row_begin == 0 && row_end == 0) row_end = p->height;
+	if (row_end > p->height || row_begin >= row_end) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: bad row range");
+	if ((uint64_t)p->width * p->height >= (1ull << 31)) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: image too large");
+	const bool clear = (p->flags & RTB_RENDER_CLEAR) != 0;
+	if (!clear && r->d_accum && (r->width != p->width || r->height != p->height))
+		return fail(RTB_ERR_STATE, "rtb_render_adaptive: the accumulator holds another image size (pass RTB_RENDER_CLEAR)");
+	CUDA_TRY(cudaSetDevice(r->device));
+	int rc = ensure_framebuffer(r, p->width, p->height);
+	if (rc) return rc;
+	rc = ensure_adaptive_buffers(r);
+	if (rc) return rc;
+
+	const uint64_t npix_range = (uint64_t)p->width * (row_end - row_begin);
+	const uint32_t max_spp = p->sample_end;
+	const uint64_t budget = batch_path_budget(r, npix_range, p->samples_per_batch);
+	uint32_t c = clear ? 0u : r->sample_cursor;
+	AdaptiveView av{};
+	av.accum = r->d_accum; av.accum2 = r->d_accum2; av.err = r->d_err; av.list = r->d_list; av.block_count = r->d_block; av.result = r->d_select;
+	av.width = p->width; av.row_begin = row_begin; av.n_rows = row_end - row_begin;
+	av.min_spp = a->min_spp; av.max_spp = max_spp; av.tolerance = a->tolerance;
+
+	cudaStream_t us = static_cast<cudaStream_t>(user_stream);
+	cudaStream_t st = r->stream;
+	CUDA_TRY(cudaEventRecord(r->ev_in, us));
+	CUDA_TRY(cudaStreamWaitEvent(st, r->ev_in, 0));
+	if (clear) {
+		size_t bytes = (size_t)p->width * p->height * sizeof(float4);
+		CUDA_TRY(cudaMemsetAsync(r->d_accum, 0, bytes, st));
+		CUDA_TRY(cudaMemsetAsync(r->d_accum2, 0, bytes, st));
+	}
+	CUDA_TRY(cudaEventRecord(r->ev_t0, st));
+	rtb_adaptive_stats stats{};
+	uint32_t n_active = 0;
+	const int rc_rounds = [&]() -> int {
+		for (;;) {
+			// select step: error, window, candidates, ascending list; then the one read-back of the round
+			av.cursor = c;
+			CUDA_TRY(cudaMemsetAsync(r->d_select, 0, 2 * sizeof(uint32_t), st));
+			prof_begin(r, 6, st); launch_adaptive_select(av, r->lc, st); prof_end(r, st);
+			r->launches += (c >= a->min_spp ? 4 : 3);
+			CUDA_TRY(cudaGetLastError());
+			CUDA_TRY(cudaMemcpyAsync(r->h_select, r->d_select, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+			CUDA_TRY(cudaStreamSynchronize(st));
+			n_active = r->h_select[0];
+			if (r->h_select[1]) return fail(RTB_ERR_STATE, "rtb_render_adaptive: the accumulator has no sums of squares (render it with RTB_RENDER_VARIANCE)");
+			if (n_active == 0 || (a->max_rounds && stats.rounds >= a->max_rounds)) break;
+
+			// round size: up to min_spp first; after that at most one doubling of the cursor and at most one batch of paths
+			const uint64_t fill = budget / n_active > 1 ? budget / n_active : 1;
+			const uint32_t k = (uint32_t)std::min<uint64_t>(max_spp - c, c < a->min_spp ? (uint64_t)(a->min_spp - c) : std::min<uint64_t>(c, fill));
+			const uint64_t S = batch_samples(budget, n_active, k, p->samples_per_batch);
+			if ((uint64_t)n_active * S >= (1ull << 31)) return fail(RTB_ERR_INVALID, "rtb_render_adaptive: batch too large (lower samples_per_batch)");
+			rc = ensure_wave(r, 0, (size_t)(n_active * S), p->max_depth);
+			if (rc) return rc;
+			r->bin_on = r->bin_forced || (r->sv.n_nodes >= 512 && n_active * S >= (8ull << 20));
+			BatchParams bp{};
+			bp.width = p->width; bp.height = p->height; bp.row_begin = row_begin; bp.n_rows = row_end - row_begin;
+			bp.npix = n_active; bp.sample_begin = c; bp.sample_end = c + k;
+			bp.samples_per_batch = (uint32_t)S; bp.max_depth = p->max_depth; bp.seed = p->seed;
+			bp.variance = 1u; bp.batch_base = 0; bp.batch_stride = 1u;
+			bp.set_pixel_list(r->d_list);
+			CUDA_TRY(cudaMemsetAsync(r->wv.batch_index, 0, sizeof(uint32_t), st));
+			r->call_params[0] = bp.sample_begin; r->call_params[1] = bp.sample_end; r->call_params[2] = bp.seed; r->call_params[3] = 0;
+			CUDA_TRY(cudaMemcpyAsync(const_cast<uint32_t*>(r->wv.call_params), r->call_params, sizeof r->call_params, cudaMemcpyHostToDevice, st));
+			const uint32_t n_batches = (uint32_t)((k + S - 1) / S);
+			for (uint32_t b = 0; b < n_batches; ++b) enqueue_batch(r, r->wv, bp, st, true);
+			CUDA_TRY(cudaGetLastError());
+			r->launches += (3 + 2ull * bp.max_depth + (r->tail_threshold ? count_tail_checkpoints(bp.max_depth) : 0) +
+			                (r->sv.has_deferred_tex ? bp.max_depth - 1 : 0) + 3ull * count_binned_bounces(r, bp.max_depth)) * n_batches;
+			r->batches += n_batches;
+			stats.samples += (uint64_t)n_active * k;
+			stats.rounds++;
+			c += k;
+		}
+		return RTB_OK;
+	}();
+	// However the rounds ended - an error included - the cursor covers every round rendered (a later call or checkpoint
+	// continues from it) and the caller's stream is ordered after the work.
+	r->sample_cursor = c;
+	r->timed = true;
+	const cudaError_t e_end[3] = {cudaEventRecord(r->ev_t1, st), cudaEventRecord(r->ev_out, st), cudaStreamWaitEvent(us, r->ev_out, 0)};
+	stats.cursor = c; stats.active_pixels = n_active;
+	if (out) *out = stats;
+	if (rc_rounds) return rc_rounds;
+	for (cudaError_t e : e_end) if (e != cudaSuccess) return fail(RTB_ERR_CUDA, std::string("rtb_render_adaptive: joining the caller's stream: ") + cudaGetErrorString(e));
 	return RTB_OK;
 }
 
@@ -625,7 +776,7 @@ int rtb_get_profile(rtb_renderer* r, rtb_profile* out) {
 	memset(out, 0, sizeof *out);
 	CUDA_TRY(cudaSetDevice(r->device));
 	CUDA_TRY(cudaStreamSynchronize(r->stream));
-	double ms[6] = {0, 0, 0, 0, 0, 0}; uint64_t cnt[6] = {0, 0, 0, 0, 0, 0};
+	double ms[7] = {0, 0, 0, 0, 0, 0, 0}; uint64_t cnt[7] = {0, 0, 0, 0, 0, 0, 0};   // (class 6, the adaptive select step, is reported per launch only)
 	for (size_t i = 0; i < r->prof_used; ++i) {
 		float t = 0.0f;
 		CUDA_TRY(cudaEventElapsedTime(&t, r->prof_events[2 * i], r->prof_events[2 * i + 1]));
@@ -666,8 +817,9 @@ int rtb_reset_counters(rtb_renderer* r) {
 	CUDA_TRY(cudaSetDevice(r->device));
 	CUDA_TRY(cudaStreamSynchronize(r->stream));
 	if (r->stream2) CUDA_TRY(cudaStreamSynchronize(r->stream2));
-	if (r->d_wave) CUDA_TRY(cudaMemset(r->wv.totals, 0, 2 * sizeof(unsigned long long)));
-	if (r->d_wave2) CUDA_TRY(cudaMemset(r->wv2.totals, 0, 2 * sizeof(unsigned long long)));
+	if (r->d_wave) CUDA_TRY(cudaMemsetAsync(r->wv.totals, 0, 2 * sizeof(unsigned long long), r->stream));
+	if (r->d_wave2) CUDA_TRY(cudaMemsetAsync(r->wv2.totals, 0, 2 * sizeof(unsigned long long), r->stream));
+	CUDA_TRY(cudaStreamSynchronize(r->stream));
 	r->launches = 0; r->batches = 0;
 	return RTB_OK;
 }

@@ -46,6 +46,10 @@ struct rtb_renderer {
 	float4 *d_accum = nullptr, *d_accum2 = nullptr, *d_out = nullptr;
 	uint8_t* d_rgb8 = nullptr;              // 8-bit output (rtb_download_rgb8)
 	uint32_t sample_cursor = 0;             // one past the last sample index accumulated since the last clear (checkpoints)
+	// adaptive select step (rtb_render_adaptive; allocated by the first adaptive render after a resize of the framebuffer):
+	// per-pixel error, the list of active pixels, per-block counts, (count, missing sums of squares) on the device and in
+	// pinned host memory
+	float* d_err = nullptr; uint32_t *d_list = nullptr, *d_block = nullptr, *d_select = nullptr, *h_select = nullptr;
 
 	// wavefront queues
 	void* d_wave = nullptr; size_t wave_paths = 0; uint32_t wave_depth = 0;
@@ -74,7 +78,7 @@ struct rtb_renderer {
 	// optional per-launch event timing (rtb_renderer_set_profiling)
 	bool profiling = false;
 	std::vector<cudaEvent_t> prof_events;      // pairs (begin, end)
-	std::vector<int> prof_class;               // 0 generate, 1 traverse, 2 shade, 3 accumulate
+	std::vector<int> prof_class;               // 0 generate, 1 traverse, 2 shade, 3 accumulate, 4 tail, 5 binning, 6 adaptive select
 	size_t prof_used = 0;
 };
 

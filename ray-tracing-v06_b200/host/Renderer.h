@@ -30,6 +30,9 @@ class Renderer {
 		rtb_multi_renderer* mr{};
 		rtb_scene* scene{};
 		uint32_t seed{1984};
+		float noise_tolerance{-1.0f};   // < 0: uniform sampling
+		uint32_t noise_min_spp{};
+		rtb_adaptive_stats last_adaptive{};
 		double last_render_ms{};
 		uint64_t last_rays{}, last_paths{};
 	} m;
@@ -64,6 +67,13 @@ public:
 	// How many GPUs of the box the next MakeRenderer uses (0: RTB_GPUS from the environment, else one).
 	static void UseGpus(int n) { _gpus() = n; }
 	void SetSeed(uint32_t seed) { m.seed = seed; }
+	// Adaptive sampling (rtb_render_adaptive): from now on Render() gives every pixel min_spp samples, then more only where
+	// the display-space standard error of its 3x3 neighbourhood is above `tolerance` (10^(-D/20) for about D dB), with
+	// samples_per_pixel as the cap.  One GPU only: a renderer on several throws.
+	void SetNoiseTarget(float tolerance, uint32_t min_spp) {
+		if (m.mr) throw std::runtime_error("Renderer::SetNoiseTarget: adaptive sampling renders on one GPU (this renderer uses " + std::to_string(gpuCount()) + ")");
+		m.noise_tolerance = tolerance; m.noise_min_spp = min_spp;
+	}
 
 	static Renderer MakeRenderer(uint32_t render_width, uint32_t render_height, uint32_t samples_per_pixel, uint32_t max_depth,
 	                             const MotionBlurCamera* cam, const Hittable* d_world_ptr) {
@@ -105,7 +115,10 @@ public:
 		} else {
 			rtb_host::check(rtb_renderer_set_camera(m.r, &c), "rtb_renderer_set_camera");
 			rtb_host::check(rtb_reset_counters(m.r), "rtb_reset_counters");
-			rtb_host::check(rtb_render(m.r, &p, nullptr), "rtb_render");
+			if (m.noise_tolerance >= 0.0f) {
+				rtb_adaptive_params a{m.noise_tolerance, m.noise_min_spp, 0, 0};
+				rtb_host::check(rtb_render_adaptive(m.r, &p, &a, &m.last_adaptive, nullptr), "rtb_render_adaptive");
+			} else rtb_host::check(rtb_render(m.r, &p, nullptr), "rtb_render");
 			rtb_host::check(rtb_synchronize(m.r), "rtb_synchronize");
 			rtb_get_counters(m.r, &k);
 		}
@@ -126,5 +139,6 @@ public:
 	double lastRenderMs() const { return m.last_render_ms; }
 	uint64_t lastRays() const { return m.last_rays; }
 	uint64_t lastPaths() const { return m.last_paths; }
+	const rtb_adaptive_stats& lastAdaptiveStats() const { return m.last_adaptive; }
 	rtb_renderer* handle() const { return m.r; }
 };

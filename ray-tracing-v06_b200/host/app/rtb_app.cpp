@@ -4,6 +4,7 @@
 //
 //   rtb_app [scene] [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--gpus N]
 //           [--out image.png|image.ppm|image.pfm] [--resume ckpt.rtba] [--checkpoint ckpt.rtba] [--sample-lights]
+//           [--target-db D [--min-spp N]]
 //   rtb_app --obj model.obj [...]     a Wavefront OBJ mesh (MeshHandle) on a checkered floor under the sky
 //
 // scene = one of rtb_scenes_name(i) (default book2_bouncing, which goes through SceneBook2BVH::Factory
@@ -14,6 +15,11 @@
 // radiance sums after the render; --resume loads such a file and renders --spp MORE samples on top of it (single GPU).
 // --sample-lights turns on light importance sampling (rtb_scene_set_sampled_lights) towards the emitters the named scene
 // lists (rtb_scene_info::lights): the same converged image with less noise per sample; refused for scenes that list none.
+// --target-db D samples adaptively (rtb_render_adaptive, DESIGN.md §5c): every pixel gets --min-spp samples (default 64),
+// then more only where its estimated error is above 10^(-D/20), with --spp as the cap per pixel; it prints the rounds, the
+// mean samples per pixel and the render time.  With --resume it continues adaptively from the checkpoint's cursor (a
+// checkpoint written by an adaptive run: it needs the sums of squares), still up to --spp in all.  One GPU only.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -43,6 +49,8 @@ int main(int argc, char** argv) {
 	std::string scene_name = "book2_bouncing", out = "render.ppm", obj_path, resume_path, checkpoint_path;
 	int width = 0, height = 0, spp = 0, depth = 0, gpus = 0;
 	bool sample_lights = false;
+	double target_db = -1.0;
+	int min_spp = 64;
 	uint32_t seed = 1984;   // the reference's seed (Renderer.cu:51, Scenes.cu:190)
 	for (int i = 1; i < argc; ++i) {
 		std::string a = argv[i];
@@ -58,6 +66,8 @@ int main(int argc, char** argv) {
 		else if (a == "--out" && i + 1 < argc) out = argv[++i];
 		else if (a == "--obj" && i + 1 < argc) obj_path = argv[++i];
 		else if (a == "--sample-lights") sample_lights = true;
+		else if (a == "--target-db" && i + 1 < argc) target_db = atof(argv[++i]);
+		else if (a == "--min-spp") min_spp = next();
 		else if (a == "--list") { for (int k = 0; k < rtb_scenes_count(); ++k) printf("%s\n", rtb_scenes_name(k)); return 0; }
 		else scene_name = a;
 	}
@@ -65,6 +75,9 @@ int main(int argc, char** argv) {
 		fprintf(stderr, "rtb_app: --sample-lights: %s lists no lights to sample\n", obj_path.empty() ? scene_name.c_str() : obj_path.c_str());
 		return 1;
 	}
+	const bool adaptive = target_db >= 0.0;
+	const float tolerance = adaptive ? (float)std::pow(10.0, -target_db / 20.0) : 0.0f;
+	if (adaptive && gpus > 1) { fprintf(stderr, "rtb_app: --target-db renders on one GPU (adaptive sampling has no multi-GPU path); drop --gpus %d\n", gpus); return 1; }
 	if (gpus > 1) Renderer::UseGpus(gpus);
 	try {
 		std::vector<glm::vec4> fb; std::vector<uint8_t> rgb8;
@@ -88,6 +101,7 @@ int main(int argc, char** argv) {
 			MotionBlurCamera cam(mid + glm::vec3(0.55f, 0.35f, 1.1f) * size, mid, glm::vec3(0, 1, 0), 40.0f, _width / (float)_height, 0.0f, 1.0f);
 			Renderer renderer = Renderer::MakeRenderer(_width, _height, spp ? spp : 64, depth ? depth : 16, &cam, &world);
 			renderer.SetSeed(seed);
+			if (adaptive) renderer.SetNoiseTarget(tolerance, (uint32_t)min_spp);
 			renderer.Render();
 			fb.resize((size_t)_width * _height); rgb8.resize((size_t)_width * _height * 3);
 			renderer.DownloadRenderbuffer(fb.data()); renderer.DownloadRenderbufferRgb8(rgb8.data());
@@ -103,6 +117,7 @@ int main(int argc, char** argv) {
 			printf("SceneBook2BVH object built.\nMaking Renderer object...\n");
 			Renderer renderer = Renderer::MakeRenderer(_width, _height, spp ? spp : 1, depth ? depth : 4, cam.get(), scene_ptr->getWorldPtr());
 			renderer.SetSeed(seed);
+			if (adaptive) renderer.SetNoiseTarget(tolerance, (uint32_t)min_spp);
 			printf("Renderer object built (%d GPU%s).\nRendering scene...\n", renderer.gpuCount(), renderer.gpuCount() > 1 ? "s" : "");
 			renderer.Render();
 			fb.resize((size_t)_width * _height); rgb8.resize((size_t)_width * _height * 3);
@@ -142,18 +157,32 @@ int main(int argc, char** argv) {
 				rtb_host::check(rtb_renderer_create(&r, 0), "rtb_renderer_create");
 				rtb_host::check(rtb_renderer_set_scene(r, s), "rtb_renderer_set_scene");
 				rtb_host::check(rtb_renderer_set_camera(r, &info.camera), "rtb_renderer_set_camera");
-				if (!resume_path.empty()) {   // continue a checkpointed render: --spp more samples from its cursor on
+				if (!resume_path.empty()) {   // continue a checkpointed render: --spp more samples from its cursor on (adaptive: up to --spp)
 					uint32_t cw = 0, ch = 0, cursor = 0;
 					rtb_host::check(rtb_load_accum(r, resume_path.c_str(), &cw, &ch, &cursor), "rtb_load_accum");
 					if ((int)cw != width || (int)ch != height) { fprintf(stderr, "rtb_app: the checkpoint is %ux%u, the render %dx%d\n", cw, ch, width, height); return 1; }
-					p.sample_begin = cursor; p.sample_end += cursor; p.flags = 0;
+					if (!adaptive) { p.sample_begin = cursor; p.sample_end += cursor; }
+					p.flags = 0;
 					printf("Resuming at sample %u.\n", cursor);
 				}
 				printf("Running render kernel...\n");
-				if (getenv("RTB_APP_WARMUP") && resume_path.empty()) { rtb_host::check(rtb_render(r, &p, nullptr), "rtb_render"); rtb_host::check(rtb_synchronize(r), "rtb_synchronize"); rtb_reset_counters(r); }
-				rtb_host::check(rtb_render(r, &p, nullptr), "rtb_render");
-				rtb_host::check(rtb_synchronize(r), "rtb_synchronize");
-				rtb_get_counters(r, &k);
+				if (adaptive) {
+					rtb_adaptive_params a{tolerance, (uint32_t)min_spp, 0, 0};
+					rtb_adaptive_stats as{};
+					rtb_host::check(rtb_render_adaptive(r, &p, &a, &as, nullptr), "rtb_render_adaptive");
+					rtb_get_counters(r, &k);
+					std::vector<float> acc((size_t)width * height * 4);
+					rtb_host::check(rtb_download_accum(r, acc.data(), nullptr), "rtb_download_accum");
+					double n = 0.0;
+					for (size_t i = 0; i < (size_t)width * height; ++i) n += acc[4 * i + 3];
+					printf("Adaptive: target %.1f dB (tolerance %.3g), %u rounds, mean %.1f spp (cap %u), render %.1f ms.\n",
+					       target_db, tolerance, as.rounds, n / ((double)width * height), p.sample_end, k.render_ms);
+				} else {
+					if (getenv("RTB_APP_WARMUP") && resume_path.empty()) { rtb_host::check(rtb_render(r, &p, nullptr), "rtb_render"); rtb_host::check(rtb_synchronize(r), "rtb_synchronize"); rtb_reset_counters(r); }
+					rtb_host::check(rtb_render(r, &p, nullptr), "rtb_render");
+					rtb_host::check(rtb_synchronize(r), "rtb_synchronize");
+					rtb_get_counters(r, &k);
+				}
 				if (!checkpoint_path.empty()) { rtb_host::check(rtb_save_accum(r, checkpoint_path.c_str()), "rtb_save_accum"); printf("Checkpoint written (%s, %u samples).\n", checkpoint_path.c_str(), rtb_renderer_sample_cursor(r)); }
 				rtb_host::check(rtb_download(r, &fb[0].x), "rtb_download");
 				rtb_host::check(rtb_download_rgb8(r, rgb8.data(), 1), "rtb_download_rgb8");
