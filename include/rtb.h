@@ -136,6 +136,19 @@ int rtb_scene_set_world_bvh(rtb_scene* s, int mode);
 #define RTB_MAX_SAMPLED_LIGHTS 16
 int rtb_scene_set_sampled_lights(rtb_scene* s, const int* objects, int n);
 
+/* HDR environment map (DESIGN.md §5d): an equirectangular map of width x height linear RGB float texels, row 0 at the
+ * top (+y), each channel multiplied by scale[c] when it is set.  While a map is set, every ray that leaves the scene
+ * returns throughput * the nearest texel in its direction instead of the background (which the scene keeps: clearing the
+ * map restores it).  RTB_ENV_SAMPLE adds the map, importance-sampled by luminance x sin(theta), as one more strategy of
+ * the light-sampling mixture at Lambertian and isotropic scatters (with or without a light list); it changes only the
+ * noise, not the expected image.  rgb = NULL with width = height = 0 clears the map.  RTB_ERR_INVALID (scene unchanged):
+ * width or height outside [1, 16384], width x height > 2^24, a texel or scale that is negative, NaN or infinite, unknown
+ * flags, or RTB_ENV_SAMPLE on a map whose sampling weights are all zero.  A scene without a map renders, serialises and
+ * hashes exactly as if this had never been called. */
+#define RTB_ENV_SAMPLE 1
+#define RTB_ENV_MAX_SIZE 16384
+int rtb_scene_set_environment(rtb_scene* s, const float* rgb, int width, int height, const float scale[3], int flags);
+
 int rtb_scene_num_objects(const rtb_scene* s);
 /* Children of a list / BVH / mesh group (1 for translate, rotate_y, constant_medium; 0 for primitives). */
 int rtb_scene_num_children(const rtb_scene* s, int object);

@@ -12,10 +12,12 @@
  *   rtbs_object   [n_objects]
  *   int32         children[n_children]     (LIST / BVH members)
  *   uint8         blob[n_blob_bytes]       (image texels RGB8; Perlin tables)
- *   int32         n_lights                 (version 2 only: the scene's sampled lights,
- *   int32         lights[n_lights]          rtb_scene_set_sampled_lights)
+ *   int32         n_lights                 (versions 2 and 3: the scene's sampled lights,
+ *   int32         lights[n_lights]          rtb_scene_set_sampled_lights; in version 3 n_lights may be 0)
+ *   rtbs_env      env                      (version 3 only: the environment map, rtb_scene_set_environment)
+ *   float         texels[height][width][3]  (row 0 = top; already multiplied by env.scale)
  *
- * A scene without sampled lights is written as version 1; readers accept versions 1 and 2.
+ * A scene without a map is written as version 1 (no sampled lights) or 2; one with a map as version 3.
  */
 #ifndef RTB_SCENE_FORMAT_H
 #define RTB_SCENE_FORMAT_H
@@ -25,6 +27,13 @@
 #define RTBS_MAGIC 0x53425452u /* "RTBS" */
 #define RTBS_VERSION 1u
 #define RTBS_VERSION_LIGHTS 2u
+#define RTBS_VERSION_ENV 3u
+
+typedef struct rtbs_env {
+	int32_t width, height;
+	int32_t flags;              /* RTB_ENV_SAMPLE */
+	float   scale[3];           /* the scale the texels were multiplied by (informational) */
+} rtbs_env;                     /* 24 B */
 
 typedef struct rtbs_header {
 	uint32_t magic, version;

@@ -24,6 +24,7 @@ SCENES_LIB_PATH = _HERE / "librtb200_scenes.so"
 DEBUG_LIB_PATH = _HERE / "librtb200_debug.so"     # the same library built with -DRTB_DEBUG_BOUNDS=1 (select it with RTB_LIB)
 BOUNDS_CLASSES = ("stack", "node", "primitive", "material", "texture", "queue", "path", "bin")   # (light indices count as "primitive")
 MAX_SAMPLED_LIGHTS = 16
+ENV_SAMPLE = 1          # rtb_scene_set_environment flag: importance-sample the map in the light mixture
 
 RTB_OK = 0
 TEX_SOLID, TEX_CHECKER, TEX_IMAGE, TEX_NOISE = 0, 1, 2, 3
@@ -142,6 +143,7 @@ ABI = {
     "rtb_scene_set_background": (C.c_int, [_P, C.c_int, _F3]),
     "rtb_scene_set_world_bvh": (C.c_int, [_P, C.c_int]),
     "rtb_scene_set_sampled_lights": (C.c_int, [_P, C.POINTER(C.c_int), C.c_int]),
+    "rtb_scene_set_environment": (C.c_int, [_P, _P, C.c_int, C.c_int, _F3, C.c_int]),
     "rtb_scene_num_children": (C.c_int, [_P, C.c_int]),
     "rtb_scene_num_objects": (C.c_int, [_P]),
     "rtb_object_bounds": (C.c_int, [_P, C.c_int, _F3]),
@@ -358,6 +360,20 @@ class Scene:
         ids = [int(i) for i in ids]
         arr = (C.c_int * max(len(ids), 1))(*ids)
         _check(lib().rtb_scene_set_sampled_lights(self.handle, arr, len(ids)), "rtb_scene_set_sampled_lights")
+    def set_environment(self, rgb, scale=(1.0, 1.0, 1.0), sample=False):
+        """HDR environment map (rtb_scene_set_environment): an (H, W, 3) float32 equirectangular map, row 0 at the top
+        (+y), multiplied per channel by `scale`; it replaces the background for every ray that leaves the scene.
+        sample=True importance-samples it in the light mixture.  None clears it (the background applies again)."""
+        if rgb is None:
+            _check(lib().rtb_scene_set_environment(self.handle, None, 0, 0, _f3(scale), 0), "rtb_scene_set_environment")
+            return
+        px = np.asarray(rgb)
+        if px.ndim != 3 or px.shape[2] != 3:
+            raise ValueError(f"set_environment: expected an (H, W, 3) array, got shape {px.shape}")
+        px = np.ascontiguousarray(px, dtype=np.float32)
+        h, w = px.shape[:2]
+        _check(lib().rtb_scene_set_environment(self.handle, px.ctypes.data, w, h, _f3(scale), ENV_SAMPLE if sample else 0),
+               "rtb_scene_set_environment")
     def num_objects(self): return lib().rtb_scene_num_objects(self.handle)
 
     def bounds(self, obj) -> np.ndarray:

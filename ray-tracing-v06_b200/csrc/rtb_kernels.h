@@ -37,7 +37,17 @@ struct SceneView {
 	// float4 (type bits, quad area, 0, 0).  n_lights = 0: no light sampling (the kernels without it are launched).
 	const float4* lights;
 	int32_t n_lights;
+	// Environment map (DESIGN.md §5d): env_width x env_height float4 texels (r, g, b, pdf numerator), row 0 = top, then the
+	// marginal CDF (env_height + 1 floats) and env_height conditional CDFs (env_width + 1 floats each).  env = null: no map
+	// (the kernels without one are launched).  env_sample: the map is one more strategy of the light mixture.
+	int32_t env_width;
+	const float4* env;
+	int32_t env_height, env_sample;
 };
+// The map's fields fill the padding after n_lights and add 16 bytes, so every kernel parameter after the SceneView keeps its
+// offset modulo 16 (see BatchParams below for what a moved parameter costs).
+static_assert(alignof(SceneView) == 8 && sizeof(SceneView) == 184 && offsetof(SceneView, n_lights) == 160 &&
+              offsetof(SceneView, env_width) == 164 && offsetof(SceneView, env) == 168, "SceneView layout changed");
 
 // One batch = `samples_per_batch` consecutive samples of every pixel of the row range.
 struct BatchParams {

@@ -374,19 +374,22 @@ extern "C" int rtb_object_bounds(const rtb_scene* s, int object, float out6[6]) 
 
 extern "C" size_t rtb_scene_serialize(const rtb_scene* s, void* buf, size_t cap) {
 	if (!s) return 0;
-	// A scene without sampled lights is written as RTBS v1, byte for byte; one with them as v2 (the list appended).
-	const bool lights = !s->sampled_lights.empty();
+	// A scene without sampled lights or a map is written as RTBS v1, byte for byte; one with lights only as v2 (the list
+	// appended); one with a map as v3 (the list, possibly empty, then the map).
+	const bool env = s->env_width > 0;
+	const bool lights = !s->sampled_lights.empty() || env;
+	const size_t env_floats = env ? (size_t)s->env_width * s->env_height * 3 : 0;
 	size_t need = sizeof(rtbs_header) + s->textures.size() * sizeof(rtbs_texture) + s->materials.size() * sizeof(rtbs_material) +
 	              s->objects.size() * sizeof(rtbs_object) + s->children.size() * 4 + s->blob.size() +
-	              (lights ? 4 + s->sampled_lights.size() * 4 : 0);
+	              (lights ? 4 + s->sampled_lights.size() * 4 : 0) + (env ? sizeof(rtbs_env) + env_floats * 4 : 0);
 	if (!buf || cap < need) return need;
-	rtbs_header h{}; h.magic = RTBS_MAGIC; h.version = lights ? RTBS_VERSION_LIGHTS : RTBS_VERSION;
+	rtbs_header h{}; h.magic = RTBS_MAGIC; h.version = env ? RTBS_VERSION_ENV : lights ? RTBS_VERSION_LIGHTS : RTBS_VERSION;
 	h.n_textures = (uint32_t)s->textures.size(); h.n_materials = (uint32_t)s->materials.size();
 	h.n_objects = (uint32_t)s->objects.size(); h.n_children = (uint32_t)s->children.size();
 	h.n_blob_bytes = (uint32_t)s->blob.size(); h.root_object = s->root; h.background_mode = s->background_mode;
 	memcpy(h.background, s->background, 12);
 	uint8_t* p = static_cast<uint8_t*>(buf);
-	auto put = [&](const void* src, size_t n) { if (n) memcpy(p, src, n); p += n; };
+	auto put = [&p](const void* src, size_t n) { if (n) { memcpy(p, src, n); p += n; } };
 	put(&h, sizeof h);
 	put(s->textures.data(), s->textures.size() * sizeof(rtbs_texture));
 	put(s->materials.data(), s->materials.size() * sizeof(rtbs_material));
@@ -397,6 +400,13 @@ extern "C" size_t rtb_scene_serialize(const rtb_scene* s, void* buf, size_t cap)
 		const int32_t n = (int32_t)s->sampled_lights.size();
 		put(&n, 4);
 		put(s->sampled_lights.data(), s->sampled_lights.size() * 4);
+	}
+	if (env) {
+		rtbs_env e{};
+		e.width = s->env_width; e.height = s->env_height; e.flags = s->env_flags;
+		memcpy(e.scale, s->env_scale, 12);
+		put(&e, sizeof e);
+		put(s->env_rgb.data(), env_floats * 4);
 	}
 	return need;
 }
@@ -1104,6 +1114,10 @@ int flatten(rtb_scene& s, FlatScene& out, const GpuBuildContext* gpu) {
 		if (rc) return rc;
 		out.lights.push_back(rec); out.light_info.push_back(info);
 	}
+	if (s.env_width > 0) {
+		build_env_tables(s.env_rgb.data(), s.env_width, s.env_height, out.env, out.env_cdf);
+		out.env_width = s.env_width; out.env_height = s.env_height; out.env_sample = (s.env_flags & RTB_ENV_SAMPLE) ? 1 : 0;
+	}
 	out.background_mode = s.background_mode;
 	memcpy(out.background, s.background, 12);
 	out.flatten_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_start).count();
@@ -1139,6 +1153,12 @@ extern "C" int rtb_scene_flatten_hash(rtb_scene* s, uint64_t* hash_out) {
 		mix(fs.lights.data(), fs.lights.size() * sizeof(rtb::DevPrim));
 		mix(fs.light_info.data(), fs.light_info.size() * sizeof(rtb::DevLightInfo));
 	}
+	if (!fs.env.empty()) {      // (likewise for the environment map)
+		const int32_t dims[3] = {fs.env_width, fs.env_height, fs.env_sample};
+		mix(dims, sizeof dims);
+		mix(fs.env.data(), fs.env.size() * sizeof(rtb::DevEnvTexel));
+		mix(fs.env_cdf.data(), fs.env_cdf.size() * sizeof(float));
+	}
 	*hash_out = h;
 	return RTB_OK;
 }
@@ -1153,6 +1173,99 @@ extern "C" int rtb_scene_set_sampled_lights(rtb_scene* s, const int* objects, in
 		if (rc) return rc;
 	}
 	s->sampled_lights.assign(objects, objects + n);
+	s->version++;
+	return RTB_OK;
+}
+
+// Environment map (DESIGN.md §5d, "Sampling").  Weights luminance(texel) * sin(theta of the row centre) in double; the CDFs
+// are prefix sums over the total (marginal) or the row sum (conditional), stored as float with the last entry exactly 1.
+// A texel's probability is defined from the stored floats, so that the sampler and the pdf agree.
+namespace {
+double env_row_sin(int j, int H) { return std::sin(3.14159265358979323846 * (j + 0.5) / H); }
+double env_luminance(const float* px) { return 0.2126 * px[0] + 0.7152 * px[1] + 0.0722 * px[2]; }
+}  // namespace
+
+double rtb::env_weight_sum(const float* rgb, int W, int H) {
+	double total = 0.0;
+	for (int j = 0; j < H; ++j) {
+		const double st = env_row_sin(j, H);
+		const float* px = rgb + (size_t)j * W * 3;
+		double acc = 0.0;
+		for (int i = 0; i < W; ++i) acc += env_luminance(px + 3 * i) * st;
+		total += acc;
+	}
+	return total;
+}
+
+void rtb::build_env_tables(const float* rgb, int W, int H, std::vector<DevEnvTexel>& texels, std::vector<float>& cdf) {
+	const double kPi = 3.14159265358979323846;
+	std::vector<double> row(H, 0.0), pre(W);
+	texels.assign((size_t)W * H, DevEnvTexel{});
+	cdf.assign((size_t)(H + 1) + (size_t)H * (W + 1), 0.0f);
+	float* cm = cdf.data();
+	for (int j = 0; j < H; ++j) {
+		const double st = env_row_sin(j, H);
+		const float* px = rgb + (size_t)j * W * 3;
+		double acc = 0.0;
+		for (int i = 0; i < W; ++i) { acc += env_luminance(px + 3 * i) * st; pre[i] = acc; }
+		row[j] = acc;
+		float* cc = cm + (H + 1) + (size_t)j * (W + 1);
+		for (int i = 0; i + 1 < W; ++i) cc[i + 1] = acc > 0.0 ? (float)(pre[i] / acc) : (float)((double)(i + 1) / W);   // (a row of weight 0 is never sampled)
+		cc[0] = 0.0f; cc[W] = 1.0f;
+	}
+	double total = 0.0;
+	for (int j = 0; j < H; ++j) total += row[j];
+	if (total > 0.0) {
+		double acc = 0.0;
+		for (int j = 0; j + 1 < H; ++j) { acc += row[j]; cm[j + 1] = (float)(acc / total); }
+	} else {
+		for (int j = 0; j + 1 < H; ++j) cm[j + 1] = (float)((double)(j + 1) / H);
+	}
+	cm[0] = 0.0f; cm[H] = 1.0f;
+	const double norm = (double)W * (double)H / (2.0 * kPi * kPi);
+	for (int j = 0; j < H; ++j) {
+		const double pj = total > 0.0 ? (double)cm[j + 1] - (double)cm[j] : 0.0;
+		const float* cc = cm + (H + 1) + (size_t)j * (W + 1);
+		for (int i = 0; i < W; ++i) {
+			DevEnvTexel& t = texels[(size_t)j * W + i];
+			const float* px = rgb + ((size_t)j * W + i) * 3;
+			t.r = px[0]; t.g = px[1]; t.b = px[2];
+			t.pdf = (float)(pj * ((double)cc[i + 1] - (double)cc[i]) * norm);
+		}
+	}
+}
+
+extern "C" int rtb_scene_set_environment(rtb_scene* s, const float* rgb, int width, int height, const float scale[3], int flags) {
+	if (!s) return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_environment: null scene");
+	if ((flags & ~RTB_ENV_SAMPLE) != 0) return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_environment: unknown flags");
+	if (!rgb && width == 0 && height == 0) {   // clear: the background applies again
+		s->env_rgb.clear(); s->env_rgb.shrink_to_fit();
+		s->env_width = s->env_height = s->env_flags = 0;
+		s->env_scale[0] = s->env_scale[1] = s->env_scale[2] = 1.0f;
+		s->version++;
+		return RTB_OK;
+	}
+	if (!rgb) return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_environment: null texels (clear with width = height = 0)");
+	if (width < 1 || width > RTB_ENV_MAX_SIZE || height < 1 || height > RTB_ENV_MAX_SIZE || (int64_t)width * height > (int64_t(1) << 24))
+		return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_environment: width and height must be in [1, 16384] with width x height <= 2^24");
+	const float one[3] = {1.0f, 1.0f, 1.0f};
+	const float* sc = scale ? scale : one;
+	for (int c = 0; c < 3; ++c)
+		if (!(sc[c] >= 0.0f) || !std::isfinite(sc[c])) return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_environment: scale must be finite and >= 0");
+	const size_t n = (size_t)width * height * 3;
+	std::vector<float> scaled(n);
+	for (size_t k = 0; k < n; ++k) {
+		const float v = rgb[k];
+		if (!(v >= 0.0f) || !std::isfinite(v))
+			return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_environment: texel " + std::to_string(k / 3) + " is negative, NaN or infinite");
+		scaled[k] = v * sc[k % 3];
+		if (!std::isfinite(scaled[k])) return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_environment: texel " + std::to_string(k / 3) + " overflows when scaled");
+	}
+	if ((flags & RTB_ENV_SAMPLE) && !(rtb::env_weight_sum(scaled.data(), width, height) > 0.0))   // (the total the flattener's tables divide by)
+			return rtb::fail(RTB_ERR_INVALID, "rtb_scene_set_environment: RTB_ENV_SAMPLE on a map whose sampling weights are all zero");
+	s->env_rgb.swap(scaled);
+	s->env_width = width; s->env_height = height; s->env_flags = flags;
+	memcpy(s->env_scale, sc, 12);
 	s->version++;
 	return RTB_OK;
 }

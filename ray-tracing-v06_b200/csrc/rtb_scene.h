@@ -22,6 +22,11 @@ struct rtb_scene {
 	uint64_t version = 0;   // bumped by every mutating call: lets a renderer skip re-flattening an unchanged scene
 	float background[3] = {0, 0, 0};
 	std::vector<int32_t> sampled_lights;   // rtb_scene_set_sampled_lights: object ids (empty: no light sampling)
+	// rtb_scene_set_environment: env_height x env_width x RGB texels already multiplied by env_scale, row 0 = top
+	// (env_width = 0: no map, the background applies).
+	std::vector<float> env_rgb;
+	int32_t env_width = 0, env_height = 0, env_flags = 0;
+	float env_scale[3] = {1, 1, 1};
 
 	// Filled by flatten(): the world BVH in the reference's node layout (parity hook).
 	std::vector<rtb_bvh_node> world_nodes;
@@ -52,6 +57,13 @@ struct GpuBuildContext { int device; void* stream; GpuScratch* scratch; };
 int build_bvh_lbvh_gpu(const std::vector<Box3>& boxes, std::vector<rtb_bvh_node>& nodes, std::vector<int>& order,
                        int& root, const GpuBuildContext& gpu);
 void free_gpu_scratch(GpuScratch& scratch);
+
+// Sampling tables of an environment map (DESIGN.md §5d) from its scaled texels: one DevEnvTexel per texel, then the
+// marginal CDF over rows (height + 1 floats) and one conditional CDF per row (width + 1 floats each).
+void build_env_tables(const float* rgb, int width, int height, std::vector<DevEnvTexel>& texels, std::vector<float>& cdf);
+// The sum of the sampling weights (the total build_env_tables divides by, summed in the same order), without the tables:
+// 0 means the map cannot be sampled.
+double env_weight_sum(const float* rgb, int width, int height);
 
 // Flattens the object graph to world-space primitives + one world BVH.
 int flatten(rtb_scene& s, FlatScene& out, const GpuBuildContext* gpu = nullptr);

@@ -57,6 +57,10 @@ struct alignas(8) DevPrimInfo { int32_t material; int32_t object; };
 // layout), then one DevLightInfo per light.
 struct alignas(16) DevLightInfo { int32_t type; float area; float pad0, pad1; };   // PRIM_SPHERE / PRIM_QUAD; quad area
 
+// Environment map (DESIGN.md §5d): per texel its scaled radiance and the numerator of its pdf per solid angle,
+// p_ij * W * H / (2 pi^2) (the pdf of a direction is this over sin theta).
+struct alignas(16) DevEnvTexel { float r, g, b, pdf; };
+
 struct alignas(16) DevMaterial { int32_t kind, tex; float param, pad; float albedo[4]; };  // 32 B
 
 struct alignas(16) DevTexture {                                                             // 48 B
@@ -79,6 +83,9 @@ struct FlatScene {
 	std::vector<uint8_t> blob;
 	std::vector<DevPrim> lights;         // sampled lights in world space (empty: no light sampling)
 	std::vector<DevLightInfo> light_info;
+	std::vector<DevEnvTexel> env;        // environment map texels, row 0 = top (empty: no map)
+	std::vector<float> env_cdf;          // its marginal CDF (env_height + 1), then env_height conditional CDFs (env_width + 1 each)
+	int32_t env_width = 0, env_height = 0, env_sample = 0;
 	int32_t n_media = 0;
 	int32_t background_mode = 0;
 	float background[3] = {0, 0, 0};

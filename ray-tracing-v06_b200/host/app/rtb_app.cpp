@@ -4,7 +4,7 @@
 //
 //   rtb_app [scene] [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--gpus N]
 //           [--out image.png|image.ppm|image.pfm] [--resume ckpt.rtba] [--checkpoint ckpt.rtba] [--sample-lights]
-//           [--target-db D [--min-spp N]]
+//           [--target-db D [--min-spp N]] [--env map.pfm [--env-scale S] [--sample-env]]
 //   rtb_app --obj model.obj [...]     a Wavefront OBJ mesh (MeshHandle) on a checkered floor under the sky
 //
 // scene = one of rtb_scenes_name(i) (default book2_bouncing, which goes through SceneBook2BVH::Factory
@@ -19,6 +19,9 @@
 // then more only where its estimated error is above 10^(-D/20), with --spp as the cap per pixel; it prints the rounds, the
 // mean samples per pixel and the render time.  With --resume it continues adaptively from the checkpoint's cursor (a
 // checkpoint written by an adaptive run: it needs the sums of squares), still up to --spp in all.  One GPU only.
+// --env map.pfm lights the scene (any named scene or --obj) with an HDR environment map (rtb_scene_set_environment,
+// DESIGN.md §5d): an equirectangular PFM, +y up, which every ray that leaves the scene reads instead of the background;
+// --env-scale S multiplies its texels by S, and --sample-env importance-samples it (same converged image, less noise).
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -51,6 +54,9 @@ int main(int argc, char** argv) {
 	bool sample_lights = false;
 	double target_db = -1.0;
 	int min_spp = 64;
+	std::string env_path;
+	float env_scale = 1.0f;
+	bool sample_env = false;
 	uint32_t seed = 1984;   // the reference's seed (Renderer.cu:51, Scenes.cu:190)
 	for (int i = 1; i < argc; ++i) {
 		std::string a = argv[i];
@@ -68,6 +74,9 @@ int main(int argc, char** argv) {
 		else if (a == "--sample-lights") sample_lights = true;
 		else if (a == "--target-db" && i + 1 < argc) target_db = atof(argv[++i]);
 		else if (a == "--min-spp") min_spp = next();
+		else if (a == "--env" && i + 1 < argc) env_path = argv[++i];
+		else if (a == "--env-scale" && i + 1 < argc) env_scale = (float)atof(argv[++i]);
+		else if (a == "--sample-env") sample_env = true;
 		else if (a == "--list") { for (int k = 0; k < rtb_scenes_count(); ++k) printf("%s\n", rtb_scenes_name(k)); return 0; }
 		else scene_name = a;
 	}
@@ -75,6 +84,20 @@ int main(int argc, char** argv) {
 		fprintf(stderr, "rtb_app: --sample-lights: %s lists no lights to sample\n", obj_path.empty() ? scene_name.c_str() : obj_path.c_str());
 		return 1;
 	}
+	if (sample_env && env_path.empty()) { fprintf(stderr, "rtb_app: --sample-env needs --env map.pfm\n"); return 1; }
+	std::vector<float> env_rgb;
+	int env_w = 0, env_h = 0;
+	if (!env_path.empty()) {
+		std::string err;
+		if (!rtb_host::read_pfm(env_path, env_rgb, env_w, env_h, err)) { fprintf(stderr, "rtb_app: --env: %s\n", err.c_str()); return 1; }
+	}
+	// the map goes on the scene before the renderer flattens it
+	auto set_env = [&](rtb_scene* s) {
+		if (env_rgb.empty()) return;
+		const float scale[3] = {env_scale, env_scale, env_scale};
+		rtb_host::check(rtb_scene_set_environment(s, env_rgb.data(), env_w, env_h, scale, sample_env ? RTB_ENV_SAMPLE : 0), "rtb_scene_set_environment");
+		printf("Environment map %s: %dx%d%s.\n", env_path.c_str(), env_w, env_h, sample_env ? ", sampled" : "");
+	};
 	const bool adaptive = target_db >= 0.0;
 	const float tolerance = adaptive ? (float)std::pow(10.0, -target_db / 20.0) : 0.0f;
 	if (adaptive && gpus > 1) { fprintf(stderr, "rtb_app: --target-db renders on one GPU (adaptive sampling has no multi-GPU path); drop --gpus %d\n", gpus); return 1; }
@@ -99,6 +122,7 @@ int main(int argc, char** argv) {
 			aabb bounds = model.getBounds(); bounds += floor.getBounds();
 			HittableList world(objs, 2, bounds);
 			MotionBlurCamera cam(mid + glm::vec3(0.55f, 0.35f, 1.1f) * size, mid, glm::vec3(0, 1, 0), 40.0f, _width / (float)_height, 0.0f, 1.0f);
+			set_env(rtb_host::scene());   // the scene the mirror's constructors recorded into, before MakeRenderer flattens it
 			Renderer renderer = Renderer::MakeRenderer(_width, _height, spp ? spp : 64, depth ? depth : 16, &cam, &world);
 			renderer.SetSeed(seed);
 			if (adaptive) renderer.SetNoiseTarget(tolerance, (uint32_t)min_spp);
@@ -115,6 +139,7 @@ int main(int argc, char** argv) {
 			SceneBook2BVH::Factory scene_factory{};
 			std::unique_ptr<SceneBook2BVH> scene_ptr(scene_factory.MakeScene());
 			printf("SceneBook2BVH object built.\nMaking Renderer object...\n");
+			set_env(rtb_host::scene());
 			Renderer renderer = Renderer::MakeRenderer(_width, _height, spp ? spp : 1, depth ? depth : 4, cam.get(), scene_ptr->getWorldPtr());
 			renderer.SetSeed(seed);
 			if (adaptive) renderer.SetNoiseTarget(tolerance, (uint32_t)min_spp);
@@ -132,6 +157,7 @@ int main(int argc, char** argv) {
 				rtb_host::check(rtb_scene_set_sampled_lights(s, info.lights, info.n_lights), "rtb_scene_set_sampled_lights");
 				printf("Sampling %d light%s.\n", info.n_lights, info.n_lights > 1 ? "s" : "");
 			}
+			set_env(s);
 			if (!width) width = info.width;
 			if (!height) height = info.height;
 			rtb_render_params p{};

@@ -1,4 +1,5 @@
-// image_write.h — the output stage after the renderer: PNG / PPM (8-bit) and PFM (float) writers.
+// image_write.h — the output stage after the renderer: PNG / PPM (8-bit) and PFM (float) writers, and the PFM reader
+// that loads environment maps.
 //
 // The reference writes a JPG through stb_image_write (write_renderbuffer, main/src/FirstApp.cpp:108-122: uint8 =
 // value * 255.999f, RGB, stbi_flip_vertically_on_write(true), quality 95).  The vendored stb header is MSVC-only
@@ -8,6 +9,7 @@
 #pragma once
 #include <cstdint>
 #include <cstdio>
+#include <cstring>
 #include <string>
 #include <vector>
 
@@ -79,6 +81,35 @@ inline bool write_pfm(const std::string& path, uint32_t width, uint32_t height, 
 	fprintf(f, "PF\n%u %u\n-1.0\n", width, height);
 	for (size_t i = 0; i < (size_t)width * height; ++i) fwrite(rgba + 4 * i, sizeof(float), 3, f);
 	return fclose(f) == 0;
+}
+
+// PFM reader (colour "PF" or greyscale "Pf", either byte order): rgb = height rows x width x RGB with row 0 = TOP (PFM
+// stores rows bottom-up, so they are flipped; a greyscale map is spread to three channels).  false with `err` set on a file
+// that is missing, truncated or not a PFM.
+inline bool read_pfm(const std::string& path, std::vector<float>& rgb, int& width, int& height, std::string& err) {
+	FILE* f = fopen(path.c_str(), "rb");
+	if (!f) { err = "cannot open " + path; return false; }
+	char kind[3] = {0, 0, 0};
+	double scale = 0.0;
+	width = height = 0;
+	const bool ok_header = fscanf(f, "%2s %d %d %lf", kind, &width, &height, &scale) == 4 && fgetc(f) != EOF;   // (one whitespace byte ends the header)
+	const int ch = kind[0] == 'P' && kind[1] == 'F' ? 3 : (kind[0] == 'P' && kind[1] == 'f' ? 1 : 0);
+	if (!ok_header || ch == 0 || width <= 0 || height <= 0 || scale == 0.0 || (int64_t)width * height > (int64_t(1) << 28)) {
+		fclose(f); err = path + " is not a PFM image"; return false;
+	}
+	std::vector<float> raw((size_t)width * height * ch);
+	const size_t got = fread(raw.data(), sizeof(float), raw.size(), f);
+	fclose(f);
+	if (got != raw.size()) { err = path + ": truncated PFM data"; return false; }
+	if (scale > 0.0) {   // big-endian file
+		for (float& v : raw) { uint32_t u; memcpy(&u, &v, 4); u = __builtin_bswap32(u); memcpy(&v, &u, 4); }
+	}
+	rgb.resize((size_t)width * height * 3);
+	for (int y = 0; y < height; ++y)
+		for (int x = 0; x < width; ++x)
+			for (int c = 0; c < 3; ++c)
+				rgb[((size_t)y * width + x) * 3 + c] = raw[((size_t)(height - 1 - y) * width + x) * ch + (ch == 3 ? c : 0)];
+	return true;
 }
 
 inline bool has_suffix(const std::string& s, const char* suf) { const std::string t(suf); return s.size() >= t.size() && s.compare(s.size() - t.size(), t.size(), t) == 0; }

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""SASS of the dense kernel instantiations of two builds of rtb_kernels.o, function by function (cuobjdump -sass):
-identical, identical apart from constant-bank parameter offsets (c[0x0][...]), or different (with a short diff).  Kernels
-that gained a LIST template parameter are matched to their dense (LIST = false) instantiation; list-mode and adaptive
-kernels are skipped.
+"""SASS of the kernel instantiations of two builds of rtb_kernels.o, function by function (cuobjdump -sass): identical,
+identical apart from constant-bank parameter offsets (c[0x0][...]), or different (with a short diff).  Every kernel of the
+old build is compared with the new build's instantiation of the same name, or, where the new build added template
+parameters at the end (LIST, ENV), with the one whose added parameters are all false.  Instantiations only the new build
+has are listed at the end.
 
     python tools/sass_diff.py OLD/build/rtb_kernels.o NEW/build/rtb_kernels.o
 """
@@ -26,13 +27,16 @@ def funcs(obj):
 def dem(n):
     return subprocess.run(["c++filt", n], capture_output=True, text=True).stdout.strip()
 
-def norm_name(d, new):
-    d = re.sub(r"^void ", "", d)
-    d = d.split("(")[0]
-    if new:
-        d = re.sub(r"<false>$", "", d) if re.search(r"(generate_kernel|accumulate_kernel)<false>$", d) else d
-        d = re.sub(r", false>$", ">", d) if re.search(r"(traverse_kernel|shade_kernel|tail_kernel)<", d) else d
-    return d
+def base_name(d):
+    return re.sub(r"^void ", "", d).split("(")[0]
+
+def strip_false(d):
+    """The name with its last template argument removed when that argument is false (None otherwise)."""
+    if d.endswith("<false>"):
+        return d[: -len("<false>")]
+    if d.endswith(", false>"):
+        return d[: -len(", false>")] + ">"
+    return None
 
 def norm_ins(s):
     s = re.sub(r"c\[0x0\]\[0x[0-9a-f]+\]", "c[0x0][P]", s)
@@ -40,13 +44,17 @@ def norm_ins(s):
     return s
 
 old, new = funcs(sys.argv[1]), funcs(sys.argv[2])
-oldn = {norm_name(dem(k), False): v for k, v in old.items()}
-newn = {}
+oldn = {base_name(dem(k)): v for k, v in old.items()}
+newn, extra = {}, []
 for k, v in new.items():
-    d = dem(k)
-    if (re.search(r"(traverse_kernel|shade_kernel|tail_kernel)<.*, true>", d) or re.search(r"(generate_kernel|accumulate_kernel)<true>", d) or "adaptive_" in d):
-        continue
-    newn[norm_name(d, True)] = v
+    d = base_name(dem(k))
+    m = d
+    while m is not None and m not in oldn:
+        m = strip_false(m)
+    if m is None or m in newn:
+        extra.append(d)
+    else:
+        newn[m] = v
 same = diff_params = diff = 0
 for k, v in sorted(oldn.items()):
     if k not in newn:
@@ -61,6 +69,6 @@ for k, v in sorted(oldn.items()):
         import difflib
         d = list(difflib.unified_diff([norm_ins(x) for x in v], [norm_ins(x) for x in w], lineterm="", n=1))
         print("DIFF", k, len(v), len(w)); print("\n".join(d[:30]))
-for k in sorted(set(newn) - set(oldn)):
-    print("NEW dense-named function:", k)
-print(f"dense kernels: {len(oldn)}; identical {same}; identical apart from parameter offsets {diff_params}; different {diff}")
+for k in sorted(extra):
+    print("only in new:", k)
+print(f"kernels of the old build: {len(oldn)}; identical {same}; identical apart from parameter offsets {diff_params}; different {diff}")
