@@ -104,6 +104,17 @@ int rtb_add_bvh(rtb_scene* s, const int* children, int n, int builder);
  * objects rtb_add_triangle + rtb_add_bvh would make (the reference has no mesh type; its GL demo loads OBJ files through
  * tiny_obj, main/src/gl_engine/gl_mesh.cpp:124-218). */
 int rtb_add_mesh(rtb_scene* s, const float* vertices, int n_vertices, const int* indices, int n_triangles, int mat);
+/* rtb_add_mesh with per-vertex attributes (DESIGN.md §5e): `normals` = n_vertices x (x, y, z) shading normals, `uvs` =
+ * n_vertices x (u, v) texture coordinates, either or both NULL.  Makes the same triangles under the same BVH group as
+ * rtb_add_mesh (the same faces are dropped); each triangle also carries its three corners' attributes.  With normals, a hit
+ * is shaded with the normal interpolated from its corners (normalised, put on the face normal's side, facing the ray);
+ * front_face and the dielectric's inside / outside test stay with the face normal.  With UVs, textures read the
+ * interpolated (u, v) instead of the triangle's own (alpha, beta).  Normals are normalised on the host in double; zero
+ * normals are kept (the face normal is used where all three corners interpolate to zero).  No correction for shading-normal
+ * artefacts is applied.  With both NULL this is rtb_add_mesh exactly.  RTB_ERR_INVALID (scene unchanged): everything
+ * rtb_add_mesh refuses, and a non-finite normal or UV component. */
+int rtb_add_mesh_ex(rtb_scene* s, const float* vertices, int n_vertices, const int* indices, int n_triangles,
+                    const float* normals, const float* uvs, int mat);
 int rtb_add_translate(rtb_scene* s, int child, const float offset[3]);
 int rtb_add_rotate_y(rtb_scene* s, int child, float degrees);
 int rtb_add_constant_medium(rtb_scene* s, int boundary, float density, int phase_mat);
@@ -351,9 +362,10 @@ typedef struct rtb_hit {                                                        
 	int32_t object;       /* scene-graph object id of the primitive */
 	int32_t material;
 	float   p[3];
-	float   n[3];         /* the normal materials see (spheres: outward; quads: facing the ray) */
+	float   n[3];         /* the normal materials see (spheres: outward; quads: facing the ray; triangles with normals:
+	                         the interpolated shading normal, facing the ray) */
 	int32_t front_face;   /* dot(d, geometric normal) <= 0 */
-	float   u, v;
+	float   u, v;         /* texture coordinates (triangles with UVs: the interpolated ones) */
 	int32_t nodes_visited;   /* traversal statistics of this ray (rtb_trace_rays only): inner nodes visited, */
 	int32_t prims_tested;    /* primitives intersected */
 	int32_t pad;

@@ -14,10 +14,14 @@
  *   uint8         blob[n_blob_bytes]       (image texels RGB8; Perlin tables)
  *   int32         n_lights                 (versions 2 and 3: the scene's sampled lights,
  *   int32         lights[n_lights]          rtb_scene_set_sampled_lights; in version 3 n_lights may be 0)
- *   rtbs_env      env                      (version 3 only: the environment map, rtb_scene_set_environment)
- *   float         texels[height][width][3]  (row 0 = top; already multiplied by env.scale)
+ *   rtbs_env      env                      (versions 3 and 4: the environment map, rtb_scene_set_environment;
+ *   float         texels[height][width][3]  in version 4 width = height = 0 when there is none; row 0 = top; already
+ *                                            multiplied by env.scale)
+ *   uint32        n_tri_attrs              (version 4 only: per-vertex attributes of mesh triangles, rtb_add_mesh_ex)
+ *   rtbs_tri_attr tri_attrs[n_tri_attrs]    (a TRIANGLE object whose `aux` is k + 1 carries tri_attrs[k]; aux = 0: none)
  *
- * A scene without a map is written as version 1 (no sampled lights) or 2; one with a map as version 3.
+ * A scene without attributes is written as version 1 (no sampled lights), 2 or 3 (a map); one with attributes as
+ * version 4.
  */
 #ifndef RTB_SCENE_FORMAT_H
 #define RTB_SCENE_FORMAT_H
@@ -28,6 +32,17 @@
 #define RTBS_VERSION 1u
 #define RTBS_VERSION_LIGHTS 2u
 #define RTBS_VERSION_ENV 3u
+#define RTBS_VERSION_ATTR 4u
+
+/* Corner attributes of one triangle (DESIGN.md §5e), in the order of its corners v0 (= Q), v1 (= Q + u), v2 (= Q + v).
+ * Normals are unit length or zero (normalised on the host); flags say which of the two are present. */
+#define RTBS_ATTR_NORMALS 1
+#define RTBS_ATTR_UVS 2
+typedef struct rtbs_tri_attr {
+	float   n[3][3];            /* corner normals (object frame of the triangle) */
+	float   uv[3][2];           /* corner texture coordinates */
+	int32_t flags;              /* RTBS_ATTR_NORMALS | RTBS_ATTR_UVS */
+} rtbs_tri_attr;                /* 64 B */
 
 typedef struct rtbs_env {
 	int32_t width, height;

@@ -136,6 +136,7 @@ ABI = {
     "rtb_add_list": (C.c_int, [_P, C.POINTER(C.c_int), C.c_int]),
     "rtb_add_bvh": (C.c_int, [_P, C.POINTER(C.c_int), C.c_int, C.c_int]),
     "rtb_add_mesh": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int]),
+    "rtb_add_mesh_ex": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P, C.c_int]),
     "rtb_add_translate": (C.c_int, [_P, C.c_int, _F3]),
     "rtb_add_rotate_y": (C.c_int, [_P, C.c_int, C.c_float]),
     "rtb_add_constant_medium": (C.c_int, [_P, C.c_int, C.c_float, C.c_int]),
@@ -343,10 +344,21 @@ class Scene:
     def bvh(self, children, builder=BVH_TOPDOWN_MEDIAN):
         arr = (C.c_int * len(children))(*children)
         return _check(lib().rtb_add_bvh(self.handle, arr, len(children), builder), "rtb_add_bvh")
-    def mesh(self, vertices, indices, mat):
-        """Triangle mesh from (n, 3) float32 vertices and (m, 3) int32 vertex indices: one BVH group of triangles."""
+    def mesh(self, vertices, indices, mat, normals=None, uvs=None):
+        """Triangle mesh from (n, 3) float32 vertices and (m, 3) int32 vertex indices: one BVH group of triangles.
+        normals (n, 3) and uvs (n, 2), per vertex, make it smooth-shaded and texture-mapped (rtb_add_mesh_ex,
+        DESIGN.md §5e)."""
         v = np.ascontiguousarray(vertices, dtype=np.float32).reshape(-1, 3); i = np.ascontiguousarray(indices, dtype=np.int32).reshape(-1, 3)
-        return _check(lib().rtb_add_mesh(self.handle, v.ctypes.data, len(v), i.ctypes.data, len(i), mat), "rtb_add_mesh")
+        if normals is None and uvs is None:
+            return _check(lib().rtb_add_mesh(self.handle, v.ctypes.data, len(v), i.ctypes.data, len(i), mat), "rtb_add_mesh")
+        n = None if normals is None else np.ascontiguousarray(normals, dtype=np.float32).reshape(-1, 3)
+        t = None if uvs is None else np.ascontiguousarray(uvs, dtype=np.float32).reshape(-1, 2)
+        for name, a in (("normals", n), ("uvs", t)):
+            if a is not None and len(a) != len(v):
+                raise ValueError(f"mesh: {name} has {len(a)} rows for {len(v)} vertices")
+        return _check(lib().rtb_add_mesh_ex(self.handle, v.ctypes.data, len(v), i.ctypes.data, len(i),
+                                            None if n is None else n.ctypes.data, None if t is None else t.ctypes.data, mat),
+                      "rtb_add_mesh_ex")
 
     def translate(self, child, off): return _check(lib().rtb_add_translate(self.handle, child, _f3(off)), "rtb_add_translate")
     def rotate_y(self, child, deg): return _check(lib().rtb_add_rotate_y(self.handle, child, deg), "rtb_add_rotate_y")

@@ -15,6 +15,7 @@
 
 #include <cfloat>
 
+#include "../../include/rtb_scene_format.h"
 #include "rtb_types.h"
 #include "rtmath.h"
 
@@ -670,10 +671,15 @@ traverse_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, i
 // ------------------------------------------------------------------------------------------------
 // surface reconstruction + textures + materials
 
-struct Surface { v3 p, n_shade, n_geom; float u, v; };
+// n_diel (ATTR only): the normal the dielectric refracts about - the shading normal on the geometric normal's side
+// (DESIGN.md §5e); the geometric normal itself everywhere else.
+struct Surface { v3 p, n_shade, n_geom, n_diel; float u, v; };
 
 // What Sphere::getNormal / MovingSphere::getNormal hand to materials: the outward normal
 // (p - c) / r, never flipped (SphereHittable.cu:43-50,64,100).  Quads face the ray (book).
+// ATTR: the scene has triangle attributes; a triangle that carries them is shaded with its interpolated normal and reads its
+// interpolated UVs (DESIGN.md §5e), in its own frame, before the instance transform.
+template <bool ATTR>
 __device__ __forceinline__ void reconstruct(const SceneView& sv, int code, v3 o, v3 d, float time, float t, bool want_uv, Surface& s) {
 	const int type = code & 15, base = type & 7;
 	const bool xf = (type & PRIM_XF) != 0;
@@ -685,6 +691,7 @@ __device__ __forceinline__ void reconstruct(const SceneView& sv, int code, v3 o,
 	if (type == PRIM_MEDIUM_SPHERE || type == PRIM_MEDIUM_BOX) {   // normal arbitrary (book constant_medium::hit)
 		s.n_geom = rt::mk(1.0f, 0.0f, 0.0f);
 		s.n_shade = s.n_geom;
+		if (ATTR) s.n_diel = s.n_geom;
 		return;
 	}
 	v3 oo = o, dd = d;                // the ray in the primitive's own frame
@@ -702,17 +709,47 @@ __device__ __forceinline__ void reconstruct(const SceneView& sv, int code, v3 o,
 		}
 		if (xf) n = xf_vec_to_world(tp, n);
 		s.n_geom = n; s.n_shade = n;
+		if (ATTR) s.n_diel = n;
 	} else {
 		const float4 q1 = ldg4(pp + 1), q2 = ldg4(pp + 2), q3 = ldg4(pp + 3);
 		v3 N = rt::mk(q1.w, q2.w, q3.w);
 		v3 ns = rt::dot(dd, N) > 0.0f ? rt::neg(N) : N;             // book set_face_normal
-		if (want_uv) {
+		v3 m = N;
+		int ai = -1;
+		if (ATTR && base == PRIM_TRIANGLE) {
+			ai = __ldg(sv.attr_slot + (code >> RTB_LEAF_TYPE_BITS));
+			RTB_CHECK(ai >= -1 && ai < sv.n_tri_attr, RTB_BOUNDS_PRIM);
+		}
+		if (ATTR && ai >= 0) {
+			// (alpha, beta) always: the normal needs them.  x interpolates as fma(x2, beta, fma(x1, alpha, x0 * w)).
+			const v3 planar = rt::sub(rt::madd(dd, t, oo), xyz(q0));
+			const float alpha = rt::dot(xyz(q3), rt::cross(planar, xyz(q2)));
+			const float beta = rt::dot(xyz(q3), rt::cross(xyz(q1), planar));
+			const float w = (1.0f - alpha) - beta;
+			const float4* ap = sv.tri_attr + 4 * (size_t)ai;
+			const float4 a0 = ldg4(ap), a1 = ldg4(ap + 1), a2 = ldg4(ap + 2), a3 = ldg4(ap + 3);
+			const uint32_t flags = __float_as_uint(a3.w);
+			if (flags & RTBS_ATTR_NORMALS) {
+				m = rt::mk(fmaf(a2.x, beta, fmaf(a1.x, alpha, a0.x * w)), fmaf(a2.y, beta, fmaf(a1.y, alpha, a0.y * w)),
+				           fmaf(a2.z, beta, fmaf(a1.z, alpha, a0.z * w)));
+				m = rt::dot(m, m) > 0.0f ? rt::normalize(m) : N;
+				if (rt::dot(m, N) < 0.0f) m = rt::neg(m);                  // on the face normal's side
+				ns = rt::dot(dd, N) > 0.0f ? rt::neg(m) : m;               // set_face_normal with m in place of N
+			}
+			if (flags & RTBS_ATTR_UVS) {
+				s.u = fmaf(a3.y, beta, fmaf(a2.w, alpha, a0.w * w));
+				s.v = fmaf(a3.z, beta, fmaf(a3.x, alpha, a1.w * w));
+			} else {
+				s.u = alpha; s.v = beta;
+			}
+		} else if (want_uv) {
 			v3 planar = rt::sub(rt::madd(dd, t, oo), xyz(q0));
 			s.u = rt::dot(xyz(q3), rt::cross(planar, xyz(q2)));
 			s.v = rt::dot(xyz(q3), rt::cross(xyz(q1), planar));
 		}
-		if (xf) { N = xf_vec_to_world(tp, N); ns = xf_vec_to_world(tp, ns); }
+		if (xf) { N = xf_vec_to_world(tp, N); ns = xf_vec_to_world(tp, ns); if (ATTR) m = xf_vec_to_world(tp, m); }
 		s.n_geom = N; s.n_shade = ns;
+		if (ATTR) s.n_diel = m;
 	}
 }
 
@@ -921,7 +958,8 @@ __device__ __forceinline__ bool light_mix(const SceneView& sv, const Surface& s,
 // With DEFER, an image / noise albedo of a scattering material is not evaluated here: attenuation is
 // left at 1 and defer_tex names the texture, to be multiplied in later by texture_kernel (dense warps).
 // With LIGHTS, Lambertian and isotropic scatters draw from the light mixture and set w (1 otherwise); ENV: with the map.
-template <bool DEFER, bool LIGHTS, bool ENV>
+// ATTR: the dielectric refracts about s.n_diel (its inside / outside test stays with the geometric normal).
+template <bool DEFER, bool LIGHTS, bool ENV, bool ATTR>
 __device__ __forceinline__ int scatter(const SceneView& sv, int mat, const Surface& s, v3 d, const rt::f4& r, const LightKey& lk,
                                        v3& dir, v3& att, float& w, int& defer_tex) {
 	RTB_CHECK(mat >= 0 && mat < sv.n_materials, RTB_BOUNDS_MATERIAL);
@@ -951,6 +989,7 @@ __device__ __forceinline__ int scatter(const SceneView& sv, int mat, const Surfa
 	case RTB_MAT_DIELECTRIC: {   // DielectricAbstract  cu_materials.cuh:115-143, reflectance :99-104
 		v3 n = s.n_geom;
 		bool back = rt::dot(d, n) > 0.0f;          // isBackfacing  ray_data.cuh:44-46
+		if (ATTR) n = s.n_diel;
 		if (back) n = rt::neg(n);
 		float ratio = back ? param : 1.0f / param;
 		v3 ud = rt::normalize(d);
@@ -997,8 +1036,8 @@ __device__ __forceinline__ v3 background(const SceneView& sv, v3 d) {
 // been written to contrib[path].
 struct DeferredTex { int tex; float u, v; v3 p; };
 
-// ENV: a miss returns the environment map's texel instead of the background.
-template <bool DEFER, bool LIGHTS, bool LIST, bool ENV>
+// ENV: a miss returns the environment map's texel instead of the background.  ATTR: the scene has triangle attributes.
+template <bool DEFER, bool LIGHTS, bool LIST, bool ENV, bool ATTR>
 __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t batch, uint32_t bounce,
                                               const float4& fo, const float4& fd, v3 thr, float t, int code,
                                               float4& no, float4& nd, v3& nthr, DeferredTex& dt) {
@@ -1016,13 +1055,13 @@ __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchPa
 	RTB_CHECK(path < wv.capacity, RTB_BOUNDS_PATH);
 	const int tex = __float_as_int(ldg4(sv.materials + 2 * info.x).y);
 	Surface s;
-	reconstruct(sv, code, o, d, fo.w, t, texture_needs_uv(sv, tex), s);
+	reconstruct<ATTR>(sv, code, o, d, fo.w, t, texture_needs_uv(sv, tex), s);
 	uint32_t pixel, sample;
 	path_pixel_sample<LIST>(bp, batch, path, pixel, sample);
 	const rt::f4 r = rt::rng4(bp.seed, pixel, sample, bounce, rt::STREAM_SCATTER);
 	v3 dir, att;
 	float w = 1.0f;
-	const int res = scatter<DEFER, LIGHTS, ENV>(sv, info.x, s, d, r, LightKey{bp.seed, pixel, sample, bounce}, dir, att, w, dt.tex);
+	const int res = scatter<DEFER, LIGHTS, ENV, ATTR>(sv, info.x, s, d, r, LightKey{bp.seed, pixel, sample, bounce}, dir, att, w, dt.tex);
 	dt.u = s.u; dt.v = s.v; dt.p = s.p;
 	if (res == 2) {                                       // emitter: throughput * emitted, path ends
 		v3 c = rt::mulv(thr, att);
@@ -1105,7 +1144,7 @@ __device__ __forceinline__ void bin_table_flush(uint32_t* s_key, uint32_t* s_cnt
 #ifndef SHADE_MIN_BLOCKS
 #define SHADE_MIN_BLOCKS 8   // 8 x 128 threads x 64 registers = the whole register file (6 / 9 / 10 blocks: 11.7 / 10.9 / 12.4 ms)
 #endif
-template <bool LIGHTS, bool LIST, bool ENV>
+template <bool LIGHTS, bool LIST, bool ENV, bool ATTR>
 __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS)
 shade_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int q) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -1136,7 +1175,7 @@ shade_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int 
 			float4 fo, fd; ld_ray(rod + 2 * (size_t)i, fo, fd);
 			const float4 ft = ldq(rt_ + i);
 			const int2 h = ldq(wv.hit + i);
-			alive = shade_segment<true, LIGHTS, LIST, ENV>(sv, bp, wv, batch, bounce, fo, fd, xyz(ft), __int_as_float(h.x), h.y, no, nd, nthr, dt);
+			alive = shade_segment<true, LIGHTS, LIST, ENV, ATTR>(sv, bp, wv, batch, bounce, fo, fd, xyz(ft), __int_as_float(h.x), h.y, no, nd, nthr, dt);
 		}
 		// live-path compaction: warp ballot/popc, one global atomic per block
 		const uint32_t mask = __ballot_sync(FULL_MASK, alive);
@@ -1338,7 +1377,7 @@ bin_permute_kernel(SceneView sv, WaveView wv, uint32_t bounce, int q_from) {
 // One persistent launch then runs every remaining path to completion (traverse + shade fused, one
 // thread per path); later traverse/shade launches of the batch see tail_from and return at once.
 
-template <bool MEDIA, int STACK, bool LIGHTS, bool LIST, bool ENV>
+template <bool MEDIA, int STACK, bool LIGHTS, bool LIST, bool ENV, bool ATTR>
 __global__ void __launch_bounds__(TRAVERSE_THREADS)
 tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int q, uint32_t threshold) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -1364,7 +1403,7 @@ tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int 
 			trace_ray<(MEDIA ? 2 : 0)>(sv, xyz(fo), xyz(fd), fo.w, mr, s_stack + threadIdx.x, STACK, t, code);
 			float4 no, nd; v3 nthr;
 			DeferredTex dt;
-			if (!shade_segment<false, LIGHTS, LIST, ENV>(sv, bp, wv, batch, b, fo, fd, thr, t, code, no, nd, nthr, dt)) break;
+			if (!shade_segment<false, LIGHTS, LIST, ENV, ATTR>(sv, bp, wv, batch, b, fo, fd, thr, t, code, no, nd, nthr, dt)) break;
 			fo = no; fd = nd; thr = nthr;
 		}
 	}
@@ -1601,7 +1640,8 @@ hit_record_kernel(SceneView sv, const float4* __restrict__ ro, const float4* __r
 			const float4 fo = ro[i], fd = rd[i];
 			const int2 info = __ldg(sv.prim_info + (h.y >> RTB_LEAF_TYPE_BITS));
 			Surface s;
-			reconstruct(sv, h.y, xyz(fo), xyz(fd), fo.w, r.t, true, s);
+			if (sv.tri_attr) reconstruct<true>(sv, h.y, xyz(fo), xyz(fd), fo.w, r.t, true, s);
+			else reconstruct<false>(sv, h.y, xyz(fo), xyz(fd), fo.w, r.t, true, s);
 			r.prim = h.y >> RTB_LEAF_TYPE_BITS; r.object = info.y; r.material = info.x;
 			r.p[0] = s.p.x; r.p[1] = s.p.y; r.p[2] = s.p.z;
 			r.n[0] = s.n_shade.x; r.n[1] = s.n_shade.y; r.n[2] = s.n_shade.z;
@@ -1633,12 +1673,12 @@ void query_occupancy(int device, LaunchCfg& lc) {
 	int occ_t = 0, occ_tm = 0, occ_s = 0, occ_g = 0;
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_t, traverse_kernel<0, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_tm, traverse_kernel<2, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, shade_kernel<false, false, false>, SHADE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, shade_kernel<false, false, false, false>, SHADE_THREADS, 0);
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_g, generate_kernel<false>, STREAM_THREADS, 0);
 	int occ_trav = occ_t < occ_tm ? occ_t : occ_tm;
 	int occ_l = 0, occ_lm = 0;
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_l, tail_kernel<false, STACK_SIZE, false, false, false>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_lm, tail_kernel<true, STACK_SIZE, false, false, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_l, tail_kernel<false, STACK_SIZE, false, false, false, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_lm, tail_kernel<true, STACK_SIZE, false, false, false, false>, TRAVERSE_THREADS, 0);
 	int occ_tail = occ_l < occ_lm ? occ_l : occ_lm;
 	lc.blocks_tail = sms * (occ_tail > 0 ? occ_tail : 1);
 	lc.sms = sms;
@@ -1673,41 +1713,49 @@ void launch_traverse(const SceneView& sv, const BatchParams& bp, const WaveView&
 }
 void launch_tail(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t bounce, int q, uint32_t threshold, const LaunchCfg& lc, cudaStream_t st) {
 	const bool deep = sv.tree_depth > STACK_SIZE - 2;
-	// (light sampling and the environment map: their own instantiations, so the kernels of scenes without them stay as they
-	// were; a sampled map is a light-mixture strategy, so it needs the LIGHTS kernels even without a light list)
+	// (light sampling, the environment map and triangle attributes: their own instantiations, so the kernels of scenes without
+	// them stay as they were; a sampled map is a light-mixture strategy, so it needs the LIGHTS kernels even without a light list)
 	const bool lights = sv.n_lights > 0 || (sv.env && sv.env_sample);
-#define RTB_LAUNCH_TAIL(M, L, P, E) \
-	do { if (deep) tail_kernel<M, DEEP_STACK_SIZE, L, P, E><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); \
-	     else tail_kernel<M, STACK_SIZE, L, P, E><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); } while (0)
-#define RTB_LAUNCH_TAIL_LM(P, E) \
+#define RTB_LAUNCH_TAIL(M, L, P, E, A) \
+	do { if (deep) tail_kernel<M, DEEP_STACK_SIZE, L, P, E, A><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); \
+	     else tail_kernel<M, STACK_SIZE, L, P, E, A><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); } while (0)
+#define RTB_LAUNCH_TAIL_LM(P, E, A) \
 	do { if (lights) { \
-	         if (sv.has_media) RTB_LAUNCH_TAIL(true, true, P, E); \
-	         else RTB_LAUNCH_TAIL(false, true, P, E); \
+	         if (sv.has_media) RTB_LAUNCH_TAIL(true, true, P, E, A); \
+	         else RTB_LAUNCH_TAIL(false, true, P, E, A); \
 	     } else { \
-	         if (sv.has_media) RTB_LAUNCH_TAIL(true, false, P, E); \
-	         else RTB_LAUNCH_TAIL(false, false, P, E); \
+	         if (sv.has_media) RTB_LAUNCH_TAIL(true, false, P, E, A); \
+	         else RTB_LAUNCH_TAIL(false, false, P, E, A); \
 	     } } while (0)
-	if (sv.env) {
-		if (bp.pixel_list()) RTB_LAUNCH_TAIL_LM(true, true);
-		else RTB_LAUNCH_TAIL_LM(false, true);
-	} else {
-		if (bp.pixel_list()) RTB_LAUNCH_TAIL_LM(true, false);
-		else RTB_LAUNCH_TAIL_LM(false, false);
-	}
+#define RTB_LAUNCH_TAIL_PE(A) \
+	do { if (sv.env) { \
+	         if (bp.pixel_list()) RTB_LAUNCH_TAIL_LM(true, true, A); \
+	         else RTB_LAUNCH_TAIL_LM(false, true, A); \
+	     } else { \
+	         if (bp.pixel_list()) RTB_LAUNCH_TAIL_LM(true, false, A); \
+	         else RTB_LAUNCH_TAIL_LM(false, false, A); \
+	     } } while (0)
+	if (sv.tri_attr) RTB_LAUNCH_TAIL_PE(true);
+	else RTB_LAUNCH_TAIL_PE(false);
+#undef RTB_LAUNCH_TAIL_PE
 #undef RTB_LAUNCH_TAIL_LM
 #undef RTB_LAUNCH_TAIL
 }
 void launch_shade(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t bounce, int q, const LaunchCfg& lc, cudaStream_t st) {
 	const bool lights = sv.n_lights > 0 || (sv.env && sv.env_sample);
-#define RTB_LAUNCH_SHADE(L, P, E) shade_kernel<L, P, E><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q)
-#define RTB_LAUNCH_SHADE_L(P, E) do { if (lights) RTB_LAUNCH_SHADE(true, P, E); else RTB_LAUNCH_SHADE(false, P, E); } while (0)
-	if (sv.env) {
-		if (bp.pixel_list()) RTB_LAUNCH_SHADE_L(true, true);
-		else RTB_LAUNCH_SHADE_L(false, true);
-	} else {
-		if (bp.pixel_list()) RTB_LAUNCH_SHADE_L(true, false);
-		else RTB_LAUNCH_SHADE_L(false, false);
-	}
+#define RTB_LAUNCH_SHADE(L, P, E, A) shade_kernel<L, P, E, A><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q)
+#define RTB_LAUNCH_SHADE_L(P, E, A) do { if (lights) RTB_LAUNCH_SHADE(true, P, E, A); else RTB_LAUNCH_SHADE(false, P, E, A); } while (0)
+#define RTB_LAUNCH_SHADE_PE(A) \
+	do { if (sv.env) { \
+	         if (bp.pixel_list()) RTB_LAUNCH_SHADE_L(true, true, A); \
+	         else RTB_LAUNCH_SHADE_L(false, true, A); \
+	     } else { \
+	         if (bp.pixel_list()) RTB_LAUNCH_SHADE_L(true, false, A); \
+	         else RTB_LAUNCH_SHADE_L(false, false, A); \
+	     } } while (0)
+	if (sv.tri_attr) RTB_LAUNCH_SHADE_PE(true);
+	else RTB_LAUNCH_SHADE_PE(false);
+#undef RTB_LAUNCH_SHADE_PE
 #undef RTB_LAUNCH_SHADE_L
 #undef RTB_LAUNCH_SHADE
 }

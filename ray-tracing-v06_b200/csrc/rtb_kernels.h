@@ -33,6 +33,7 @@ struct SceneView {
 	// bounds, directions on a 2^dir_bits square of the octahedral map; 0 / 0 switches binning off.
 	float bin_min[3], bin_scale[3];   // cell coordinate = (o - bin_min) * bin_scale, clamped to [0, 2^org_bits)
 	int32_t bin_org_bits, bin_dir_bits;
+	int32_t n_tri_attr;         // triangle attribute records (in the padding before `lights`)
 	// Sampled lights (DESIGN.md §5b): n_lights world-space records (4 x float4, SPHERE / QUAD layout), then n_lights
 	// float4 (type bits, quad area, 0, 0).  n_lights = 0: no light sampling (the kernels without it are launched).
 	const float4* lights;
@@ -43,11 +44,17 @@ struct SceneView {
 	int32_t env_width;
 	const float4* env;
 	int32_t env_height, env_sample;
+	// Triangle attributes (DESIGN.md §5e): n_tri_attr records of 4 x float4 (DevTriAttr), and per record slot the index of its
+	// triangle's record or -1.  tri_attr = null: no attributes (the kernels without them are launched).
+	const float4* tri_attr;
+	const int32_t* attr_slot;
 };
-// The map's fields fill the padding after n_lights and add 16 bytes, so every kernel parameter after the SceneView keeps its
-// offset modulo 16 (see BatchParams below for what a moved parameter costs).
-static_assert(alignof(SceneView) == 8 && sizeof(SceneView) == 184 && offsetof(SceneView, n_lights) == 160 &&
-              offsetof(SceneView, env_width) == 164 && offsetof(SceneView, env) == 168, "SceneView layout changed");
+// The map's fields fill the padding after n_lights and add 16 bytes, the attribute count fills the padding before `lights`
+// and its two pointers add 16 more, so every kernel parameter after the SceneView keeps its offset modulo 16 (see BatchParams
+// below for what a moved parameter costs).
+static_assert(alignof(SceneView) == 8 && sizeof(SceneView) == 200 && offsetof(SceneView, n_tri_attr) == 148 &&
+              offsetof(SceneView, lights) == 152 && offsetof(SceneView, n_lights) == 160 && offsetof(SceneView, env_width) == 164 &&
+              offsetof(SceneView, env) == 168 && offsetof(SceneView, tri_attr) == 184, "SceneView layout changed");
 
 // One batch = `samples_per_batch` consecutive samples of every pixel of the row range.
 struct BatchParams {

@@ -133,7 +133,8 @@ int rtb_renderer_set_scene(rtb_renderer* r, rtb_scene* s) {
 		size_t off_pre = align_up(off_blob + fs.blob.size(), 256);
 		size_t off_lights = align_up(off_pre + fs.pre_list.size() * 4, 256);   // (no lights: the arena is what it was without them)
 		size_t off_env = align_up(off_lights + fs.lights.size() * (sizeof(DevPrim) + sizeof(DevLightInfo)), 256);   // (likewise without a map)
-		size_t total = align_up(off_env + fs.env.size() * sizeof(DevEnvTexel) + fs.env_cdf.size() * sizeof(float), 256) + 256;
+		size_t off_attr = align_up(off_env + fs.env.size() * sizeof(DevEnvTexel) + fs.env_cdf.size() * sizeof(float), 256);   // (likewise without attributes)
+		size_t total = align_up(off_attr + fs.tri_attr.size() * sizeof(DevTriAttr) + fs.attr_slot.size() * sizeof(int32_t), 256) + 256;
 		r->staging.assign(total, 0);
 		uint8_t* st = r->staging.data();
 		if (!fs.nodes.empty()) memcpy(st + off_nodes, fs.nodes.data(), fs.nodes.size() * sizeof(DevNode));
@@ -152,7 +153,11 @@ int rtb_renderer_set_scene(rtb_renderer* r, rtb_scene* s) {
 			memcpy(st + off_env, fs.env.data(), fs.env.size() * sizeof(DevEnvTexel));
 			memcpy(st + off_env + fs.env.size() * sizeof(DevEnvTexel), fs.env_cdf.data(), fs.env_cdf.size() * sizeof(float));
 		}
-		r->off[7] = off_lights; r->off[8] = off_env;
+		if (!fs.tri_attr.empty()) {   // the per-slot record indices follow the records directly
+			memcpy(st + off_attr, fs.tri_attr.data(), fs.tri_attr.size() * sizeof(DevTriAttr));
+			memcpy(st + off_attr + fs.tri_attr.size() * sizeof(DevTriAttr), fs.attr_slot.data(), fs.attr_slot.size() * sizeof(int32_t));
+		}
+		r->off[7] = off_lights; r->off[8] = off_env; r->off[9] = off_attr;
 		r->staged_sv = SceneView{};
 		r->staged_sv.root_ref = fs.root_ref;
 		r->staged_sv.n_prims = (int32_t)fs.prims.size();
@@ -163,6 +168,7 @@ int rtb_renderer_set_scene(rtb_renderer* r, rtb_scene* s) {
 		r->staged_sv.bvh_empty = fs.bvh_empty;
 		r->staged_sv.n_lights = (int32_t)fs.lights.size();
 		r->staged_sv.env_width = fs.env_width; r->staged_sv.env_height = fs.env_height; r->staged_sv.env_sample = fs.env_sample;
+		r->staged_sv.n_tri_attr = (int32_t)fs.tri_attr.size();
 		r->staged_sv.has_media = fs.n_media == 0 ? 0 : (fs.n_media <= (int32_t)fs.pre_list.size() ? 1 : 2);
 		r->staged_sv.has_deferred_tex = 0;
 		for (size_t i = 0; i < fs.materials.size(); ++i) {
@@ -194,7 +200,7 @@ int rtb_renderer_share_scene(rtb_renderer* r, const rtb_renderer* src) {
 	const bool same = r->staged_uid == src->staged_uid && r->staged_version == src->staged_version && r->staging.size() == src->staging.size() && r->has_scene;
 	if (!same) {
 		r->staging = src->staging;
-		for (int i = 0; i < 9; ++i) r->off[i] = src->off[i];
+		for (int i = 0; i < 10; ++i) r->off[i] = src->off[i];
 		r->staged_sv = src->staged_sv; r->staged_uid = src->staged_uid; r->staged_version = src->staged_version;
 		for (int k = 0; k < 3; ++k) r->staged_sv.bin_scale[k] *= (float)(1 << r->bin_org_bits) / (float)(1 << src->bin_org_bits);   // (this renderer's own bin settings)
 		r->staged_sv.bin_org_bits = r->bin_org_bits; r->staged_sv.bin_dir_bits = r->bin_dir_bits;
@@ -230,6 +236,8 @@ static int upload_staged_scene(rtb_renderer* r) {
 	r->sv.pre_list = reinterpret_cast<const int32_t*>(base + r->off[6]);
 	r->sv.lights = r->sv.n_lights > 0 ? reinterpret_cast<const float4*>(base + r->off[7]) : nullptr;
 	r->sv.env = r->sv.env_width > 0 ? reinterpret_cast<const float4*>(base + r->off[8]) : nullptr;
+	r->sv.tri_attr = r->sv.n_tri_attr > 0 ? reinterpret_cast<const float4*>(base + r->off[9]) : nullptr;
+	r->sv.attr_slot = r->sv.n_tri_attr > 0 ? reinterpret_cast<const int32_t*>(base + r->off[9] + (size_t)r->sv.n_tri_attr * sizeof(DevTriAttr)) : nullptr;
 	r->has_scene = true;
 	r->scene_upload_bytes = total;
 	return RTB_OK;

@@ -30,7 +30,7 @@ struct rtb_renderer {
 	void* d_scene = nullptr; size_t scene_bytes = 0, scene_upload_bytes = 0;
 	SceneView sv{};
 	std::vector<uint8_t> staging;           // host copy of the arena of the last flattened scene
-	size_t off[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};   // arena sections: nodes, prims, prim info, materials, textures, blob, pre-test list, lights, environment map
+	size_t off[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};   // arena sections: nodes, prims, prim info, materials, textures, blob, pre-test list, lights, environment map, triangle attributes
 	SceneView staged_sv{};
 	uint64_t staged_uid = 0, staged_version = 0;
 	bool has_scene = false;

@@ -239,9 +239,19 @@ int rtb_add_bvh(rtb_scene* s, const int* ch, int n, int builder) {
 	if (n < 1) return fail(RTB_ERR_INVALID, "rtb_add_bvh: needs at least one child");
 	return add_group(s, RTB_OBJ_BVH, ch, n, builder);
 }
-int rtb_add_mesh(rtb_scene* s, const float* vertices, int n_vertices, const int* indices, int n_triangles, int mat) {
+// Corner normal k of a mesh_ex call: normalised in double when non-zero, zero kept.
+static void put_corner_normal(const float* n, float out[3]) {
+	const double x = n[0], y = n[1], z = n[2], len = std::sqrt(x * x + y * y + z * z);
+	for (int c = 0; c < 3; ++c) out[c] = len > 0.0 ? (float)((double)n[c] / len) : 0.0f;
+}
+static int add_mesh(rtb_scene* s, const float* vertices, int n_vertices, const int* indices, int n_triangles,
+                    const float* normals, const float* uvs, int mat) {
 	if (!s || !vertices || !indices || n_vertices < 3 || n_triangles < 1 || !mat_ok(s, mat)) return fail(RTB_ERR_INVALID, "rtb_add_mesh: bad argument");
 	for (int i = 0; i < 3 * n_triangles; ++i) if (indices[i] < 0 || indices[i] >= n_vertices) return fail(RTB_ERR_INVALID, "rtb_add_mesh: vertex index out of range");
+	for (size_t i = 0; normals && i < 3 * (size_t)n_vertices; ++i)
+		if (!std::isfinite(normals[i])) return fail(RTB_ERR_INVALID, "rtb_add_mesh_ex: normal of vertex " + std::to_string(i / 3) + " is not finite");
+	for (size_t i = 0; uvs && i < 2 * (size_t)n_vertices; ++i)
+		if (!std::isfinite(uvs[i])) return fail(RTB_ERR_INVALID, "rtb_add_mesh_ex: UV of vertex " + std::to_string(i / 2) + " is not finite");
 	std::vector<int> ids; ids.reserve(n_triangles);
 	s->objects.reserve(s->objects.size() + (size_t)n_triangles + 1);
 	for (int t = 0; t < n_triangles; ++t) {
@@ -254,9 +264,27 @@ int rtb_add_mesh(rtb_scene* s, const float* vertices, int n_vertices, const int*
 		const float nx = u[1] * v[2] - u[2] * v[1], ny = u[2] * v[0] - u[0] * v[2], nz = u[0] * v[1] - u[1] * v[0];
 		if (!(nx * nx + ny * ny + nz * nz > 0.0f)) continue;
 		ids.push_back(add_planar(s, RTB_OBJ_TRIANGLE, a, u, v, mat));
+		if (normals || uvs) {
+			rtbs_tri_attr at{};
+			for (int k = 0; k < 3; ++k) {
+				const size_t vi = (size_t)indices[3 * t + k];
+				if (normals) put_corner_normal(normals + 3 * vi, at.n[k]);
+				if (uvs) { at.uv[k][0] = uvs[2 * vi]; at.uv[k][1] = uvs[2 * vi + 1]; }
+			}
+			at.flags = (normals ? RTBS_ATTR_NORMALS : 0) | (uvs ? RTBS_ATTR_UVS : 0);
+			s->tri_attrs.push_back(at);
+			s->objects.back().aux = (int32_t)s->tri_attrs.size();
+		}
 	}
 	if (ids.empty()) return fail(RTB_ERR_INVALID, "rtb_add_mesh: no triangle has an area");
 	return add_group(s, RTB_OBJ_BVH, ids.data(), (int)ids.size(), RTB_BVH_TOPDOWN_MEDIAN);
+}
+int rtb_add_mesh(rtb_scene* s, const float* vertices, int n_vertices, const int* indices, int n_triangles, int mat) {
+	return add_mesh(s, vertices, n_vertices, indices, n_triangles, nullptr, nullptr, mat);
+}
+int rtb_add_mesh_ex(rtb_scene* s, const float* vertices, int n_vertices, const int* indices, int n_triangles,
+                    const float* normals, const float* uvs, int mat) {
+	return add_mesh(s, vertices, n_vertices, indices, n_triangles, normals, uvs, mat);
 }
 int rtb_add_translate(rtb_scene* s, int child, const float off[3]) {
 	if (!s || !off || !obj_ok(s, child)) return fail(RTB_ERR_INVALID, "rtb_add_translate: bad argument");
@@ -372,18 +400,24 @@ extern "C" int rtb_object_bounds(const rtb_scene* s, int object, float out6[6]) 
 
 // ============================================================== serialisation
 
+static_assert(sizeof(rtbs_tri_attr) == 64, "rtbs_tri_attr is a 64-byte record");
+
 extern "C" size_t rtb_scene_serialize(const rtb_scene* s, void* buf, size_t cap) {
 	if (!s) return 0;
 	// A scene without sampled lights or a map is written as RTBS v1, byte for byte; one with lights only as v2 (the list
 	// appended); one with a map as v3 (the list, possibly empty, then the map).
-	const bool env = s->env_width > 0;
+	// One with triangle attributes as v4: the v3 content (an empty map record when there is no map), then the attributes.
+	const bool attr = !s->tri_attrs.empty();
+	const bool env = s->env_width > 0 || attr;
 	const bool lights = !s->sampled_lights.empty() || env;
-	const size_t env_floats = env ? (size_t)s->env_width * s->env_height * 3 : 0;
+	const size_t env_floats = (size_t)s->env_width * s->env_height * 3;
 	size_t need = sizeof(rtbs_header) + s->textures.size() * sizeof(rtbs_texture) + s->materials.size() * sizeof(rtbs_material) +
 	              s->objects.size() * sizeof(rtbs_object) + s->children.size() * 4 + s->blob.size() +
-	              (lights ? 4 + s->sampled_lights.size() * 4 : 0) + (env ? sizeof(rtbs_env) + env_floats * 4 : 0);
+	              (lights ? 4 + s->sampled_lights.size() * 4 : 0) + (env ? sizeof(rtbs_env) + env_floats * 4 : 0) +
+	              (attr ? 4 + s->tri_attrs.size() * sizeof(rtbs_tri_attr) : 0);
 	if (!buf || cap < need) return need;
-	rtbs_header h{}; h.magic = RTBS_MAGIC; h.version = env ? RTBS_VERSION_ENV : lights ? RTBS_VERSION_LIGHTS : RTBS_VERSION;
+	rtbs_header h{}; h.magic = RTBS_MAGIC;
+	h.version = attr ? RTBS_VERSION_ATTR : env ? RTBS_VERSION_ENV : lights ? RTBS_VERSION_LIGHTS : RTBS_VERSION;
 	h.n_textures = (uint32_t)s->textures.size(); h.n_materials = (uint32_t)s->materials.size();
 	h.n_objects = (uint32_t)s->objects.size(); h.n_children = (uint32_t)s->children.size();
 	h.n_blob_bytes = (uint32_t)s->blob.size(); h.root_object = s->root; h.background_mode = s->background_mode;
@@ -407,6 +441,11 @@ extern "C" size_t rtb_scene_serialize(const rtb_scene* s, void* buf, size_t cap)
 		memcpy(e.scale, s->env_scale, 12);
 		put(&e, sizeof e);
 		put(s->env_rgb.data(), env_floats * 4);
+	}
+	if (attr) {
+		const uint32_t n = (uint32_t)s->tri_attrs.size();
+		put(&n, 4);
+		put(s->tri_attrs.data(), s->tri_attrs.size() * sizeof(rtbs_tri_attr));
 	}
 	return need;
 }
@@ -690,7 +729,7 @@ struct Flattener {
 	FlatScene& out;
 	// One item per logical primitive (= one BVH leaf); an item owns one or two 64-byte record slots.
 	// Records live in one pool; rec_type tags the first slot of everything a hit can name (-1 = continuation slot).
-	struct Item { int first; int nrec; int type; DevPrimInfo info; };
+	struct Item { int first; int nrec; int type; DevPrimInfo info; int attr = -1; };   // attr: index of the triangle's attributes
 	std::vector<Item> items;
 	std::vector<Box3> prim_boxes;
 	std::vector<DevPrim> recs;
@@ -867,7 +906,13 @@ struct Flattener {
 		case RTB_OBJ_SPHERE: emit_sphere(o, id, x); return RTB_OK;
 		case RTB_OBJ_MOVING_SPHERE: emit_moving_sphere(o, id, x); return RTB_OK;
 		case RTB_OBJ_QUAD: emit_planar(PRIM_QUAD, o.f, o.f + 3, o.f + 6, o.mat, id, x); return RTB_OK;
-		case RTB_OBJ_TRIANGLE: emit_planar(PRIM_TRIANGLE, o.f, o.f + 3, o.f + 6, o.mat, id, x); return RTB_OK;
+		case RTB_OBJ_TRIANGLE:
+			emit_planar(PRIM_TRIANGLE, o.f, o.f + 3, o.f + 6, o.mat, id, x);
+			if (o.aux > 0) {
+				if ((size_t)o.aux > s.tri_attrs.size()) return fail(RTB_ERR_INVALID, "triangle " + std::to_string(id) + ": bad attribute index");
+				items.back().attr = o.aux - 1;
+			}
+			return RTB_OK;
 		case RTB_OBJ_BOX: emit_box(o, id, x); return RTB_OK;
 		case RTB_OBJ_LIST: case RTB_OBJ_BVH: {
 			for (int k = 0; k < o.child_count; ++k) { int rc = walk(s.children[o.child_begin + k], x, depth + 1); if (rc) return rc; }
@@ -1023,6 +1068,19 @@ int flatten(rtb_scene& s, FlatScene& out, const GpuBuildContext* gpu) {
 		}
 	});
 	if (out.prims.size() >= (1u << (31 - RTB_LEAF_TYPE_BITS))) return fail(RTB_ERR_UNSUPPORTED, "too many primitive record slots for a leaf reference (2^27)");
+	// Triangle attributes (DESIGN.md §5e): the records, and per slot the index of its record (-1: none).  The primitive
+	// records and the tree stay those of the same scene without attributes.
+	if (!s.tri_attrs.empty()) {
+		out.attr_slot.assign(out.prims.size(), -1);
+		for (size_t i = 0; i < order.size(); ++i) out.attr_slot[slot_of[i]] = fl.items[order[i]].attr;
+		out.tri_attr.resize(s.tri_attrs.size());
+		for (size_t k = 0; k < s.tri_attrs.size(); ++k) {
+			const rtbs_tri_attr& a = s.tri_attrs[k]; float* q = out.tri_attr[k].q;
+			for (int c = 0; c < 3; ++c) { q[4 * c] = a.n[c][0]; q[4 * c + 1] = a.n[c][1]; q[4 * c + 2] = a.n[c][2]; }
+			q[3] = a.uv[0][0]; q[7] = a.uv[0][1]; q[11] = a.uv[1][0];
+			q[12] = a.uv[1][1]; q[13] = a.uv[2][0]; q[14] = a.uv[2][1]; q[15] = rt::u2f((uint32_t)a.flags);
+		}
+	}
 	lap("layout");
 
 	// Wide layout: one 64-byte record per inner node carrying both children's boxes, numbered in
@@ -1158,6 +1216,10 @@ extern "C" int rtb_scene_flatten_hash(rtb_scene* s, uint64_t* hash_out) {
 		mix(dims, sizeof dims);
 		mix(fs.env.data(), fs.env.size() * sizeof(rtb::DevEnvTexel));
 		mix(fs.env_cdf.data(), fs.env_cdf.size() * sizeof(float));
+	}
+	if (!fs.tri_attr.empty()) { // (likewise for triangle attributes)
+		mix(fs.tri_attr.data(), fs.tri_attr.size() * sizeof(rtb::DevTriAttr));
+		mix(fs.attr_slot.data(), fs.attr_slot.size() * sizeof(int32_t));
 	}
 	*hash_out = h;
 	return RTB_OK;

@@ -27,6 +27,9 @@ struct rtb_scene {
 	std::vector<float> env_rgb;
 	int32_t env_width = 0, env_height = 0, env_flags = 0;
 	float env_scale[3] = {1, 1, 1};
+	// rtb_add_mesh_ex: corner attributes of mesh triangles; triangle object k carries tri_attrs[objects[k].aux - 1] when its
+	// aux is non-zero (empty: no attributes, the scene serialises as v1 - v3).
+	std::vector<rtbs_tri_attr> tri_attrs;
 
 	// Filled by flatten(): the world BVH in the reference's node layout (parity hook).
 	std::vector<rtb_bvh_node> world_nodes;

@@ -61,6 +61,10 @@ struct alignas(16) DevLightInfo { int32_t type; float area; float pad0, pad1; };
 // p_ij * W * H / (2 pi^2) (the pdf of a direction is this over sin theta).
 struct alignas(16) DevEnvTexel { float r, g, b, pdf; };
 
+// Corner attributes of a mesh triangle (DESIGN.md §5e), in the triangle's own frame, as four float4:
+//   (n0.xyz, uv0.x)  (n1.xyz, uv0.y)  (n2.xyz, uv1.x)  (uv1.y, uv2.x, uv2.y, flags bits = RTBS_ATTR_NORMALS | RTBS_ATTR_UVS)
+struct alignas(64) DevTriAttr { float q[16]; };
+
 struct alignas(16) DevMaterial { int32_t kind, tex; float param, pad; float albedo[4]; };  // 32 B
 
 struct alignas(16) DevTexture {                                                             // 48 B
@@ -86,6 +90,8 @@ struct FlatScene {
 	std::vector<DevEnvTexel> env;        // environment map texels, row 0 = top (empty: no map)
 	std::vector<float> env_cdf;          // its marginal CDF (env_height + 1), then env_height conditional CDFs (env_width + 1 each)
 	int32_t env_width = 0, env_height = 0, env_sample = 0;
+	std::vector<DevTriAttr> tri_attr;    // triangle attribute records (empty: no attributes)
+	std::vector<int32_t> attr_slot;      // per record slot: its tri_attr index, or -1 (empty when tri_attr is)
 	int32_t n_media = 0;
 	int32_t background_mode = 0;
 	float background[3] = {0, 0, 0};

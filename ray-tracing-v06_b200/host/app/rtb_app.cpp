@@ -5,7 +5,8 @@
 //   rtb_app [scene] [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--gpus N]
 //           [--out image.png|image.ppm|image.pfm] [--resume ckpt.rtba] [--checkpoint ckpt.rtba] [--sample-lights]
 //           [--target-db D [--min-spp N]] [--env map.pfm [--env-scale S] [--sample-env]]
-//   rtb_app --obj model.obj [...]     a Wavefront OBJ mesh (MeshHandle) on a checkered floor under the sky
+//   rtb_app --obj model.obj [--smooth [--obj-texture image.ppm]] [...]
+//                                     a Wavefront OBJ mesh (MeshHandle) on a checkered floor under the sky
 //
 // scene = one of rtb_scenes_name(i) (default book2_bouncing, which goes through SceneBook2BVH::Factory
 // and Renderer::MakeRenderer exactly like FirstApp::MakeApp).  --gpus N renders on N GPUs of the box (sample range split,
@@ -22,6 +23,9 @@
 // --env map.pfm lights the scene (any named scene or --obj) with an HDR environment map (rtb_scene_set_environment,
 // DESIGN.md §5d): an equirectangular PFM, +y up, which every ray that leaves the scene reads instead of the background;
 // --env-scale S multiplies its texels by S, and --sample-env importance-samples it (same converged image, less noise).
+// --smooth loads the --obj model with MeshHandle::LoadObjShaded: smooth shading from its `vn` normals (computed from the faces
+// when it has none) and its `vt` texture coordinates (DESIGN.md §5e).  --obj-texture image.ppm (binary P6) then maps that
+// image onto the model through its texture coordinates; it needs --smooth and a model with `vt` on every corner.
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -54,7 +58,8 @@ int main(int argc, char** argv) {
 	bool sample_lights = false;
 	double target_db = -1.0;
 	int min_spp = 64;
-	std::string env_path;
+	std::string env_path, obj_texture;
+	bool smooth = false;
 	float env_scale = 1.0f;
 	bool sample_env = false;
 	uint32_t seed = 1984;   // the reference's seed (Renderer.cu:51, Scenes.cu:190)
@@ -77,6 +82,8 @@ int main(int argc, char** argv) {
 		else if (a == "--env" && i + 1 < argc) env_path = argv[++i];
 		else if (a == "--env-scale" && i + 1 < argc) env_scale = (float)atof(argv[++i]);
 		else if (a == "--sample-env") sample_env = true;
+		else if (a == "--smooth") smooth = true;
+		else if (a == "--obj-texture" && i + 1 < argc) obj_texture = argv[++i];
 		else if (a == "--list") { for (int k = 0; k < rtb_scenes_count(); ++k) printf("%s\n", rtb_scenes_name(k)); return 0; }
 		else scene_name = a;
 	}
@@ -84,6 +91,8 @@ int main(int argc, char** argv) {
 		fprintf(stderr, "rtb_app: --sample-lights: %s lists no lights to sample\n", obj_path.empty() ? scene_name.c_str() : obj_path.c_str());
 		return 1;
 	}
+	if ((smooth || !obj_texture.empty()) && obj_path.empty()) { fprintf(stderr, "rtb_app: --smooth and --obj-texture apply to an --obj model\n"); return 1; }
+	if (!obj_texture.empty() && !smooth) { fprintf(stderr, "rtb_app: --obj-texture needs --smooth (the texture coordinates come with LoadObjShaded)\n"); return 1; }
 	if (sample_env && env_path.empty()) { fprintf(stderr, "rtb_app: --sample-env needs --env map.pfm\n"); return 1; }
 	std::vector<float> env_rgb;
 	int env_w = 0, env_h = 0;
@@ -108,10 +117,19 @@ int main(int argc, char** argv) {
 			// A mesh scene assembled the way FirstApp assembles its world: materials, handles, a HittableList, MakeRenderer.
 			uint32_t _width = width ? width : 800, _height = height ? height : 600;
 			printf("Loading %s... ", obj_path.c_str());
-			Mesh mesh = MeshHandle::LoadObj(obj_path);
+			Mesh mesh = smooth ? MeshHandle::LoadObjShaded(obj_path) : MeshHandle::LoadObj(obj_path);
 			Lambertian clay(glm::vec3(0.73f, 0.73f, 0.73f));
-			MeshHandle model = MeshHandle::MakeMesh(mesh, &clay);
-			printf("%d triangles.\n", model.triangleCount());
+			std::unique_ptr<image_texture> skin;
+			std::unique_ptr<Lambertian> skin_mat;
+			if (!obj_texture.empty()) {
+				if (mesh.uvs.empty()) { fprintf(stderr, "\nrtb_app: --obj-texture: %s has no texture coordinates (`vt` on every face corner)\n", obj_path.c_str()); return 1; }
+				std::vector<uint8_t> px; int tw = 0, th = 0; std::string err;
+				if (!rtb_host::read_ppm(obj_texture, px, tw, th, err)) { fprintf(stderr, "\nrtb_app: --obj-texture: %s\n", err.c_str()); return 1; }
+				skin = std::make_unique<image_texture>(px.data(), tw, th, 3);
+				skin_mat = std::make_unique<Lambertian>(skin.get());
+			}
+			MeshHandle model = skin_mat ? MeshHandle::MakeMesh(mesh, skin_mat.get()) : MeshHandle::MakeMesh(mesh, &clay);
+			printf("%d triangles%s.\n", model.triangleCount(), smooth ? (skin ? ", smooth, textured" : ", smooth") : "");
 			const glm::vec3 lo = model.getBounds().getMin(), hi = model.getBounds().getMax(), mid = (lo + hi) * 0.5f;
 			const float size = glm::length(hi - lo);
 			solid_texture dark(glm::vec3(.2f, .3f, .1f)), light(glm::vec3(.9f, .9f, .9f));

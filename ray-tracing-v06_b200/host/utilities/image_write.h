@@ -112,6 +112,35 @@ inline bool read_pfm(const std::string& path, std::vector<float>& rgb, int& widt
 	return true;
 }
 
+// Binary PPM (P6, maxval 255) -> width x height x RGB8, row 0 = the top row of the picture (the row order image textures use).
+inline bool read_ppm(const std::string& path, std::vector<uint8_t>& rgb, int& width, int& height, std::string& err) {
+	FILE* f = fopen(path.c_str(), "rb");
+	if (!f) { err = "cannot open " + path; return false; }
+	auto field = [f](int& v) {   // the next decimal field of the header, skipping whitespace and # comments
+		int c = fgetc(f);
+		for (;;) {
+			while (c == ' ' || c == '\t' || c == '\r' || c == '\n') c = fgetc(f);
+			if (c != '#') break;
+			while (c != '\n' && c != EOF) c = fgetc(f);
+		}
+		if (c < '0' || c > '9') return false;
+		v = 0;
+		for (; c >= '0' && c <= '9'; c = fgetc(f)) { v = v * 10 + (c - '0'); if (v > (1 << 20)) return false; }
+		return c == ' ' || c == '\t' || c == '\r' || c == '\n';   // (one whitespace byte ends the header)
+	};
+	int maxval = 0;
+	width = height = 0;
+	const bool ok = fgetc(f) == 'P' && fgetc(f) == '6' && field(width) && field(height) && field(maxval);
+	if (!ok || width <= 0 || height <= 0 || maxval != 255 || (int64_t)width * height > (int64_t(1) << 26)) {
+		fclose(f); err = path + " is not a binary PPM (P6) image with 8-bit samples"; return false;
+	}
+	rgb.resize((size_t)width * height * 3);
+	const size_t got = fread(rgb.data(), 1, rgb.size(), f);
+	fclose(f);
+	if (got != rgb.size()) { err = path + ": truncated PPM data"; return false; }
+	return true;
+}
+
 inline bool has_suffix(const std::string& s, const char* suf) { const std::string t(suf); return s.size() >= t.size() && s.compare(s.size() - t.size(), t.size(), t) == 0; }
 
 }  // namespace rtb_host
