@@ -57,7 +57,8 @@ typedef struct rtb_scene rtb_scene;
 enum rtb_texture_kind { RTB_TEX_SOLID = 0, RTB_TEX_CHECKER = 1, RTB_TEX_IMAGE = 2, RTB_TEX_NOISE = 3 };
 enum rtb_material_kind {
 	RTB_MAT_LAMBERTIAN = 0, RTB_MAT_METAL = 1, RTB_MAT_DIELECTRIC = 2,
-	RTB_MAT_DIFFUSE_LIGHT = 3, RTB_MAT_ISOTROPIC = 4
+	RTB_MAT_DIFFUSE_LIGHT = 3, RTB_MAT_ISOTROPIC = 4,
+	RTB_MAT_ROUGH_METAL = 5, RTB_MAT_ROUGH_DIELECTRIC = 6
 };
 enum rtb_object_kind {
 	RTB_OBJ_SPHERE = 0, RTB_OBJ_MOVING_SPHERE = 1, RTB_OBJ_QUAD = 2, RTB_OBJ_TRIANGLE = 3,
@@ -90,6 +91,16 @@ int rtb_add_metal(rtb_scene* s, const float albedo[3], float fuzz);
 int rtb_add_dielectric(rtb_scene* s, const float albedo[3], float ior);
 int rtb_add_diffuse_light(rtb_scene* s, int tex);
 int rtb_add_isotropic(rtb_scene* s, int tex);
+/* GGX (Trowbridge-Reitz) microfacet materials with isotropic width `alpha` in [RTB_ROUGH_ALPHA_MIN, 1] (DESIGN.md §5f).
+ * Directions are drawn from the distribution of visible normals; the throughput weight of a sampled direction is
+ * G2 / G1 (height-correlated Smith) times Schlick's Fresnel term (metal, F0 per channel) or the albedo (dielectric).
+ * Single scattering only: the energy that multiple scattering between microfacets would return is lost, more of it
+ * the larger alpha.  Neither kind is part of the light mixture of rtb_scene_set_sampled_lights.  As alpha -> 0 the
+ * metal tends to rtb_add_metal(f0, 0) and the dielectric to rtb_add_dielectric (no 1/ior^2 radiance factor either).
+ * RTB_ERR_INVALID (scene unchanged): a null pointer, a non-finite value, alpha outside the range, ior not > 0. */
+#define RTB_ROUGH_ALPHA_MIN 0.001f
+int rtb_add_rough_metal(rtb_scene* s, const float f0[3], float alpha);
+int rtb_add_rough_dielectric(rtb_scene* s, const float albedo[3], float ior, float alpha);
 
 /* Hittables: return an object id >= 0, or a negative rtb_status. */
 int rtb_add_sphere(rtb_scene* s, const float center[3], float radius, int mat);

@@ -19,9 +19,11 @@
  *                                            multiplied by env.scale)
  *   uint32        n_tri_attrs              (version 4 only: per-vertex attributes of mesh triangles, rtb_add_mesh_ex)
  *   rtbs_tri_attr tri_attrs[n_tri_attrs]    (a TRIANGLE object whose `aux` is k + 1 carries tri_attrs[k]; aux = 0: none)
+ *   uint32        n_materials              (version 5 only: the GGX width of every material, rtb_add_rough_metal /
+ *   float         alpha[n_materials]        rtb_add_rough_dielectric; 0 for the other kinds)
  *
  * A scene without attributes is written as version 1 (no sampled lights), 2 or 3 (a map); one with attributes as
- * version 4.
+ * version 4; one with a rough material as version 5 (the version 4 content, then the widths).
  */
 #ifndef RTB_SCENE_FORMAT_H
 #define RTB_SCENE_FORMAT_H
@@ -33,6 +35,7 @@
 #define RTBS_VERSION_LIGHTS 2u
 #define RTBS_VERSION_ENV 3u
 #define RTBS_VERSION_ATTR 4u
+#define RTBS_VERSION_ROUGH 5u
 
 /* Corner attributes of one triangle (DESIGN.md §5e), in the order of its corners v0 (= Q), v1 (= Q + u), v2 (= Q + v).
  * Normals are unit length or zero (normalised on the host); flags say which of the two are present. */
@@ -78,7 +81,7 @@ typedef struct rtbs_material {
 	int32_t kind;           /* rtb_material_kind */
 	int32_t tex;            /* albedo / emission / phase texture id, -1 = use `albedo` */
 	float   albedo[3];
-	float   param;          /* metal: fuzz; dielectric: ior */
+	float   param;          /* metal: fuzz; dielectric, rough dielectric: ior */
 } rtbs_material;            /* 24 B */
 
 /* f[] per kind:

@@ -128,6 +128,8 @@ ABI = {
     "rtb_add_dielectric": (C.c_int, [_P, _F3, C.c_float]),
     "rtb_add_diffuse_light": (C.c_int, [_P, C.c_int]),
     "rtb_add_isotropic": (C.c_int, [_P, C.c_int]),
+    "rtb_add_rough_metal": (C.c_int, [_P, _F3, C.c_float]),
+    "rtb_add_rough_dielectric": (C.c_int, [_P, _F3, C.c_float, C.c_float]),
     "rtb_add_sphere": (C.c_int, [_P, _F3, C.c_float, C.c_int]),
     "rtb_add_moving_sphere": (C.c_int, [_P, _F3, _F3, C.c_float, C.c_int]),
     "rtb_add_quad": (C.c_int, [_P, _F3, _F3, _F3, C.c_int]),
@@ -333,6 +335,12 @@ class Scene:
     def dielectric(self, ior, albedo=(1, 1, 1)): return _check(lib().rtb_add_dielectric(self.handle, _f3(albedo), ior), "rtb_add_dielectric")
     def diffuse_light(self, tex): return _check(lib().rtb_add_diffuse_light(self.handle, tex), "rtb_add_diffuse_light")
     def isotropic(self, tex): return _check(lib().rtb_add_isotropic(self.handle, tex), "rtb_add_isotropic")
+    def rough_metal(self, f0, alpha):
+        """GGX conductor: Schlick Fresnel from the per-channel reflectance f0, width alpha in [0.001, 1] (DESIGN.md §5f)."""
+        return _check(lib().rtb_add_rough_metal(self.handle, _f3(f0), alpha), "rtb_add_rough_metal")
+    def rough_dielectric(self, ior, alpha, albedo=(1, 1, 1)):
+        """GGX glass: the dielectric's Schlick reflect / refract choice about a visible normal of width alpha in [0.001, 1]."""
+        return _check(lib().rtb_add_rough_dielectric(self.handle, _f3(albedo), ior, alpha), "rtb_add_rough_dielectric")
     def sphere(self, c, r, mat): return _check(lib().rtb_add_sphere(self.handle, _f3(c), r, mat), "rtb_add_sphere")
     def moving_sphere(self, c0, c1, r, mat): return _check(lib().rtb_add_moving_sphere(self.handle, _f3(c0), _f3(c1), r, mat), "rtb_add_moving_sphere")
     def quad(self, Q, u, v, mat): return _check(lib().rtb_add_quad(self.handle, _f3(Q), _f3(u), _f3(v), mat), "rtb_add_quad")

@@ -953,13 +953,82 @@ __device__ __forceinline__ bool light_mix(const SceneView& sv, const Surface& s,
 	return w > 0.0f;
 }
 
+// ------------------------------------------------------------------------------------------------
+// GGX microfacet materials (DESIGN.md §5f): visible-normal sampling (Dupuy & Benyoub 2023, spherical caps), weight G2 / G1
+// of the height-correlated Smith term; no pdf is evaluated and the light mixture is not involved.
+
+// Smith Lambda of a local direction for the GGX width a2 = alpha^2
+__device__ __forceinline__ float ggx_lambda(v3 w, float a2) {
+	const float t = fmaf(w.y, w.y, w.x * w.x) / (w.z * w.z);
+	return (sqrtf(fmaf(a2, t, 1.0f)) - 1.0f) * 0.5f;
+}
+
+// Rough metal (DIEL = false: F0 = albedo, frame normal n_shade) or rough dielectric (DIEL: the dielectric's normal, which
+// the caller passes as n with its ior ratio).  0 = the path ends black, 1 = scattered.
+template <bool DIEL>
+__device__ __forceinline__ int rough_scatter(v3 n, v3 d, const rt::f4& r, float alpha, float ratio, v3 albedo, v3& dir, v3& att) {
+	// frame (U, V, W = n) as rt::cone_direction builds it; wo local
+	const v3 ud = rt::normalize(d);
+	const v3 wo_w = rt::neg(ud);
+	const v3 A = fabsf(n.x) > 0.9f ? rt::mk(0.0f, 1.0f, 0.0f) : rt::mk(1.0f, 0.0f, 0.0f);
+	const v3 V = rt::normalize(rt::cross(n, A));
+	const v3 U = rt::cross(n, V);
+	const v3 wo = rt::mk(rt::dot(wo_w, U), rt::dot(wo_w, V), rt::dot(wo_w, n));
+	if (!(wo.z > 0.0f)) return 0;
+	// visible normal: spherical cap around the stretched wo
+	const v3 wh = rt::normalize(rt::mk(alpha * wo.x, alpha * wo.y, wo.z));
+	float sn, cs; rt::sincos2pi(r.x, sn, cs);
+	const float z = fmaf(1.0f - r.y, 1.0f + wh.z, -wh.z);
+	const float st = sqrtf(fmaxf(0.0f, fmaf(-z, z, 1.0f)));
+	const v3 h = rt::mk(st * cs + wh.x, st * sn + wh.y, z + wh.z);
+	if (!(rt::dot(h, h) > 0.0f)) return 0;
+	const v3 wm = rt::normalize(rt::mk(alpha * h.x, alpha * h.y, h.z));
+	const float cos_om = rt::dot(wo, wm);
+	if (!(cos_om > 0.0f)) return 0;
+	v3 wi;
+	if (!DIEL) {
+		wi = rt::reflect(rt::neg(wo), wm);
+		if (!(wi.z > 0.0f)) return 0;
+	} else {                                     // the dielectric of scatter() about wm
+		const v3 ui = rt::neg(wo);
+		const float cos_theta = fminf(cos_om, 1.0f);
+		const float sin_theta = sqrtf(fmaf(-cos_theta, cos_theta, 1.0f));
+		float r0 = (1.0f - ratio) / (1.0f + ratio); r0 = r0 * r0;
+		const float x = 1.0f - cos_theta, x2 = x * x;
+		const float prob = fmaf(1.0f - r0, x2 * x2 * x, r0);
+		if (ratio * sin_theta > 1.0f || prob > r.z) {
+			wi = rt::reflect(ui, wm);
+			if (!(wi.z > 0.0f)) return 0;
+		} else {
+			const float dv = rt::dot(wm, ui);
+			const float k = fmaf(-(ratio * ratio), fmaf(-dv, dv, 1.0f), 1.0f);
+			if (k < 0.0f) return 0;
+			const float coef = fmaf(ratio, dv, sqrtf(k));
+			wi = rt::mk(fmaf(-coef, wm.x, ratio * ui.x), fmaf(-coef, wm.y, ratio * ui.y), fmaf(-coef, wm.z, ratio * ui.z));
+			if (!(wi.z < 0.0f)) return 0;
+		}
+	}
+	const float a2 = alpha * alpha;
+	const float lo = 1.0f + ggx_lambda(wo, a2);
+	const float g = lo / (lo + ggx_lambda(wi, a2));
+	if (!DIEL) {
+		const float x = 1.0f - cos_om, x2 = x * x, x5 = x2 * x2 * x;
+		att = rt::mk(fmaf(1.0f - albedo.x, x5, albedo.x) * g, fmaf(1.0f - albedo.y, x5, albedo.y) * g, fmaf(1.0f - albedo.z, x5, albedo.z) * g);
+	} else {
+		att = rt::mul(albedo, g);
+	}
+	dir = rt::mk(fmaf(wi.z, n.x, fmaf(wi.y, V.x, wi.x * U.x)), fmaf(wi.z, n.y, fmaf(wi.y, V.y, wi.x * U.y)), fmaf(wi.z, n.z, fmaf(wi.y, V.z, wi.x * U.z)));
+	return 1;
+}
+
 // Material::Scatter for every material kind.  Returns 0 = absorbed (path ends black),
 // 1 = scattered (dir/attenuation valid), 2 = emitted (attenuation holds the emitted radiance).
 // With DEFER, an image / noise albedo of a scattering material is not evaluated here: attenuation is
 // left at 1 and defer_tex names the texture, to be multiplied in later by texture_kernel (dense warps).
 // With LIGHTS, Lambertian and isotropic scatters draw from the light mixture and set w (1 otherwise); ENV: with the map.
 // ATTR: the dielectric refracts about s.n_diel (its inside / outside test stays with the geometric normal).
-template <bool DEFER, bool LIGHTS, bool ENV, bool ATTR>
+// ROUGH: the scene has GGX materials (their width is the material's fourth word); never part of the light mixture.
+template <bool DEFER, bool LIGHTS, bool ENV, bool ATTR, bool ROUGH>
 __device__ __forceinline__ int scatter(const SceneView& sv, int mat, const Surface& s, v3 d, const rt::f4& r, const LightKey& lk,
                                        v3& dir, v3& att, float& w, int& defer_tex) {
 	RTB_CHECK(mat >= 0 && mat < sv.n_materials, RTB_BOUNDS_MATERIAL);
@@ -973,6 +1042,14 @@ __device__ __forceinline__ int scatter(const SceneView& sv, int mat, const Surfa
 		const int tkind = __float_as_int(ldg4(sv.textures + 3 * tex).x);
 		if (DEFER && kind != RTB_MAT_DIFFUSE_LIGHT && (tkind == RTB_TEX_NOISE || tkind == RTB_TEX_IMAGE)) { defer_tex = tex; albedo = rt::mk(1.0f, 1.0f, 1.0f); }
 		else albedo = texture_value(sv, tex, s.u, s.v, s.p);
+	}
+	if (ROUGH && kind == RTB_MAT_ROUGH_METAL) return rough_scatter<false>(s.n_shade, d, r, m0.w, 0.0f, albedo, dir, att);
+	if (ROUGH && kind == RTB_MAT_ROUGH_DIELECTRIC) {   // the dielectric's normal and ratio (below)
+		v3 n = s.n_geom;
+		const bool back = rt::dot(d, n) > 0.0f;
+		if (ATTR) n = s.n_diel;
+		if (back) n = rt::neg(n);
+		return rough_scatter<true>(n, d, r, m0.w, back ? param : 1.0f / param, albedo, dir, att);
 	}
 	switch (kind) {
 	case RTB_MAT_LAMBERTIAN: {   // LambertianAbstract / LambertianTexture  cu_materials.cuh:26-40,52-64
@@ -1037,7 +1114,8 @@ __device__ __forceinline__ v3 background(const SceneView& sv, v3 d) {
 struct DeferredTex { int tex; float u, v; v3 p; };
 
 // ENV: a miss returns the environment map's texel instead of the background.  ATTR: the scene has triangle attributes.
-template <bool DEFER, bool LIGHTS, bool LIST, bool ENV, bool ATTR>
+// ROUGH: the scene has GGX materials.
+template <bool DEFER, bool LIGHTS, bool LIST, bool ENV, bool ATTR, bool ROUGH>
 __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t batch, uint32_t bounce,
                                               const float4& fo, const float4& fd, v3 thr, float t, int code,
                                               float4& no, float4& nd, v3& nthr, DeferredTex& dt) {
@@ -1061,7 +1139,7 @@ __device__ __forceinline__ bool shade_segment(const SceneView& sv, const BatchPa
 	const rt::f4 r = rt::rng4(bp.seed, pixel, sample, bounce, rt::STREAM_SCATTER);
 	v3 dir, att;
 	float w = 1.0f;
-	const int res = scatter<DEFER, LIGHTS, ENV, ATTR>(sv, info.x, s, d, r, LightKey{bp.seed, pixel, sample, bounce}, dir, att, w, dt.tex);
+	const int res = scatter<DEFER, LIGHTS, ENV, ATTR, ROUGH>(sv, info.x, s, d, r, LightKey{bp.seed, pixel, sample, bounce}, dir, att, w, dt.tex);
 	dt.u = s.u; dt.v = s.v; dt.p = s.p;
 	if (res == 2) {                                       // emitter: throughput * emitted, path ends
 		v3 c = rt::mulv(thr, att);
@@ -1144,7 +1222,7 @@ __device__ __forceinline__ void bin_table_flush(uint32_t* s_key, uint32_t* s_cnt
 #ifndef SHADE_MIN_BLOCKS
 #define SHADE_MIN_BLOCKS 8   // 8 x 128 threads x 64 registers = the whole register file (6 / 9 / 10 blocks: 11.7 / 10.9 / 12.4 ms)
 #endif
-template <bool LIGHTS, bool LIST, bool ENV, bool ATTR>
+template <bool LIGHTS, bool LIST, bool ENV, bool ATTR, bool ROUGH>
 __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS)
 shade_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int q) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -1175,7 +1253,7 @@ shade_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce, int 
 			float4 fo, fd; ld_ray(rod + 2 * (size_t)i, fo, fd);
 			const float4 ft = ldq(rt_ + i);
 			const int2 h = ldq(wv.hit + i);
-			alive = shade_segment<true, LIGHTS, LIST, ENV, ATTR>(sv, bp, wv, batch, bounce, fo, fd, xyz(ft), __int_as_float(h.x), h.y, no, nd, nthr, dt);
+			alive = shade_segment<true, LIGHTS, LIST, ENV, ATTR, ROUGH>(sv, bp, wv, batch, bounce, fo, fd, xyz(ft), __int_as_float(h.x), h.y, no, nd, nthr, dt);
 		}
 		// live-path compaction: warp ballot/popc, one global atomic per block
 		const uint32_t mask = __ballot_sync(FULL_MASK, alive);
@@ -1377,7 +1455,7 @@ bin_permute_kernel(SceneView sv, WaveView wv, uint32_t bounce, int q_from) {
 // One persistent launch then runs every remaining path to completion (traverse + shade fused, one
 // thread per path); later traverse/shade launches of the batch see tail_from and return at once.
 
-template <bool MEDIA, int STACK, bool LIGHTS, bool LIST, bool ENV, bool ATTR>
+template <bool MEDIA, int STACK, bool LIGHTS, bool LIST, bool ENV, bool ATTR, bool ROUGH>
 __global__ void __launch_bounds__(TRAVERSE_THREADS)
 tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int q, uint32_t threshold) {
 	const BatchParams bp = with_call_params(bp_in, wv);
@@ -1403,7 +1481,7 @@ tail_kernel(SceneView sv, BatchParams bp_in, WaveView wv, uint32_t bounce0, int 
 			trace_ray<(MEDIA ? 2 : 0)>(sv, xyz(fo), xyz(fd), fo.w, mr, s_stack + threadIdx.x, STACK, t, code);
 			float4 no, nd; v3 nthr;
 			DeferredTex dt;
-			if (!shade_segment<false, LIGHTS, LIST, ENV, ATTR>(sv, bp, wv, batch, b, fo, fd, thr, t, code, no, nd, nthr, dt)) break;
+			if (!shade_segment<false, LIGHTS, LIST, ENV, ATTR, ROUGH>(sv, bp, wv, batch, b, fo, fd, thr, t, code, no, nd, nthr, dt)) break;
 			fo = no; fd = nd; thr = nthr;
 		}
 	}
@@ -1673,12 +1751,12 @@ void query_occupancy(int device, LaunchCfg& lc) {
 	int occ_t = 0, occ_tm = 0, occ_s = 0, occ_g = 0;
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_t, traverse_kernel<0, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_tm, traverse_kernel<2, STACK_SIZE, false>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, shade_kernel<false, false, false, false>, SHADE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, shade_kernel<false, false, false, false, false>, SHADE_THREADS, 0);
 	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_g, generate_kernel<false>, STREAM_THREADS, 0);
 	int occ_trav = occ_t < occ_tm ? occ_t : occ_tm;
 	int occ_l = 0, occ_lm = 0;
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_l, tail_kernel<false, STACK_SIZE, false, false, false, false>, TRAVERSE_THREADS, 0);
-	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_lm, tail_kernel<true, STACK_SIZE, false, false, false, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_l, tail_kernel<false, STACK_SIZE, false, false, false, false, false>, TRAVERSE_THREADS, 0);
+	cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_lm, tail_kernel<true, STACK_SIZE, false, false, false, false, false>, TRAVERSE_THREADS, 0);
 	int occ_tail = occ_l < occ_lm ? occ_l : occ_lm;
 	lc.blocks_tail = sms * (occ_tail > 0 ? occ_tail : 1);
 	lc.sms = sms;
@@ -1716,9 +1794,12 @@ void launch_tail(const SceneView& sv, const BatchParams& bp, const WaveView& wv,
 	// (light sampling, the environment map and triangle attributes: their own instantiations, so the kernels of scenes without
 	// them stay as they were; a sampled map is a light-mixture strategy, so it needs the LIGHTS kernels even without a light list)
 	const bool lights = sv.n_lights > 0 || (sv.env && sv.env_sample);
+	const bool rough = (sv.launch_flags & SV_ROUGH) != 0;   // (GGX materials: likewise)
+#define RTB_LAUNCH_TAIL_R(M, L, P, E, A, R) \
+	do { if (deep) tail_kernel<M, DEEP_STACK_SIZE, L, P, E, A, R><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); \
+	     else tail_kernel<M, STACK_SIZE, L, P, E, A, R><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); } while (0)
 #define RTB_LAUNCH_TAIL(M, L, P, E, A) \
-	do { if (deep) tail_kernel<M, DEEP_STACK_SIZE, L, P, E, A><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); \
-	     else tail_kernel<M, STACK_SIZE, L, P, E, A><<<lc.blocks_tail, TRAVERSE_THREADS, 0, st>>>(sv, bp, wv, bounce, q, threshold); } while (0)
+	do { if (rough) RTB_LAUNCH_TAIL_R(M, L, P, E, A, true); else RTB_LAUNCH_TAIL_R(M, L, P, E, A, false); } while (0)
 #define RTB_LAUNCH_TAIL_LM(P, E, A) \
 	do { if (lights) { \
 	         if (sv.has_media) RTB_LAUNCH_TAIL(true, true, P, E, A); \
@@ -1740,10 +1821,13 @@ void launch_tail(const SceneView& sv, const BatchParams& bp, const WaveView& wv,
 #undef RTB_LAUNCH_TAIL_PE
 #undef RTB_LAUNCH_TAIL_LM
 #undef RTB_LAUNCH_TAIL
+#undef RTB_LAUNCH_TAIL_R
 }
 void launch_shade(const SceneView& sv, const BatchParams& bp, const WaveView& wv, uint32_t bounce, int q, const LaunchCfg& lc, cudaStream_t st) {
 	const bool lights = sv.n_lights > 0 || (sv.env && sv.env_sample);
-#define RTB_LAUNCH_SHADE(L, P, E, A) shade_kernel<L, P, E, A><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q)
+	const bool rough = (sv.launch_flags & SV_ROUGH) != 0;
+#define RTB_LAUNCH_SHADE_R(L, P, E, A, R) shade_kernel<L, P, E, A, R><<<lc.blocks_shade, SHADE_THREADS, 0, st>>>(sv, bp, wv, bounce, q)
+#define RTB_LAUNCH_SHADE(L, P, E, A) do { if (rough) RTB_LAUNCH_SHADE_R(L, P, E, A, true); else RTB_LAUNCH_SHADE_R(L, P, E, A, false); } while (0)
 #define RTB_LAUNCH_SHADE_L(P, E, A) do { if (lights) RTB_LAUNCH_SHADE(true, P, E, A); else RTB_LAUNCH_SHADE(false, P, E, A); } while (0)
 #define RTB_LAUNCH_SHADE_PE(A) \
 	do { if (sv.env) { \
@@ -1758,6 +1842,7 @@ void launch_shade(const SceneView& sv, const BatchParams& bp, const WaveView& wv
 #undef RTB_LAUNCH_SHADE_PE
 #undef RTB_LAUNCH_SHADE_L
 #undef RTB_LAUNCH_SHADE
+#undef RTB_LAUNCH_SHADE_R
 }
 void launch_texture(const SceneView& sv, const WaveView& wv, uint32_t bounce, int q_out, const LaunchCfg& lc, cudaStream_t st) {
 	const int blocks = lc.sms * 2 < lc.blocks_stream ? lc.sms * 2 : lc.blocks_stream;   // short work lists: a small grid keeps the launch cheap

@@ -26,7 +26,8 @@ struct SceneView {
 	uint32_t n_blob;
 	int32_t tree_depth;         // depth of the world BVH in nodes (selects the stack size of the traverse kernel)
 	int32_t has_media;          // 0 none, 1 all media in the pre-test list, 2 some media are BVH leaves (selects the traverse variant)
-	int32_t has_deferred_tex;   // some material has an image / noise albedo: texture_kernel is launched after shade
+	int32_t launch_flags;       // SV_DEFERRED_TEX: some material has an image / noise albedo, texture_kernel is launched after
+	                            // shade; SV_ROUGH: some material is a GGX one (DESIGN.md §5f), the ROUGH shade / tail kernels run
 	int32_t background_mode;
 	float bg_r, bg_g, bg_b;
 	// Ray binning (bin_scan / bin_permute kernels): origin cells are counted on a 2^org_bits cube over the world BVH's
@@ -49,10 +50,12 @@ struct SceneView {
 	const float4* tri_attr;
 	const int32_t* attr_slot;
 };
+enum { SV_DEFERRED_TEX = 1, SV_ROUGH = 2 };   // bits of SceneView::launch_flags (read by the launchers only, never on the device)
 // The map's fields fill the padding after n_lights and add 16 bytes, the attribute count fills the padding before `lights`
 // and its two pointers add 16 more, so every kernel parameter after the SceneView keeps its offset modulo 16 (see BatchParams
 // below for what a moved parameter costs).
-static_assert(alignof(SceneView) == 8 && sizeof(SceneView) == 200 && offsetof(SceneView, n_tri_attr) == 148 &&
+// The ROUGH selection is a bit of launch_flags, not a field of its own, for the same reason.
+static_assert(alignof(SceneView) == 8 && sizeof(SceneView) == 200 && offsetof(SceneView, launch_flags) == 96 && offsetof(SceneView, n_tri_attr) == 148 &&
               offsetof(SceneView, lights) == 152 && offsetof(SceneView, n_lights) == 160 && offsetof(SceneView, env_width) == 164 &&
               offsetof(SceneView, env) == 168 && offsetof(SceneView, tri_attr) == 184, "SceneView layout changed");
 

@@ -170,10 +170,11 @@ int rtb_renderer_set_scene(rtb_renderer* r, rtb_scene* s) {
 		r->staged_sv.env_width = fs.env_width; r->staged_sv.env_height = fs.env_height; r->staged_sv.env_sample = fs.env_sample;
 		r->staged_sv.n_tri_attr = (int32_t)fs.tri_attr.size();
 		r->staged_sv.has_media = fs.n_media == 0 ? 0 : (fs.n_media <= (int32_t)fs.pre_list.size() ? 1 : 2);
-		r->staged_sv.has_deferred_tex = 0;
+		r->staged_sv.launch_flags = 0;
 		for (size_t i = 0; i < fs.materials.size(); ++i) {
 			const DevMaterial& m = fs.materials[i];
-			if (m.tex >= 0 && m.kind != RTB_MAT_DIFFUSE_LIGHT && (fs.textures[m.tex].kind == RTB_TEX_NOISE || fs.textures[m.tex].kind == RTB_TEX_IMAGE)) r->staged_sv.has_deferred_tex = 1;
+			if (m.tex >= 0 && m.kind != RTB_MAT_DIFFUSE_LIGHT && (fs.textures[m.tex].kind == RTB_TEX_NOISE || fs.textures[m.tex].kind == RTB_TEX_IMAGE)) r->staged_sv.launch_flags |= SV_DEFERRED_TEX;
+			if (m.kind == RTB_MAT_ROUGH_METAL || m.kind == RTB_MAT_ROUGH_DIELECTRIC) r->staged_sv.launch_flags |= SV_ROUGH;
 		}
 		r->staged_sv.background_mode = fs.background_mode;
 		r->staged_sv.bg_r = fs.background[0]; r->staged_sv.bg_g = fs.background[1]; r->staged_sv.bg_b = fs.background[2];
@@ -372,7 +373,7 @@ static void enqueue_batch(rtb_renderer* r, const WaveView& wv, const BatchParams
 		prof_begin(r, 1, st); launch_traverse(r->sv, bp, wv, b, q, r->lc, st); prof_end(r, st);
 		const bool bin_next = b + 1 < bp.max_depth && binned_bounce(r, b + 1);
 		prof_begin(r, 2, st); launch_shade(r->sv, bp, wv, b, q, r->lc, st);
-		if (r->sv.has_deferred_tex && b + 1 < bp.max_depth) launch_texture(r->sv, wv, b, q ^ 1, r->lc, st);
+		if ((r->sv.launch_flags & SV_DEFERRED_TEX) && b + 1 < bp.max_depth) launch_texture(r->sv, wv, b, q ^ 1, r->lc, st);
 		prof_end(r, st);
 		if (bin_next) { prof_begin(r, 5, st); launch_bin_rays(r->sv, wv, b + 1, q ^ 1, r->lc, st); prof_end(r, st); }   // ... and back into queue q
 		else q ^= 1;
@@ -485,7 +486,7 @@ int rtb_render(rtb_renderer* r, const rtb_render_params* p, void* user_stream) {
 	CUDA_TRY(cudaEventRecord(r->ev_t0, st));
 
 	const uint64_t launches_per_batch = 3 + 2ull * bp.max_depth + (r->tail_threshold ? count_tail_checkpoints(bp.max_depth) : 0) +
-	                                    (r->sv.has_deferred_tex ? bp.max_depth - 1 : 0) + 3ull * count_binned_bounces(r, bp.max_depth);
+	                                    ((r->sv.launch_flags & SV_DEFERRED_TEX) ? bp.max_depth - 1 : 0) + 3ull * count_binned_bounces(r, bp.max_depth);
 	if (use_graph) {
 		BatchParams key = bp; key.sample_begin = key.sample_end = key.seed = 0;   // (those three travel through device memory: call_params)
 		bool reuse = r->graph_valid && r->graph_bin_on == r->bin_on && memcmp(&r->graph_bp, &key, sizeof key) == 0 && memcmp(&r->graph_cam, &r->cam, sizeof r->cam) == 0 &&
@@ -621,7 +622,7 @@ int rtb_render_adaptive(rtb_renderer* r, const rtb_render_params* p, const rtb_a
 			for (uint32_t b = 0; b < n_batches; ++b) enqueue_batch(r, r->wv, bp, st, true);
 			CUDA_TRY(cudaGetLastError());
 			r->launches += (3 + 2ull * bp.max_depth + (r->tail_threshold ? count_tail_checkpoints(bp.max_depth) : 0) +
-			                (r->sv.has_deferred_tex ? bp.max_depth - 1 : 0) + 3ull * count_binned_bounces(r, bp.max_depth)) * n_batches;
+			                ((r->sv.launch_flags & SV_DEFERRED_TEX) ? bp.max_depth - 1 : 0) + 3ull * count_binned_bounces(r, bp.max_depth)) * n_batches;
 			r->batches += n_batches;
 			stats.samples += (uint64_t)n_active * k;
 			stats.rounds++;

@@ -162,10 +162,10 @@ int rtb_add_noise_texture(rtb_scene* s, float scale, uint32_t seed) {
 	return push_texture(s, t);
 }
 
-static int push_material(rtb_scene* s, int kind, int tex, const float a[3], float param) {
+static int push_material(rtb_scene* s, int kind, int tex, const float a[3], float param, float alpha = 0.0f) {
 	rtbs_material m{}; m.kind = kind; m.tex = tex; m.param = param;
 	m.albedo[0] = a ? a[0] : 1.0f; m.albedo[1] = a ? a[1] : 1.0f; m.albedo[2] = a ? a[2] : 1.0f;
-	s->version++; s->materials.push_back(m); return (int)s->materials.size() - 1;
+	s->version++; s->materials.push_back(m); s->mat_alpha.push_back(alpha); return (int)s->materials.size() - 1;
 }
 int rtb_add_lambertian(rtb_scene* s, int tex) {
 	if (!s || !tex_ok(s, tex)) return fail(RTB_ERR_INVALID, "rtb_add_lambertian: bad texture id");
@@ -182,6 +182,19 @@ int rtb_add_metal(rtb_scene* s, const float albedo[3], float fuzz) {
 int rtb_add_dielectric(rtb_scene* s, const float albedo[3], float ior) {
 	if (!s || !albedo) return fail(RTB_ERR_INVALID, "rtb_add_dielectric: null argument");
 	return push_material(s, RTB_MAT_DIELECTRIC, -1, albedo, ior);
+}
+// GGX materials (DESIGN.md §5f): everything is checked before the scene is touched.
+static bool rough_args_ok(const float c[3], float alpha) {
+	return c && std::isfinite(c[0]) && std::isfinite(c[1]) && std::isfinite(c[2]) && alpha >= RTB_ROUGH_ALPHA_MIN && alpha <= 1.0f;
+}
+int rtb_add_rough_metal(rtb_scene* s, const float f0[3], float alpha) {
+	if (!s || !rough_args_ok(f0, alpha)) return fail(RTB_ERR_INVALID, "rtb_add_rough_metal: needs a finite f0 and alpha in [0.001, 1]");
+	return push_material(s, RTB_MAT_ROUGH_METAL, -1, f0, 0.0f, alpha);
+}
+int rtb_add_rough_dielectric(rtb_scene* s, const float albedo[3], float ior, float alpha) {
+	if (!s || !rough_args_ok(albedo, alpha) || !(ior > 0.0f) || !std::isfinite(ior))
+		return fail(RTB_ERR_INVALID, "rtb_add_rough_dielectric: needs a finite albedo, a finite ior > 0 and alpha in [0.001, 1]");
+	return push_material(s, RTB_MAT_ROUGH_DIELECTRIC, -1, albedo, ior, alpha);
 }
 int rtb_add_diffuse_light(rtb_scene* s, int tex) {
 	if (!s || !tex_ok(s, tex)) return fail(RTB_ERR_INVALID, "rtb_add_diffuse_light: bad texture id");
@@ -407,17 +420,19 @@ extern "C" size_t rtb_scene_serialize(const rtb_scene* s, void* buf, size_t cap)
 	// A scene without sampled lights or a map is written as RTBS v1, byte for byte; one with lights only as v2 (the list
 	// appended); one with a map as v3 (the list, possibly empty, then the map).
 	// One with triangle attributes as v4: the v3 content (an empty map record when there is no map), then the attributes.
-	const bool attr = !s->tri_attrs.empty();
+	// One with a rough material as v5: the v4 content (possibly no attributes), then the GGX width of every material.
+	const bool rough = s->has_rough();
+	const bool attr = !s->tri_attrs.empty() || rough;
 	const bool env = s->env_width > 0 || attr;
 	const bool lights = !s->sampled_lights.empty() || env;
 	const size_t env_floats = (size_t)s->env_width * s->env_height * 3;
 	size_t need = sizeof(rtbs_header) + s->textures.size() * sizeof(rtbs_texture) + s->materials.size() * sizeof(rtbs_material) +
 	              s->objects.size() * sizeof(rtbs_object) + s->children.size() * 4 + s->blob.size() +
 	              (lights ? 4 + s->sampled_lights.size() * 4 : 0) + (env ? sizeof(rtbs_env) + env_floats * 4 : 0) +
-	              (attr ? 4 + s->tri_attrs.size() * sizeof(rtbs_tri_attr) : 0);
+	              (attr ? 4 + s->tri_attrs.size() * sizeof(rtbs_tri_attr) : 0) + (rough ? 4 + s->mat_alpha.size() * 4 : 0);
 	if (!buf || cap < need) return need;
 	rtbs_header h{}; h.magic = RTBS_MAGIC;
-	h.version = attr ? RTBS_VERSION_ATTR : env ? RTBS_VERSION_ENV : lights ? RTBS_VERSION_LIGHTS : RTBS_VERSION;
+	h.version = rough ? RTBS_VERSION_ROUGH : attr ? RTBS_VERSION_ATTR : env ? RTBS_VERSION_ENV : lights ? RTBS_VERSION_LIGHTS : RTBS_VERSION;
 	h.n_textures = (uint32_t)s->textures.size(); h.n_materials = (uint32_t)s->materials.size();
 	h.n_objects = (uint32_t)s->objects.size(); h.n_children = (uint32_t)s->children.size();
 	h.n_blob_bytes = (uint32_t)s->blob.size(); h.root_object = s->root; h.background_mode = s->background_mode;
@@ -446,6 +461,11 @@ extern "C" size_t rtb_scene_serialize(const rtb_scene* s, void* buf, size_t cap)
 		const uint32_t n = (uint32_t)s->tri_attrs.size();
 		put(&n, 4);
 		put(s->tri_attrs.data(), s->tri_attrs.size() * sizeof(rtbs_tri_attr));
+	}
+	if (rough) {
+		const uint32_t n = (uint32_t)s->mat_alpha.size();
+		put(&n, 4);
+		put(s->mat_alpha.data(), s->mat_alpha.size() * 4);
 	}
 	return need;
 }
@@ -1154,7 +1174,7 @@ int flatten(rtb_scene& s, FlatScene& out, const GpuBuildContext* gpu) {
 	out.materials.resize(s.materials.size());
 	for (size_t i = 0; i < s.materials.size(); ++i) {
 		const rtbs_material& m = s.materials[i]; DevMaterial& d = out.materials[i];
-		d.kind = m.kind; d.tex = m.tex; d.param = m.param; d.pad = 0.0f;
+		d.kind = m.kind; d.tex = m.tex; d.param = m.param; d.pad = s.mat_alpha[i];   // the GGX width (0 unless rough)
 		d.albedo[0] = m.albedo[0]; d.albedo[1] = m.albedo[1]; d.albedo[2] = m.albedo[2]; d.albedo[3] = 0.0f;
 	}
 	out.textures.resize(s.textures.size());
@@ -1220,6 +1240,9 @@ extern "C" int rtb_scene_flatten_hash(rtb_scene* s, uint64_t* hash_out) {
 	if (!fs.tri_attr.empty()) { // (likewise for triangle attributes)
 		mix(fs.tri_attr.data(), fs.tri_attr.size() * sizeof(rtb::DevTriAttr));
 		mix(fs.attr_slot.data(), fs.attr_slot.size() * sizeof(int32_t));
+	}
+	if (s->has_rough()) {       // (likewise for the GGX widths)
+		for (const rtb::DevMaterial& m : fs.materials) mix(&m.pad, sizeof m.pad);
 	}
 	*hash_out = h;
 	return RTB_OK;

@@ -30,6 +30,10 @@ struct rtb_scene {
 	// rtb_add_mesh_ex: corner attributes of mesh triangles; triangle object k carries tri_attrs[objects[k].aux - 1] when its
 	// aux is non-zero (empty: no attributes, the scene serialises as v1 - v3).
 	std::vector<rtbs_tri_attr> tri_attrs;
+	// GGX width per material (rtb_add_rough_metal / rtb_add_rough_dielectric; 0 for the other kinds).  The scene serialises
+	// as v5 and the flatten hash covers the widths only when a rough material exists.
+	std::vector<float> mat_alpha;
+	bool has_rough() const { for (const rtbs_material& m : materials) if (m.kind == RTB_MAT_ROUGH_METAL || m.kind == RTB_MAT_ROUGH_DIELECTRIC) return true; return false; }
 
 	// Filled by flatten(): the world BVH in the reference's node layout (parity hook).
 	std::vector<rtb_bvh_node> world_nodes;

@@ -5,7 +5,7 @@
 //   rtb_app [scene] [--width W] [--height H] [--spp N] [--depth D] [--seed S] [--gpus N]
 //           [--out image.png|image.ppm|image.pfm] [--resume ckpt.rtba] [--checkpoint ckpt.rtba] [--sample-lights]
 //           [--target-db D [--min-spp N]] [--env map.pfm [--env-scale S] [--sample-env]]
-//   rtb_app --obj model.obj [--smooth [--obj-texture image.ppm]] [...]
+//   rtb_app --obj model.obj [--smooth [--obj-texture image.ppm]] [--obj-material clay|rough-metal|rough-glass [--alpha A]] [...]
 //                                     a Wavefront OBJ mesh (MeshHandle) on a checkered floor under the sky
 //
 // scene = one of rtb_scenes_name(i) (default book2_bouncing, which goes through SceneBook2BVH::Factory
@@ -26,6 +26,9 @@
 // --smooth loads the --obj model with MeshHandle::LoadObjShaded: smooth shading from its `vn` normals (computed from the faces
 // when it has none) and its `vt` texture coordinates (DESIGN.md §5e).  --obj-texture image.ppm (binary P6) then maps that
 // image onto the model through its texture coordinates; it needs --smooth and a model with `vt` on every corner.
+// --obj-material picks the model's material: clay (the default Lambertian), rough-metal (a copper-coloured GGX conductor) or
+// rough-glass (GGX glass, ior 1.5), of width --alpha A (default 0.2; DESIGN.md §5f).  --obj-texture implies the textured
+// Lambertian, so it takes no rough material; --alpha needs a rough one.
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -58,7 +61,8 @@ int main(int argc, char** argv) {
 	bool sample_lights = false;
 	double target_db = -1.0;
 	int min_spp = 64;
-	std::string env_path, obj_texture;
+	std::string env_path, obj_texture, obj_material;
+	float alpha = -1.0f;
 	bool smooth = false;
 	float env_scale = 1.0f;
 	bool sample_env = false;
@@ -84,6 +88,8 @@ int main(int argc, char** argv) {
 		else if (a == "--sample-env") sample_env = true;
 		else if (a == "--smooth") smooth = true;
 		else if (a == "--obj-texture" && i + 1 < argc) obj_texture = argv[++i];
+		else if (a == "--obj-material" && i + 1 < argc) obj_material = argv[++i];
+		else if (a == "--alpha" && i + 1 < argc) alpha = (float)atof(argv[++i]);
 		else if (a == "--list") { for (int k = 0; k < rtb_scenes_count(); ++k) printf("%s\n", rtb_scenes_name(k)); return 0; }
 		else scene_name = a;
 	}
@@ -93,6 +99,13 @@ int main(int argc, char** argv) {
 	}
 	if ((smooth || !obj_texture.empty()) && obj_path.empty()) { fprintf(stderr, "rtb_app: --smooth and --obj-texture apply to an --obj model\n"); return 1; }
 	if (!obj_texture.empty() && !smooth) { fprintf(stderr, "rtb_app: --obj-texture needs --smooth (the texture coordinates come with LoadObjShaded)\n"); return 1; }
+	const bool rough = obj_material == "rough-metal" || obj_material == "rough-glass";
+	if ((!obj_material.empty() || alpha >= 0.0f) && obj_path.empty()) { fprintf(stderr, "rtb_app: --obj-material and --alpha apply to an --obj model\n"); return 1; }
+	if (!obj_material.empty() && !rough && obj_material != "clay") { fprintf(stderr, "rtb_app: --obj-material: expected clay, rough-metal or rough-glass, got %s\n", obj_material.c_str()); return 1; }
+	if (alpha >= 0.0f && !rough) { fprintf(stderr, "rtb_app: --alpha needs --obj-material rough-metal or rough-glass\n"); return 1; }
+	if (rough && !obj_texture.empty()) { fprintf(stderr, "rtb_app: --obj-texture makes the model a textured Lambertian; drop --obj-material %s\n", obj_material.c_str()); return 1; }
+	if (rough && alpha < 0.0f) alpha = 0.2f;
+	if (rough && !(alpha >= RTB_ROUGH_ALPHA_MIN && alpha <= 1.0f)) { fprintf(stderr, "rtb_app: --alpha must be in [0.001, 1]\n"); return 1; }
 	if (sample_env && env_path.empty()) { fprintf(stderr, "rtb_app: --sample-env needs --env map.pfm\n"); return 1; }
 	std::vector<float> env_rgb;
 	int env_w = 0, env_h = 0;
@@ -128,8 +141,12 @@ int main(int argc, char** argv) {
 				skin = std::make_unique<image_texture>(px.data(), tw, th, 3);
 				skin_mat = std::make_unique<Lambertian>(skin.get());
 			}
-			MeshHandle model = skin_mat ? MeshHandle::MakeMesh(mesh, skin_mat.get()) : MeshHandle::MakeMesh(mesh, &clay);
-			printf("%d triangles%s.\n", model.triangleCount(), smooth ? (skin ? ", smooth, textured" : ", smooth") : "");
+			std::unique_ptr<GeoIndependantMaterial> rough_mat;
+			if (obj_material == "rough-metal") rough_mat = std::make_unique<RoughMetal>(glm::vec3(0.95f, 0.64f, 0.54f), alpha);
+			else if (obj_material == "rough-glass") rough_mat = std::make_unique<RoughDielectric>(1.5f, alpha);
+			GeoIndependantMaterial* model_mat = skin_mat ? static_cast<GeoIndependantMaterial*>(skin_mat.get()) : rough_mat ? rough_mat.get() : &clay;
+			MeshHandle model = MeshHandle::MakeMesh(mesh, model_mat);
+			printf("%d triangles%s%s.\n", model.triangleCount(), smooth ? (skin ? ", smooth, textured" : ", smooth") : "", rough ? (obj_material == "rough-metal" ? ", rough metal" : ", rough glass") : "");
 			const glm::vec3 lo = model.getBounds().getMin(), hi = model.getBounds().getMax(), mid = (lo + hi) * 0.5f;
 			const float size = glm::length(hi - lo);
 			solid_texture dark(glm::vec3(.2f, .3f, .1f)), light(glm::vec3(.9f, .9f, .9f));

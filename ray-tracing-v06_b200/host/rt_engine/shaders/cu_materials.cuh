@@ -56,6 +56,17 @@ class Dielectric : public GeoIndependantMaterial {
 public:
 	Dielectric(glm::vec3 albedo, float ior) { rtb_material = rtb_host::check(rtb_add_dielectric(rtb_host::scene(), &albedo.x, ior), "Dielectric"); }
 };
+// GGX microfacet materials (DESIGN.md §5f; not in the reference): width alpha in [0.001, 1].
+class RoughMetal : public GeoIndependantMaterial {
+public:
+	RoughMetal(glm::vec3 f0, float alpha) { rtb_material = rtb_host::check(rtb_add_rough_metal(rtb_host::scene(), &f0.x, alpha), "RoughMetal"); }
+};
+class RoughDielectric : public GeoIndependantMaterial {
+public:
+	RoughDielectric(float ior, float alpha, glm::vec3 albedo = glm::vec3(1.0f)) {
+		rtb_material = rtb_host::check(rtb_add_rough_dielectric(rtb_host::scene(), &albedo.x, ior, alpha), "RoughDielectric");
+	}
+};
 class diffuse_light : public GeoIndependantMaterial {
 public:
 	diffuse_light(glm::vec3 emit) { solid_texture t(emit); rtb_material = rtb_host::check(rtb_add_diffuse_light(rtb_host::scene(), t.rtb_texture), "diffuse_light"); }
