@@ -45,7 +45,7 @@ class RtbError(RuntimeError):
 
 def build(verbose: bool = False) -> None:
     """Compile librtb200.so and librtb200_scenes.so in-tree (nvcc cross-compiles without a GPU)."""
-    res = subprocess.run(["make", "-C", str(_HERE), "all"], capture_output=True, text=True)
+    res = subprocess.run(["make", f"-j{os.cpu_count() or 1}", "-C", str(_HERE), "all"], capture_output=True, text=True)
     if verbose or res.returncode != 0:
         print(res.stdout[-4000:])
         print(res.stderr[-4000:])

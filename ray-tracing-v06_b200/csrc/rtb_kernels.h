@@ -26,8 +26,8 @@ struct SceneView {
 	uint32_t n_blob;
 	int32_t tree_depth;         // depth of the world BVH in nodes (selects the stack size of the traverse kernel)
 	int32_t has_media;          // 0 none, 1 all media in the pre-test list, 2 some media are BVH leaves (selects the traverse variant)
-	int32_t launch_flags;       // SV_DEFERRED_TEX: some material has an image / noise albedo, texture_kernel is launched after
-	                            // shade; SV_ROUGH: some material is a GGX one (DESIGN.md §5f), the ROUGH shade / tail kernels run
+	int32_t launch_flags;       // the scene's part of the feature word (below); SV_DEFERRED_TEX: some material has an image /
+	                            // noise albedo, texture_kernel is launched after shade
 	int32_t background_mode;
 	float bg_r, bg_g, bg_b;
 	// Ray binning (bin_scan / bin_permute kernels): origin cells are counted on a 2^org_bits cube over the world BVH's
@@ -50,11 +50,22 @@ struct SceneView {
 	const float4* tri_attr;
 	const int32_t* attr_slot;
 };
-enum { SV_DEFERRED_TEX = 1, SV_ROUGH = 2 };   // bits of SceneView::launch_flags (read by the launchers only, never on the device)
+// The feature word F of the shade and tail kernels (their last template parameter): which code a scene or a batch needs.
+// Each bit is one feature, and a kernel without a feature's bit is the kernel of scenes without that feature.  A new
+// feature takes the next bit, so every existing word, and the instantiation and kernel name it stands for, stays.
+//   F_LIGHTS  the light mixture (DESIGN.md §5b): sampled lights, or a sampled environment map (one more strategy of it)
+//   F_LIST    an adaptive round (DESIGN.md §5c): local pixels come from BatchParams::pixel_list()
+//   F_ENV     an environment map (DESIGN.md §5d): a miss returns its texel
+//   F_ATTR    triangle attributes (DESIGN.md §5e)
+//   F_ROUGH   GGX materials (DESIGN.md §5f)
+enum : uint32_t { F_LIGHTS = 1, F_LIST = 2, F_ENV = 4, F_ATTR = 8, F_ROUGH = 16, F_WORDS = 32 };
+// SceneView::launch_flags (read by the launchers only, never on the device): the word's scene bits, computed once where the
+// scene is staged (every bit but F_LIST, which the launchers add from the batch), and SV_DEFERRED_TEX above the word.
+enum : uint32_t { SV_DEFERRED_TEX = 1u << 16 };
 // The map's fields fill the padding after n_lights and add 16 bytes, the attribute count fills the padding before `lights`
 // and its two pointers add 16 more, so every kernel parameter after the SceneView keeps its offset modulo 16 (see BatchParams
 // below for what a moved parameter costs).
-// The ROUGH selection is a bit of launch_flags, not a field of its own, for the same reason.
+// The scene's feature bits are part of launch_flags, not fields of their own, for the same reason.
 static_assert(alignof(SceneView) == 8 && sizeof(SceneView) == 200 && offsetof(SceneView, launch_flags) == 96 && offsetof(SceneView, n_tri_attr) == 148 &&
               offsetof(SceneView, lights) == 152 && offsetof(SceneView, n_lights) == 160 && offsetof(SceneView, env_width) == 164 &&
               offsetof(SceneView, env) == 168 && offsetof(SceneView, tri_attr) == 184, "SceneView layout changed");

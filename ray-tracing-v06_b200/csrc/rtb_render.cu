@@ -170,12 +170,18 @@ int rtb_renderer_set_scene(rtb_renderer* r, rtb_scene* s) {
 		r->staged_sv.env_width = fs.env_width; r->staged_sv.env_height = fs.env_height; r->staged_sv.env_sample = fs.env_sample;
 		r->staged_sv.n_tri_attr = (int32_t)fs.tri_attr.size();
 		r->staged_sv.has_media = fs.n_media == 0 ? 0 : (fs.n_media <= (int32_t)fs.pre_list.size() ? 1 : 2);
-		r->staged_sv.launch_flags = 0;
+		// The scene's part of the feature word that selects the shade and tail kernels (rtb_kernels.h), decided here only.
+		// (A sampled map is a strategy of the light mixture, so it needs the LIGHTS kernels even without a light list.)
+		uint32_t flags = 0;
+		if (fs.lights.size() > 0 || (fs.env_width > 0 && fs.env_sample)) flags |= F_LIGHTS;
+		if (fs.env_width > 0) flags |= F_ENV;
+		if (!fs.tri_attr.empty()) flags |= F_ATTR;
 		for (size_t i = 0; i < fs.materials.size(); ++i) {
 			const DevMaterial& m = fs.materials[i];
-			if (m.tex >= 0 && m.kind != RTB_MAT_DIFFUSE_LIGHT && (fs.textures[m.tex].kind == RTB_TEX_NOISE || fs.textures[m.tex].kind == RTB_TEX_IMAGE)) r->staged_sv.launch_flags |= SV_DEFERRED_TEX;
-			if (m.kind == RTB_MAT_ROUGH_METAL || m.kind == RTB_MAT_ROUGH_DIELECTRIC) r->staged_sv.launch_flags |= SV_ROUGH;
+			if (m.tex >= 0 && m.kind != RTB_MAT_DIFFUSE_LIGHT && (fs.textures[m.tex].kind == RTB_TEX_NOISE || fs.textures[m.tex].kind == RTB_TEX_IMAGE)) flags |= SV_DEFERRED_TEX;
+			if (m.kind == RTB_MAT_ROUGH_METAL || m.kind == RTB_MAT_ROUGH_DIELECTRIC) flags |= F_ROUGH;
 		}
+		r->staged_sv.launch_flags = (int32_t)flags;
 		r->staged_sv.background_mode = fs.background_mode;
 		r->staged_sv.bg_r = fs.background[0]; r->staged_sv.bg_g = fs.background[1]; r->staged_sv.bg_b = fs.background[2];
 		for (int k = 0; k < 3; ++k) { r->world_min[k] = fs.world_min[k]; r->world_max[k] = fs.world_max[k]; }

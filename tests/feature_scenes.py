@@ -1,6 +1,8 @@
 """TEST INFRASTRUCTURE: one scene builder whose switches pick, one by one, the template instantiations the kernel launchers
-choose from (launch_traverse / launch_shade / launch_tail in rtb_kernels.cu), and the case list that the schedule tests
-(tests/test_gpu_schedules.py, tests/test_gpu_adaptive_scale.py) run.  Nothing here renders.
+choose from, and the case list that the schedule tests (tests/test_gpu_schedules.py, tests/test_gpu_adaptive_scale.py) run.
+Nothing here renders.  The shade and tail kernels are selected by their feature word (rtb_kernels.h), whose scene bits are
+decided in one place, where rtb_render.cu stages the flattened scene (SceneView::launch_flags); launch_traverse and
+launch_tail in rtb_kernels.cu add the stack size and media variant.
 
 What selects what, as the launchers read a flattened scene:
   media     none; "pre": one medium, tested before the walk (has_media = 1); "bvh": more media than the eight the
@@ -60,7 +62,7 @@ class Case:
         return (self.has_media, {"shallow": 16, "normal": 32, "deep": 64}[self.tree], bool(list_mode and self.has_media))
 
     def shade_kernel(self, list_mode: bool) -> tuple:
-        """(LIGHTS, LIST, ENV, ATTR)."""
+        """(LIGHTS, LIST, ENV, ATTR): bits 0-3 of the feature word."""
         return (self.LIGHTS, bool(list_mode), self.ENV, self.attr)
 
     def tail_kernel(self, list_mode: bool) -> tuple:
