@@ -685,6 +685,52 @@ Ray camera_ray(const rtb_camera& cam, float s, float t, Ctx& ctx) {
 	return Ray(o, d, time);
 }
 
+// Renders samples [s0, s1) of every pixel, rows handed out to `threads` workers; ADDS into sum (and sum2), and stores the
+// number of traced segments in *rays_out.  trace(ray, ctx) is the integrator: it returns the sample's radiance.
+template <class Trace>
+void render_rows(const rtb_camera& cam, uint32_t W, uint32_t H, uint32_t s0, uint32_t s1, uint32_t seed, int mode, int threads,
+                 bool want_uv, float* sum, float* sum2, uint64_t* rays_out, const Trace& trace) {
+	if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
+	if (threads <= 0) threads = 1;
+	std::atomic<uint32_t> next_row{0};
+	std::atomic<uint64_t> total_rays{0};
+	const float px = 1.0f / (float)W, py = 1.0f / (float)H;   // pixel_size  Renderer.cu:188
+	auto worker = [&]() {
+		uint64_t rays = 0;
+		for (;;) {
+			uint32_t y = next_row.fetch_add(1);
+			if (y >= H) break;
+			for (uint32_t x = 0; x < W; ++x) {
+				uint32_t gid = y * W + x;
+				Xorwow xw((uint64_t)seed + gid);             // init_random_states: cuRandom(seed + gid, 0, 0)  Renderer.cu:22-29
+				Ctx ctx; ctx.mode = mode; ctx.seed = seed; ctx.pixel = gid; ctx.xw = &xw; ctx.want_uv = want_uv;
+				float ndcx = std::fmaf(((float)x + 0.5f) * px, 2.0f, -1.0f);   // Renderer.cu:192
+				float ndcy = std::fmaf(((float)y + 0.5f) * py, 2.0f, -1.0f);
+				float ax = 0, ay = 0, az = 0, qx = 0, qy = 0, qz = 0;
+				for (uint32_t smp = s0; smp < s1; ++smp) {
+					ctx.sample = smp;
+					ctx.begin(CAMERA_BOUNCE);
+					float jx, jy; ctx.in_unit_disc(jx, jy, false);          // Renderer.cu:199
+					Ray ray = camera_ray(cam, std::fmaf(jx, px, ndcx), std::fmaf(jy, py, ndcy), ctx);
+					V3 c = trace(ray, ctx);
+					ax += c.x; ay += c.y; az += c.z;
+					qx = std::fmaf(c.x, c.x, qx); qy = std::fmaf(c.y, c.y, qy); qz = std::fmaf(c.z, c.z, qz);
+				}
+				float* o = sum + 4 * (size_t)gid;
+				o[0] += ax; o[1] += ay; o[2] += az; o[3] += (float)(s1 - s0);
+				if (sum2) { float* q = sum2 + 4 * (size_t)gid; q[0] += qx; q[1] += qy; q[2] += qz; q[3] += (float)(s1 - s0); }
+				rays += ctx.rays;
+			}
+		}
+		total_rays += rays;
+	};
+	std::vector<std::thread> pool;
+	for (int t = 1; t < threads; ++t) pool.emplace_back(worker);
+	worker();
+	for (auto& t : pool) t.join();
+	if (rays_out) *rays_out = total_rays.load();
+}
+
 }  // namespace
 
 // ================================================================= C API
@@ -723,46 +769,9 @@ int orc_render(const orc_scene* s, const rtb_camera* cam, uint32_t W, uint32_t H
                uint32_t seed, int mode, int threads, float* sum, float* sum2, uint64_t* rays_out) {
 	if (!s || !cam || !sum || W == 0 || H == 0) { g_err = "orc_render: bad argument"; return -1; }
 	if (mode == ORC_RNG_XORWOW && s0 != 0) { g_err = "orc_render: XORWOW mode renders from sample 0 (per-pixel sequential streams)"; return -1; }
-	if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
-	if (threads <= 0) threads = 1;
 	const Scene& sc = s->sc;
-	std::atomic<uint32_t> next_row{0};
-	std::atomic<uint64_t> total_rays{0};
-	const float px = 1.0f / (float)W, py = 1.0f / (float)H;   // pixel_size  Renderer.cu:188
-	auto worker = [&]() {
-		uint64_t rays = 0;
-		for (;;) {
-			uint32_t y = next_row.fetch_add(1);
-			if (y >= H) break;
-			for (uint32_t x = 0; x < W; ++x) {
-				uint32_t gid = y * W + x;
-				Xorwow xw((uint64_t)seed + gid);             // init_random_states: cuRandom(seed + gid, 0, 0)  Renderer.cu:22-29
-				Ctx ctx; ctx.mode = mode; ctx.seed = seed; ctx.pixel = gid; ctx.xw = &xw; ctx.want_uv = sc.any_uv_texture;
-				float ndcx = std::fmaf(((float)x + 0.5f) * px, 2.0f, -1.0f);   // Renderer.cu:192
-				float ndcy = std::fmaf(((float)y + 0.5f) * py, 2.0f, -1.0f);
-				float ax = 0, ay = 0, az = 0, qx = 0, qy = 0, qz = 0;
-				for (uint32_t smp = s0; smp < s1; ++smp) {
-					ctx.sample = smp;
-					ctx.begin(CAMERA_BOUNCE);
-					float jx, jy; ctx.in_unit_disc(jx, jy, false);          // Renderer.cu:199
-					Ray ray = camera_ray(*cam, std::fmaf(jx, px, ndcx), std::fmaf(jy, py, ndcy), ctx);
-					V3 c = sample_world(sc, ray, max_depth, ctx);
-					ax += c.x; ay += c.y; az += c.z;
-					qx = std::fmaf(c.x, c.x, qx); qy = std::fmaf(c.y, c.y, qy); qz = std::fmaf(c.z, c.z, qz);
-				}
-				float* o = sum + 4 * (size_t)gid;
-				o[0] += ax; o[1] += ay; o[2] += az; o[3] += (float)(s1 - s0);
-				if (sum2) { float* q = sum2 + 4 * (size_t)gid; q[0] += qx; q[1] += qy; q[2] += qz; q[3] += (float)(s1 - s0); }
-				rays += ctx.rays;
-			}
-		}
-		total_rays += rays;
-	};
-	std::vector<std::thread> pool;
-	for (int t = 1; t < threads; ++t) pool.emplace_back(worker);
-	worker();
-	for (auto& t : pool) t.join();
-	if (rays_out) *rays_out = total_rays.load();
+	render_rows(*cam, W, H, s0, s1, seed, mode, threads, sc.any_uv_texture, sum, sum2, rays_out,
+	            [&](const Ray& ray, Ctx& ctx) { return sample_world(sc, ray, max_depth, ctx); });
 	return 0;
 }
 

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE: the environment-map scenes and hand-derived answers shared by tests/test_cpu_environment.py and
 tests/test_gpu_environment.py (DESIGN.md §5d).  Nothing here renders: the tests render these scenes on the CPU oracle
-(tests/env_oracle.py) and on the GPU."""
+(tests/feature_oracle.py) and on the GPU."""
 from __future__ import annotations
 
 import numpy as np

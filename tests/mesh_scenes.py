@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE: the mesh scenes and hand-derived answers shared by tests/test_cpu_mesh_attributes.py and
 tests/test_gpu_mesh_attributes.py (DESIGN.md §5e).  Nothing here renders: the tests render these scenes on the CPU oracle
-(tests/mesh_oracle.py) and on the GPU."""
+(tests/feature_oracle.py) and on the GPU."""
 from __future__ import annotations
 
 import numpy as np

@@ -1,5 +1,5 @@
 """CPU tests of the HDR environment map (DESIGN.md §5d): the rtb_scene_set_environment API, the RTBS v3 blob, the flatten
-hash, the map's sampler and pdf on the CPU restatement (tests/env_oracle.cpp), and the hand-derived answers rendered on
+hash, the map's sampler and pdf on the CPU restatement (tests/feature_oracle.cpp), and the hand-derived answers rendered on
 that restatement: a 1 x 1 map is the constant background, the axis directions read the tabulated texels, one lit texel
 gives its irradiance integral, and the white furnace returns exactly 1."""
 import ctypes as C
@@ -9,9 +9,8 @@ import pytest
 from scipy import stats
 
 import env_scenes as es
-from env_oracle import EnvOracleScene
+from feature_oracle import FeatureOracleScene
 from helpers import parse_blob
-from light_oracle import LightOracleScene
 
 ERR_INVALID = -1
 
@@ -58,7 +57,7 @@ def test_api_validation(rtb):
 
 def test_blob_round_trips(rtb, orc):
     """Without a map: v1 / v2 byte for byte.  With one: v3 = the v1 body, the light list (n may be 0), rtbs_env and the
-    scaled texels; setting then clearing restores the bytes and the flatten hash; the plain and light oracles refuse v3."""
+    scaled texels; setting then clearing restores the bytes and the flatten hash; the plain oracle refuses v3."""
     s = rtb.Scene.named("book2_final")
     v1, h1 = s.serialize(), s.flatten_hash()
     m = es.distinct_map(6, 4)
@@ -77,10 +76,9 @@ def test_blob_round_trips(rtb, orc):
     assert h3 != h1
     s.set_environment(m, scale=(2.0, 0.5, 1.0), sample=False)
     assert s.flatten_hash() not in (h1, h3)                     # the sampling flag is part of the flattened scene
-    for oracle in (orc.OracleScene, LightOracleScene):
-        with pytest.raises(RuntimeError, match="version"):
-            oracle(v3)
-    assert EnvOracleScene(v3).dims() == (6, 4)
+    with pytest.raises(RuntimeError, match="version"):
+        orc.OracleScene(v3)
+    assert FeatureOracleScene(v3).dims() == (6, 4)
     s.sample_lights(s.info.light_ids)                           # lights and a map: the list, then the map
     v3l = s.serialize()
     n = len(s.info.light_ids)
@@ -104,7 +102,7 @@ def _env(rtb, m, sample=True, scale=(1, 1, 1)):
     s = rtb.Scene()
     s.set_root(s.sphere((0, 0, 0), 1.0, s.lambertian((0.5, 0.5, 0.5))))
     s.set_environment(m, scale=scale, sample=sample)
-    return EnvOracleScene(s.serialize())
+    return FeatureOracleScene(s.serialize())
 
 
 def test_tables(rtb):
@@ -186,9 +184,9 @@ def test_axis_directions_read_the_tabulated_texels(rtb):
 
 def test_one_by_one_map_is_the_constant_background(rtb):
     s, cam = es.sky_scene(rtb)
-    a, a2, ra = EnvOracleScene(s.serialize()).render(cam, 24, 16, 0, 8, 12, seed=3, want_sum2=True)
+    a, a2, ra = FeatureOracleScene(s.serialize()).render(cam, 24, 16, 0, 8, 12, seed=3, want_sum2=True)
     s.set_environment(np.float32(es.SKY).reshape(1, 1, 3))
-    b, b2, rb = EnvOracleScene(s.serialize()).render(cam, 24, 16, 0, 8, 12, seed=3, want_sum2=True)
+    b, b2, rb = FeatureOracleScene(s.serialize()).render(cam, 24, 16, 0, 8, 12, seed=3, want_sum2=True)
     assert np.array_equal(a, b) and np.array_equal(a2, b2) and ra == rb
     assert (a[..., 2] > 0).all()
 
@@ -196,7 +194,7 @@ def test_one_by_one_map_is_the_constant_background(rtb):
 def test_orientation_on_the_oracle(rtb):
     want = es.orientation_map()
     s = es.orientation_scene(rtb)
-    o = EnvOracleScene(s.serialize())
+    o = FeatureOracleScene(s.serialize())
     for axis, (i, j) in es.axis_texels().items():
         a, _, _ = o.render(es.orientation_camera(rtb, axis), 1, 1, 0, 16, 4, seed=1)
         assert np.array_equal(a[0, 0, :3] / 16, want[j, i]), (axis, a[0, 0], want[j, i])
@@ -217,7 +215,7 @@ def test_one_texel_irradiance_on_the_oracle(rtb):
     var = {}
     for sample in (False, True):
         s, cam = es.one_texel_scene(rtb, sample)
-        a, a2, _ = EnvOracleScene(s.serialize()).render(cam, 8, 8, 0, 2048, 2, seed=5 + sample, want_sum2=True)
+        a, a2, _ = FeatureOracleScene(s.serialize()).render(cam, 8, 8, 0, 2048, 2, seed=5 + sample, want_sum2=True)
         var[sample] = check_mean(a, a2, 2048, want, f"oracle one texel sample={sample}")
     print(f"variance sampled / unsampled {var[True] / var[False]:.3f}")
     assert var[True] <= 0.25 * var[False]
@@ -225,10 +223,10 @@ def test_one_texel_irradiance_on_the_oracle(rtb):
 
 def test_furnace_on_the_oracle(rtb):
     s, cam = es.furnace_scene(rtb, False)
-    a, _, _ = EnvOracleScene(s.serialize()).render(cam, 16, 16, 0, 64, 8, seed=7)
+    a, _, _ = FeatureOracleScene(s.serialize()).render(cam, 16, 16, 0, 64, 8, seed=7)
     assert np.array_equal(a[..., :3], np.full((16, 16, 3), 64.0, np.float32))
     s, cam = es.furnace_scene(rtb, True)
-    a, a2, _ = EnvOracleScene(s.serialize()).render(cam, 16, 16, 0, 1024, 8, seed=7, want_sum2=True)
+    a, a2, _ = FeatureOracleScene(s.serialize()).render(cam, 16, 16, 0, 1024, 8, seed=7, want_sum2=True)
     check_mean(a, a2, 1024, 1.0, "oracle furnace sampled", k=3.0)
 
 

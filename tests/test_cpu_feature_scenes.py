@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 
 import feature_scenes as fs
-from mesh_oracle import MeshOracleScene
+from feature_oracle import FeatureOracleScene
 
 
 def test_cases_cover_every_instantiation():
@@ -28,12 +28,12 @@ def test_scene_selects_what_its_case_says(rtb, case):
     else:
         stats = scene.flatten_stats()
     fs.check_selection(case, scene, stats)
-    MeshOracleScene(scene.serialize())
+    FeatureOracleScene(scene.serialize())
 
 
 def test_oracle_renders_a_case(rtb):
     """The oracle half of one parity case of tests/test_gpu_schedules.py (every switch on, at a smaller size)."""
     case = fs.Case("bvh", "normal", True, "sampled", True)
     scene, cam = fs.build(rtb, case)
-    ref, _, rays = MeshOracleScene(scene.serialize()).render(cam, 48, 32, 0, 4, 24, seed=1984)
+    ref, _, rays = FeatureOracleScene(scene.serialize()).render(cam, 48, 32, 0, 4, 24, seed=1984)
     assert rays > 48 * 32 * 4 and np.isfinite(ref).all() and (ref[..., 3] == 4).all() and ref[..., :3].sum() > 0

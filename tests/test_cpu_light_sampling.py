@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 from helpers import parse_blob
-from light_oracle import RNG_XORWOW, LightOracleScene
+from feature_oracle import RNG_XORWOW, FeatureOracleScene
 
 ERR_INVALID, ERR_UNSUPPORTED = -1, -5
 
@@ -74,13 +74,13 @@ def test_blob_round_trips(rtb, orc):
     assert len(v2) == len(v1) + 4 + 4 * n
     assert v2[8:len(v1)] == v1[8:] and v2[:4] == v1[:4]
     assert np.array_equal(np.frombuffer(v2[len(v1):], dtype=np.int32), np.array([n, *s.info.light_ids], dtype=np.int32))
-    assert LightOracleScene(v2).num_lights == n and LightOracleScene(v1).num_lights == 0
+    assert FeatureOracleScene(v2).num_lights == n and FeatureOracleScene(v1).num_lights == 0
     with pytest.raises(RuntimeError, match="version"):
         orc.OracleScene(v2)                      # the plain oracle cannot drop a light list silently: it refuses the blob
     s.sample_lights([])
     assert s.serialize() == v1
     with pytest.raises(RuntimeError, match="bad light list"):
-        LightOracleScene(v2[:len(v1)] + np.array([0], dtype=np.int32).tobytes())
+        FeatureOracleScene(v2[:len(v1)] + np.array([0], dtype=np.int32).tobytes())
 
 
 def test_named_scenes_list_their_lights_without_setting_them(rtb):
@@ -109,15 +109,15 @@ def test_xorwow_mode_refuses_light_sampling(rtb, orc):
     s = rtb.Scene.named("book2_cornell"); cam = s.info.camera
     s.sample_lights(s.info.light_ids)
     with pytest.raises(RuntimeError, match="XORWOW"):
-        LightOracleScene(s.serialize()).render(cam, 8, 8, 0, 2, 4, seed=1, mode=RNG_XORWOW)
+        FeatureOracleScene(s.serialize()).render(cam, 8, 8, 0, 2, 4, seed=1, mode=RNG_XORWOW)
 
 
 @pytest.mark.parametrize("name", ["book2_simple_light", "book2_cornell_smoke"])
 def test_light_oracle_without_lights_is_the_oracle(rtb, orc, name):
-    """tests/light_oracle.cpp on a blob without a light list renders exactly what the oracle renders: same sums, same rays."""
+    """tests/feature_oracle.cpp on a blob without a light list renders exactly what the oracle renders: same sums, same rays."""
     s = rtb.Scene.named(name); cam = s.info.camera
     a, a2, ra = orc.OracleScene(s.serialize()).render(cam, 24, 16, 0, 8, 20, seed=5, want_sum2=True)
-    b, b2, rb = LightOracleScene(s.serialize()).render(cam, 24, 16, 0, 8, 20, seed=5, want_sum2=True)
+    b, b2, rb = FeatureOracleScene(s.serialize()).render(cam, 24, 16, 0, 8, 20, seed=5, want_sum2=True)
     assert np.array_equal(a, b) and np.array_equal(a2, b2) and ra == rb
 
 
@@ -197,7 +197,7 @@ def test_known_answer_on_the_oracle(rtb, orc, kind):
     variances = {}
     for lights in (False, True):
         s.sample_lights([light] if lights else [])
-        a, a2, _ = LightOracleScene(s.serialize()).render(cam, KW, KH, 0, spp, 2, seed=11 + lights, want_sum2=True)
+        a, a2, _ = FeatureOracleScene(s.serialize()).render(cam, KW, KH, 0, spp, 2, seed=11 + lights, want_sum2=True)
         variances[lights] = check_known_answer(a, a2, spp, want, f"oracle {kind} lights={lights}")
     assert variances[True] < 0.5 * variances[False]
 
@@ -218,7 +218,7 @@ def test_oracle_light_sampling_is_unbiased(rtb, orc, name):
     W = H = 24; spp = 512
     a, a2, _ = orc.OracleScene(s.serialize()).render(cam, W, H, 0, spp, 50, seed=21, want_sum2=True)
     s.sample_lights(s.info.light_ids)
-    b, b2, _ = LightOracleScene(s.serialize()).render(cam, W, H, 0, spp, 50, seed=22, want_sum2=True)
+    b, b2, _ = FeatureOracleScene(s.serialize()).render(cam, W, H, 0, spp, 50, seed=22, want_sum2=True)
     for c, (bias, sigma) in enumerate(mean_error_sigmas(b, b2, a, a2, spp)):
         print(f"{name} channel {c}: error / sigma {bias / sigma:+.2f}")
         assert abs(bias) <= 3.0 * sigma, (name, c, bias, sigma)
@@ -240,7 +240,7 @@ def test_oracle_variance_reduction_on_the_cornell_box(rtb, orc):
     W = H = 48; spp = 256
     a, a2, _ = orc.OracleScene(s.serialize()).render(cam, W, H, 0, spp, 50, seed=7, want_sum2=True)
     s.sample_lights(s.info.light_ids)
-    b, b2, _ = LightOracleScene(s.serialize()).render(cam, W, H, 0, spp, 50, seed=7, want_sum2=True)
+    b, b2, _ = FeatureOracleScene(s.serialize()).render(cam, W, H, 0, spp, 50, seed=7, want_sum2=True)
     ratio = pixel_variance(b, b2, spp).mean() / pixel_variance(a, a2, spp).mean()
     print(f"book2_cornell 48x48x{spp}: variance with / without light sampling {ratio:.3f}")
     assert ratio <= VARIANCE_RATIO_BAR

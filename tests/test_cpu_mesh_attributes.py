@@ -1,6 +1,6 @@
 """CPU tests of per-vertex shading normals and texture coordinates of mesh triangles (DESIGN.md §5e): the rtb_add_mesh_ex
 API, the RTBS v4 blob, the flattener, MeshHandle::LoadObjShaded, rtb_app's --smooth / --obj-texture, and hand-derived
-answers on the CPU restatement (tests/mesh_oracle.cpp): interpolated normals and UVs on one triangle, plain and instanced,
+answers on the CPU restatement (tests/feature_oracle.cpp): interpolated normals and UVs on one triangle, plain and instanced,
 canonical UVs reproducing the plain mesh bit for bit, and the white furnace on a smooth icosphere."""
 import ctypes as C
 import subprocess
@@ -10,10 +10,8 @@ import numpy as np
 import pytest
 
 import mesh_scenes as ms
-from env_oracle import EnvOracleScene
+from feature_oracle import FeatureOracleScene
 from helpers import parse_blob
-from light_oracle import LightOracleScene
-from mesh_oracle import MeshOracleScene
 
 ROOT = Path(__file__).resolve().parent.parent
 PKG = ROOT / "ray-tracing-v06_b200"
@@ -81,7 +79,7 @@ def test_null_attributes_are_the_plain_mesh(rtb):
 
 def test_v4_blob_round_trip(rtb, orc):
     """With attributes: v4 = the v1 body with each attributed triangle's aux = record + 1, an empty light list, an empty
-    map record, n and the records (normals normalised in double, zero kept).  The older oracles refuse v4; the mesh oracle
+    map record, n and the records (normals normalised in double, zero kept).  The plain oracle refuses v4; the feature oracle
     reads back what was given."""
     v, f = ms.icosphere(1)
     n = v * np.float32(3.0)
@@ -101,28 +99,27 @@ def test_v4_blob_round_trip(rtb, orc):
     assert np.frombuffer(tail[:4], np.int32)[0] == 0
     assert list(np.frombuffer(tail[4:16], np.int32)) == [0, 0, 0]
     assert np.frombuffer(tail[28:32], np.uint32)[0] == len(f)
-    got = MeshOracleScene(blob).attrs()
+    got = FeatureOracleScene(blob).attrs()
     assert len(got) == len(f) and np.all(got["flags"] == 3)
     n64 = n.astype(np.float64); ln = np.linalg.norm(n64, axis=1, keepdims=True)
     unit = np.where(ln > 0, n64 / np.where(ln > 0, ln, 1), 0).astype(np.float32)
     assert np.array_equal(got["n"], unit[f]) and np.array_equal(got["uv"], uv[f])
-    for oracle in (orc.OracleScene, LightOracleScene, EnvOracleScene):
-        with pytest.raises(RuntimeError, match="version"):
-            oracle(blob)
+    with pytest.raises(RuntimeError, match="version"):
+        orc.OracleScene(blob)
     # with a light list and a map too: the list, the map, then the attributes
     s.set_environment(np.ones((2, 4, 3), np.float32))
     blob3 = s.serialize()
     assert parse_blob(blob3)[0]["version"] == 4 and len(blob3) == len(blob) + 4 * 2 * 3 * 4
-    assert len(MeshOracleScene(blob3).attrs()) == len(f)
+    assert len(FeatureOracleScene(blob3).attrs()) == len(f)
 
 
 def test_scenes_without_attributes_keep_their_format(rtb):
-    """Registry scenes through the mesh oracle's loader, and a mesh without attributes: unchanged versions and hashes."""
+    """Registry scenes through the feature oracle's loader, and a mesh without attributes: unchanged versions and hashes."""
     for name in ("mesh_icospheres", "book2_final"):
         s = rtb.Scene.named(name)
         blob = s.serialize()
         assert parse_blob(blob)[0]["version"] == 1
-        MeshOracleScene(blob)
+        FeatureOracleScene(blob)
 
 
 @pytest.mark.parametrize("attrs", ["normals", "uvs", "both"])
@@ -233,7 +230,7 @@ int main(int, char** argv) {
                     "-o", str(tmp_path / "m"), str(tmp_path / "m.cpp"), f"-L{PKG}", "-lrtb200", f"-Wl,-rpath,{PKG}"], check=True, capture_output=True)
     out = subprocess.run([str(tmp_path / "m"), str(tmp_path / "ico.obj"), str(tmp_path / "m.rtbs")], check=True, capture_output=True, text=True).stdout.split()
     assert out == [str(len(v)), str(len(f))]
-    at = MeshOracleScene((tmp_path / "m.rtbs").read_bytes()).attrs()
+    at = FeatureOracleScene((tmp_path / "m.rtbs").read_bytes()).attrs()
     assert len(at) == len(f) and np.all(at["flags"] == 1)
     # on a unit icosphere the computed normals are close to the positions
     assert np.allclose(at["n"], v[f], atol=0.02)
@@ -271,7 +268,7 @@ def test_triangle_known_answers_oracle(rtb, instanced, flip, normals, uvs):
         pytest.skip("flip negates normals")
     s = ms.triangle_scene(rtb, normals=normals, flip=flip, uvs=uvs, instanced=instanced)
     rays, ab, back = ms.triangle_rays(rtb, instanced=instanced, inset=1e-4)
-    got = MeshOracleScene(s.serialize()).trace(rays, rtb.HIT_DTYPE)
+    got = FeatureOracleScene(s.serialize()).trace(rays, rtb.HIT_DTYPE)
     _check_hits(got, rays, ab, back, normals, uvs, instanced)
 
 
@@ -280,8 +277,8 @@ def test_canonical_uvs_reproduce_the_plain_mesh_oracle(rtb):
     accumulators equal the plain mesh's bit for bit."""
     (a, cam), (b, _) = ms.canonical_uv_scene(rtb, False), ms.canonical_uv_scene(rtb, True)
     assert parse_blob(b.serialize())[0]["version"] == 4
-    ra = MeshOracleScene(a.serialize()).render(cam, 48, 32, 0, 4, 8)
-    rb = MeshOracleScene(b.serialize()).render(cam, 48, 32, 0, 4, 8)
+    ra = FeatureOracleScene(a.serialize()).render(cam, 48, 32, 0, 4, 8)
+    rb = FeatureOracleScene(b.serialize()).render(cam, 48, 32, 0, 4, 8)
     assert ra[2] == rb[2] and np.array_equal(ra[0], rb[0])
 
 
@@ -292,7 +289,7 @@ def test_white_furnace_on_an_icosphere_oracle(rtb, smooth):
     into the closed mesh), and no pixel exceeds spp."""
     s, cam = ms.furnace_scene(rtb, smooth=smooth)
     spp = 16
-    acc, _, _ = MeshOracleScene(s.serialize()).render(cam, 32, 32, 0, spp, 20)
+    acc, _, _ = FeatureOracleScene(s.serialize()).render(cam, 32, 32, 0, spp, 20)
     rgb = acc[..., :3]
     assert np.all(rgb == np.round(rgb)) and np.all(rgb <= spp) and np.all(rgb >= 0)
     assert np.all(rgb[..., 0] == rgb[..., 1]) and np.all(rgb[..., 1] == rgb[..., 2])

@@ -1,6 +1,6 @@
 """CPU tests of the GGX microfacet materials (DESIGN.md §5f): the rtb_add_rough_metal / rtb_add_rough_dielectric API, the
-RTBS v5 blob and flatten hash, the older oracles' refusal of v5, rtb_app's --obj-material / --alpha refusals, the float64
-reference integral's own checks (tests/microfacet_reference.py), and the CPU restatement (tests/rough_oracle.cpp) against
+RTBS v5 blob and flatten hash, the plain oracle's refusal of v5, rtb_app's --obj-material / --alpha refusals, the float64
+reference integral's own checks (tests/microfacet_reference.py), and the CPU restatement (tests/feature_oracle.cpp) against
 that integral on the plane scenes the GPU tests use."""
 import ctypes as C
 import math
@@ -11,11 +11,8 @@ import numpy as np
 import pytest
 
 import microfacet_reference as mr
-from env_oracle import EnvOracleScene
+from feature_oracle import FeatureOracleScene
 from helpers import parse_blob
-from light_oracle import LightOracleScene
-from mesh_oracle import MeshOracleScene
-from rough_oracle import RoughOracleScene
 
 ROOT = Path(__file__).resolve().parent.parent
 PKG = ROOT / "ray-tracing-v06_b200"
@@ -93,7 +90,7 @@ def test_api_refusals_leave_the_scene_unchanged(rtb):
 
 def test_v5_blob_round_trip(rtb, orc):
     """v5 = the v4 content (empty light list, empty map record, no attributes), then n_materials and one width per material
-    (0 for the other kinds).  The plain, light, environment and mesh oracles refuse it; the rough oracle reads it back."""
+    (0 for the other kinds).  The plain oracle refuses it; the feature oracle reads it back."""
     def build(rough):
         s = rtb.Scene()
         lam = s.lambertian((0.5, 0.5, 0.5))
@@ -114,17 +111,16 @@ def test_v5_blob_round_trip(rtb, orc):
     assert np.frombuffer(tail[:4], np.int32)[0] == 0 and list(np.frombuffer(tail[4:16], np.int32)) == [0, 0, 0]
     assert np.frombuffer(tail[28:32], np.uint32)[0] == 0 and np.frombuffer(tail[32:36], np.uint32)[0] == 4
     assert np.array_equal(np.frombuffer(tail[36:], np.float32), np.float32([0, 0, 0.25, 0.7]))
-    assert np.array_equal(RoughOracleScene(blob).alphas(), np.float32([0, 0, 0.25, 0.7]))
-    for oracle in (orc.OracleScene, LightOracleScene, EnvOracleScene, MeshOracleScene):
-        with pytest.raises(RuntimeError, match="version"):
-            oracle(blob)
+    assert np.array_equal(FeatureOracleScene(blob).alphas(), np.float32([0, 0, 0.25, 0.7]))
+    with pytest.raises(RuntimeError, match="version"):
+        orc.OracleScene(blob)
     # the same geometry without the rough materials hashes differently only through them
     assert s.flatten_hash() != p.flatten_hash()
     # with a map, a light list and attributes too: the v4 content in full, then the widths
     s.set_environment(np.ones((2, 4, 3), np.float32))
     blob2 = s.serialize()
     assert parse_blob(blob2)[0]["version"] == 5 and len(blob2) == len(blob) + 2 * 4 * 3 * 4
-    assert np.array_equal(RoughOracleScene(blob2).alphas(), np.float32([0, 0, 0.25, 0.7]))
+    assert np.array_equal(FeatureOracleScene(blob2).alphas(), np.float32([0, 0, 0.25, 0.7]))
 
 
 def test_alpha_changes_the_hash(rtb):
@@ -136,12 +132,12 @@ def test_alpha_changes_the_hash(rtb):
 
 @pytest.mark.parametrize("name", ["book2_bouncing", "book2_final", "mesh_icospheres"])
 def test_scenes_without_rough_materials_keep_their_bytes(rtb, name):
-    """Registry scenes serialise as before (v1) and are read by the rough oracle's loader; adding a material of another
+    """Registry scenes serialise as before (v1) and are read by the feature oracle's loader; adding a material of another
     kind keeps v1."""
     s = rtb.Scene.named(name)
     blob = s.serialize()
     assert parse_blob(blob)[0]["version"] == 1
-    assert np.all(RoughOracleScene(blob).alphas() == 0)
+    assert np.all(FeatureOracleScene(blob).alphas() == 0)
 
 
 def test_app_option_refusals(rtb, tmp_path):
@@ -215,7 +211,7 @@ def test_oracle_matches_the_integral(rtb, kind, alpha, theta, back):
     """The CPU restatement on the white-sky plane (E_R for the metal, E_R + E_T for the glass) within 4 sigma."""
     s, cam = plane_scene(rtb, kind, theta, alpha, back=back)
     W, S = 8, 512
-    sum_, sum2, _ = RoughOracleScene(s.serialize()).render(cam, W, W, 0, S, 2, seed=3, want_sum2=True)
+    sum_, sum2, _ = FeatureOracleScene(s.serialize()).render(cam, W, W, 0, S, 2, seed=3, want_sum2=True)
     m, e = mean_and_error(sum_, sum2)
     if kind == "metal":
         want = mr.albedo(theta, alpha, "R", f0=1.0)

@@ -1,5 +1,5 @@
 """GPU tests of the HDR environment map (DESIGN.md §5d): the known answers of tests/test_cpu_environment.py through
-rtb_render, the CUDA path against the CPU restatement (tests/env_oracle.cpp) on the same Philox streams, unbiasedness of
+rtb_render, the CUDA path against the CPU restatement (tests/feature_oracle.cpp) on the same Philox streams, unbiasedness of
 the sampled map against the oracle's plain one, and the invariances a map must keep (specular-only paths, progressive,
 resumed and adaptive renders, two GPUs, the bounds-checked build, rtb_app)."""
 import json
@@ -12,7 +12,7 @@ import pytest
 
 import env_scenes as es
 from conftest import ROOT
-from env_oracle import EnvOracleScene
+from feature_oracle import FeatureOracleScene
 from helpers import psnr, tonemap
 from test_cpu_environment import SMALL_OBJ, check_mean, write_pfm
 from test_cpu_light_sampling import mean_error_sigmas
@@ -127,7 +127,7 @@ def test_same_streams_as_the_oracle(rtb, case, W, H, S, D):
     scene, cam = CASES[case](rtb)
     r = rtb.Renderer(0); r.set_scene(scene); r.set_camera(cam)
     r.reset_counters(); r.render(W, H, 0, S, D, seed=1984); g = r.download_accum(); cnt = r.counters()
-    ref, _, rays = EnvOracleScene(scene.serialize()).render(cam, W, H, 0, S, D, seed=1984)
+    ref, _, rays = FeatureOracleScene(scene.serialize()).render(cam, W, H, 0, S, D, seed=1984)
     diff = np.abs(g[..., :3] - ref[..., :3]).max(axis=2)
     bad = float((diff > 1e-4 * np.maximum(np.abs(ref[..., :3]).max(axis=2), 1.0)).mean())
     print(f"{case} {W}x{H}x{S}: {bad * 100:.4f} % of pixels differ, rays gpu {cnt.rays} oracle {rays}, PSNR {psnr(tonemap(g), tonemap(ref)):.1f} dB")
@@ -140,7 +140,7 @@ def test_sampled_map_agrees_with_the_oracle_unsampled(rtb):
     streams, per channel within 3 sigma."""
     W, H, SPP, D = 48, 32, 2048, 12
     plain, cam = sun_scene(rtb, 64, 32, sample=False, sun_deg=8.0)
-    a, a2, _ = EnvOracleScene(plain.serialize()).render(cam, W, H, 0, SPP, D, seed=202, want_sum2=True)
+    a, a2, _ = FeatureOracleScene(plain.serialize()).render(cam, W, H, 0, SPP, D, seed=202, want_sum2=True)
     sampled, _ = sun_scene(rtb, 64, 32, sample=True, sun_deg=8.0)
     g, g2 = _render(rtb, sampled, cam, W, H, SPP, D, 101)
     for c, (bias, sigma) in enumerate(mean_error_sigmas(g, g2, a, a2, SPP)):

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from helpers import psnr, tonemap
-from light_oracle import LightOracleScene
+from feature_oracle import FeatureOracleScene
 from test_cpu_light_sampling import (KH, KW, VARIANCE_RATIO_BAR, check_known_answer, known_answer_scene, mean_error_sigmas,
                                      pixel_variance)
 
@@ -29,7 +29,7 @@ def test_same_streams_as_the_oracle(rtb, name, W, H, S, D):
     scene, cam = _lit(rtb, name)
     r = rtb.Renderer(0); r.set_scene(scene); r.set_camera(cam)
     r.reset_counters(); r.render(W, H, 0, S, D, seed=1984); g = r.download_accum(); cnt = r.counters()
-    ref, _, rays = LightOracleScene(scene.serialize()).render(cam, W, H, 0, S, D, seed=1984)
+    ref, _, rays = FeatureOracleScene(scene.serialize()).render(cam, W, H, 0, S, D, seed=1984)
     diff = np.abs(g[..., :3] - ref[..., :3]).max(axis=2)
     bad = float((diff > 1e-4 * np.maximum(np.abs(ref[..., :3]).max(axis=2), 1.0)).mean())
     print(f"{name} {W}x{H}x{S} with lights: {bad * 100:.4f} % of pixels differ, rays gpu {cnt.rays} oracle {rays}, PSNR {psnr(tonemap(g), tonemap(ref)):.1f} dB")

@@ -1,6 +1,6 @@
 """GPU tests of per-vertex shading normals and texture coordinates of mesh triangles (DESIGN.md §5e): the known answers of
 tests/test_cpu_mesh_attributes.py through rtb_trace_rays and rtb_render, the CUDA path against the CPU restatement
-(tests/mesh_oracle.cpp) on the same Philox streams, adaptive rounds, light sampling, what smooth shading buys against an
+(tests/feature_oracle.cpp) on the same Philox streams, adaptive rounds, light sampling, what smooth shading buys against an
 analytic sphere, two GPUs, the bounds-checked build and rtb_app."""
 import json
 import os
@@ -13,7 +13,7 @@ import pytest
 import mesh_scenes as ms
 from conftest import ROOT
 from helpers import psnr, tonemap
-from mesh_oracle import MeshOracleScene
+from feature_oracle import FeatureOracleScene
 from test_cpu_light_sampling import mean_error_sigmas
 from test_cpu_mesh_attributes import _check_hits
 from test_gpu_adaptive import _dense_snapshots, _expect_per_pixel
@@ -50,7 +50,7 @@ def test_triangle_known_answers_trace_rays(rtb, instanced, flip, normals, uvs):
     r = rtb.Renderer(0); r.set_scene(s)
     got = r.trace_rays(rays)
     _check_hits(got, rays, ab, back, normals, uvs, instanced)
-    _same_hits(got, MeshOracleScene(s.serialize()).trace(rays, rtb.HIT_DTYPE))
+    _same_hits(got, FeatureOracleScene(s.serialize()).trace(rays, rtb.HIT_DTYPE))
 
 
 def test_canonical_uvs_reproduce_the_plain_mesh(rtb):
@@ -60,7 +60,7 @@ def test_canonical_uvs_reproduce_the_plain_mesh(rtb):
     ga, ga2, ra = _render(rtb, a, cam, W, H, S, D, 5)
     gb, gb2, rb = _render(rtb, b, cam, W, H, S, D, 5)
     assert np.array_equal(ga, gb) and np.array_equal(ga2, gb2) and ra == rb
-    ref, _, rays = MeshOracleScene(b.serialize()).render(cam, W, H, 0, S, D, seed=5)
+    ref, _, rays = FeatureOracleScene(b.serialize()).render(cam, W, H, 0, S, D, seed=5)
     assert np.array_equal(gb, ref) and rays == rb
 
 
@@ -71,7 +71,7 @@ def test_white_furnace_smooth_icosphere(rtb):
     g, _, _ = _render(rtb, s, cam, 48, 48, spp, 20, 7)
     rgb = g[..., :3]
     assert np.all(rgb == np.round(rgb)) and np.all(rgb <= spp)
-    ref, _, _ = MeshOracleScene(s.serialize()).render(cam, 48, 48, 0, spp, 20, seed=7)
+    ref, _, _ = FeatureOracleScene(s.serialize()).render(cam, 48, 48, 0, spp, 20, seed=7)
     assert np.array_equal(g, ref)
 
 
@@ -87,7 +87,7 @@ def test_same_streams_as_the_oracle(rtb, kind, monkeypatch):
     scene, cam = ms.parity_scene(rtb, "glass_metal" if kind == "binned_tail" else kind)
     W, H, S, D = 192, 128, 8, 30
     g, _, rays_g = _render(rtb, scene, cam, W, H, S, D, 1984)
-    ref, _, rays = MeshOracleScene(scene.serialize()).render(cam, W, H, 0, S, D, seed=1984)
+    ref, _, rays = FeatureOracleScene(scene.serialize()).render(cam, W, H, 0, S, D, seed=1984)
     diff = np.abs(g[..., :3] - ref[..., :3]).max(axis=2)
     bad = float((diff > 1e-4 * np.maximum(np.abs(ref[..., :3]).max(axis=2), 1.0)).mean())
     print(f"{kind} {W}x{H}x{S}: {bad * 100:.4f} % of pixels differ, exact {np.array_equal(g, ref)}, rays gpu {rays_g} oracle {rays}, "
@@ -129,7 +129,7 @@ def test_trace_rays_on_a_deep_gpu_lbvh(rtb):
     from helpers import camera_rays
     rays = camera_rays(rtb, cam, 160, 160)
     got = r.trace_rays(rays)
-    want = MeshOracleScene(scene.serialize()).trace(rays, rtb.HIT_DTYPE)
+    want = FeatureOracleScene(scene.serialize()).trace(rays, rtb.HIT_DTYPE)
     assert (got["t"] < 1e30).mean() > 0.5
     tri = got["material"] == 0                                  # the mesh's material (the ball's is 1)
     assert tri.mean() > 0.3

@@ -1,5 +1,5 @@
 """GPU tests of the GGX microfacet materials (DESIGN.md §5f): directional albedo against the float64 integral of the BSDF
-(tests/microfacet_reference.py), path for path against the CPU restatement (tests/rough_oracle.cpp) on every case of
+(tests/microfacet_reference.py), path for path against the CPU restatement (tests/feature_oracle.cpp) on every case of
 tests/feature_scenes.py with rough objects added, the smooth limits and the white furnace, schedule invariance of the
 ROUGH instantiations, checkpoints, two GPUs, rtb_app and the bounds-checked build."""
 import json
@@ -14,7 +14,7 @@ import feature_scenes as fs
 import microfacet_reference as mr
 from conftest import ROOT
 from helpers import psnr, tonemap
-from rough_oracle import RoughOracleScene
+from feature_oracle import FeatureOracleScene
 from test_cpu_rough_materials import half_sky, mean_and_error, plane_scene
 from test_gpu_schedules import SCHEDULES, schedule
 
@@ -111,7 +111,7 @@ def test_same_streams_as_the_rough_oracle(rtb, monkeypatch, case):
     scene, cam = rough_case(rtb, case)
     assert scene.serialize()[4] == 5
     W, H, S, D = 128, 96, 6, 24
-    ref, _, rays = RoughOracleScene(scene.serialize()).render(cam, W, H, 0, S, D, seed=1984)
+    ref, _, rays = FeatureOracleScene(scene.serialize()).render(cam, W, H, 0, S, D, seed=1984)
     for name in ("B", "A", "D"):
         with schedule(monkeypatch, name):
             r = rtb.Renderer(0); r.set_scene(scene); r.set_camera(cam); r.reset_counters()

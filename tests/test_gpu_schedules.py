@@ -18,7 +18,7 @@ import pytest
 
 import feature_scenes as fs
 from conftest import ROOT
-from mesh_oracle import MeshOracleScene
+from feature_oracle import FeatureOracleScene
 
 pytestmark = pytest.mark.gpu
 
@@ -127,7 +127,7 @@ def test_wavefront_every_bounce_matches_the_oracle(rtb, monkeypatch, case):
         r.render(OW, OH, 0, OS, OD, seed=1984)
         g = r.download_accum(); rays_g = int(r.counters().rays)
     t = time.time()
-    ref, _, rays = MeshOracleScene(scene.serialize()).render(cam, OW, OH, 0, OS, OD, seed=1984)
+    ref, _, rays = FeatureOracleScene(scene.serialize()).render(cam, OW, OH, 0, OS, OD, seed=1984)
     t = time.time() - t
     diff = np.abs(g[..., :3] - ref[..., :3]).max(axis=2)
     bad = float((diff > 1e-4 * np.maximum(np.abs(ref[..., :3]).max(axis=2), 1.0)).mean())

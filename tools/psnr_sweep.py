@@ -37,7 +37,7 @@ def psnr(a, b):
 if __name__ == "__main__":
     rtb = importlib.import_module("ray-tracing-v06_b200")
     orc = importlib.import_module("pyoracle")
-    light_oracle = importlib.import_module("light_oracle")
+    feature_oracle = importlib.import_module("feature_oracle")
     lights = "--sample-lights" in sys.argv[1:]
     out = []
     for cfg, name in (("4", "book2_cornell_smoke"), ("5", "book2_final")):
@@ -69,7 +69,7 @@ if __name__ == "__main__":
         # same streams, GPU vs oracle (256 spp at a quarter of the size to keep the CPU side short)
         w2, h2 = W // 4, H // 4
         r.render(w2, h2, 0, 256, D, seed=1984); g = r.download_accum()
-        cpu = light_oracle.LightOracleScene if lights else orc.OracleScene   # (the CPU integrator with the light mixture)
+        cpu = feature_oracle.FeatureOracleScene if lights else orc.OracleScene   # (the CPU integrator with the light mixture)
         o, _, _ = cpu(s.serialize()).render(i.camera, w2, h2, 0, 256, D, seed=1984)
         row["same_streams_vs_oracle"] = {"width": w2, "height": h2, "spp": 256, "psnr_db": round(psnr(tonemap(g), tonemap(o)), 2),
                                          "pixels_differing": float((np.abs(g[..., :3] - o[..., :3]).max(axis=2) > 1e-4 * np.maximum(np.abs(o[..., :3]).max(axis=2), 1.0)).mean())}
